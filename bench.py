@@ -1,7 +1,7 @@
 """bench.py - TwoWL forward+backward target-links/s on synthetic graphs (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload rmat|collab|cora] [--hidden H]
-                    [--impl ours|reference]
+                    [--impl ours|reference] [--dump-outputs DIR]
 
 One *step* = LocalWLNet.forward + binary_cross_entropy_with_logits + backward on one batch
 (reference TwoWL/model/train.py:36-38) through the drop-in API of link-prediction-gnn_b200/TwoWL.
@@ -17,6 +17,9 @@ One *step* = LocalWLNet.forward + binary_cross_entropy_with_logits + backward on
            north_star's partition), next to the target-link data-parallel `value`.
 `--impl reference` times that CPU path alone (the reference is pure Python/torch-CPU; its hot loop is
 restated 1:1 by the oracle, which is pinned to the reference by tests/golden).
+`--dump-outputs DIR` writes what the last timed step computed - loss, logits and every parameter gradient - as
+DIR/<name>.npy (float32). Graph, weights and batches are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -321,6 +324,28 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+DUMP_BYTES = 60 << 20          # array data; with the .npy headers a dump stays under 64 MB
+
+
+def dump_outputs(arrays, out_dir):
+    """Write every float32 array as out_dir/<name>.npy, at most DUMP_BYTES in all. Smaller arrays are written whole; an array
+    larger than an equal share of what is left keeps that share of its elements, at positions drawn with a fixed seed (sorted,
+    from the flattened array): the same positions on every run with the same arguments."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    left, sampled = DUMP_BYTES // 4, []
+    by_size = sorted(arrays.items(), key=lambda kv: kv[1].size)
+    for i, (name, a) in enumerate(by_size):
+        keep = min(a.size, left // (len(by_size) - i))
+        left -= keep
+        if keep < a.size:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+            sampled.append(name)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print(f"dump-outputs: {len(arrays)} arrays ({total / 2**20:.1f} MiB) -> {out_dir}"
+          + (f"; sampled: {', '.join(sampled)}" if sampled else ""), file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------ our arm
 
 def main():
@@ -344,7 +369,14 @@ def main():
                     help="multi-GPU: 'links' = every rank steps its own disjoint slice of the target links (weak scaling, the "
                          "default); 'rows' = ONE step whose pair rows are cut into row blocks over the ranks (strong scaling, "
                          "twowl_b200.rowshard)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's loss, logits and parameter gradients as DIR/<name>.npy (float32, at most "
+                         "64 MB in all: larger outputs keep a fixed seeded sample of their elements)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -391,9 +423,10 @@ def main():
 
     l2_flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
 
-    def measure(rows: bool):
+    def measure(rows: bool, keep_outputs: bool = False):
         """One measurement of K steps. rows = False: every rank steps its own disjoint slice of the target links (data parallel,
-        weak scaling); rows = True: ONE batch per step, its pair rows cut into row blocks over the ranks (strong scaling)."""
+        weak scaling); rows = True: ONE batch per step, its pair rows cut into row blocks over the ranks (strong scaling).
+        keep_outputs: also return the last timed step's loss, logits and gradients as host arrays."""
         nb = max(2, g["und"] // 10)
         if world > 1 and not rows:         # the slices of the ranks are disjoint: cap the global batch at the id range
             nb = min(nb, g["und"] // world, (P // 2) // world)
@@ -426,10 +459,15 @@ def main():
             ei_new, x_new, ei2_new = U.sample_block(idx1, n, pos, ei2)
             return x_new, ei_new, torch.cat((idx1, idx2)), ei2_new, y
 
-        def fwd_bwd(inp):
+        kept = {}
+
+        def fwd_bwd(inp, keep=False):
+            """keep: also hold on to this step's loss and logits in `kept` (--dump-outputs)."""
             if len(inp) == 3:
                 loss = gstep(*inp)
                 sync_grads()
+                if keep:
+                    kept.update(loss=loss, logits=gstep.logits)
                 return loss
             x_new, ei_new, idx, ei2_new, y = inp
             for p_ in mod.parameters():
@@ -438,6 +476,8 @@ def main():
             loss = torch.nn.functional.binary_cross_entropy_with_logits(out, y)
             loss.backward()
             sync_grads()
+            if keep:
+                kept.update(loss=loss, logits=out)
             return loss
 
         batches = [draw_batch(g["und"], P // 2, nb, i, replicate=rows) for i in range(args.steps + args.warmup)]
@@ -452,11 +492,16 @@ def main():
             for i in range(args.steps):
                 l2_flush.fill_(i & 255)     # evict L2 between timed steps (inputs also exceed L2 at rmat/collab size)
                 ev[i][0].record()
-                fwd_bwd(inputs[args.warmup + i])
+                fwd_bwd(inputs[args.warmup + i], keep=keep_outputs and i + 1 == args.steps)
                 ev[i][1].record()
             barrier()
         launches = ops.launches() - launches0
         step_ms = [a.elapsed_time(b) for a, b in ev]
+        outputs = None
+        if keep_outputs:                # copied now: the next steps overwrite the gradients (and a replayed graph its logits)
+            named = list(kept.items()) + [("grad." + k, p.grad) for k, p in mod.named_parameters() if p.grad is not None]
+            outputs = {k: v.detach().float().cpu().numpy() for k, v in named}
+            kept.clear()
         # ---- the same K steps once more with CUDA events around every kernel group (roofline); kept out of the timed
         #      region above because two extra events per op are not free for the launch-bound small workloads ----
         if gstep is not None:   # a replayed graph has no per-op events: the per-kernel roofline comes from the eager path
@@ -503,10 +548,10 @@ def main():
             comm = rowshard.comm_summary()
         del mod, gstep
         return dict(total_ms=total_ms, e2e_ms=e2e_ms, launches=launches, prof=prof, sb_ms=sb_ms, links=links, L=L, h2d=h2d,
-                    clocks=clocks.summary(), comm=comm)
+                    clocks=clocks.summary(), comm=comm, outputs=outputs)
 
     rows_main = args.shard == "rows" and world > 1
-    m = measure(rows_main)
+    m = measure(rows_main, keep_outputs=bool(args.dump_outputs) and rank == 0)
     strong = None
     if world > 1 and not rows_main and not args.graph and not explicit and not args.no_strong:
         # north_star's partition, measured in the same run: one batch per step, pair rows cut over the ranks
@@ -529,6 +574,8 @@ def main():
             dist.destroy_process_group()
         return
     total_ms, e2e_ms, prof, launches = m["total_ms"], m["e2e_ms"], m["prof"], m["launches"]
+    if args.dump_outputs:
+        dump_outputs(m["outputs"], args.dump_outputs)
 
     # ---- roofline of the dominant kernel ----
     peaks = {}
