@@ -104,6 +104,18 @@ int twowl_nonedge_sample(const int64_t* row, int64_t s_row, const int64_t* col, 
                          int64_t count, int32_t undirected, uint64_t seed, int32_t rounds, int64_t* out_row, int64_t* out_col,
                          uint8_t* done, int32_t* unresolved, void* ws, size_t ws_bytes, void* stream);
 
+/* Per-source negatives for ranking evaluation (OGB's filtered tail corruption, ogbl-citation2 style): row i of out (int64[P*k],
+ * row-major) holds k DISTINCT nodes w, uniform over the nodes allowed for src[i] (int64[P], contiguous): w != src[i] and neither
+ * (src[i], w) nor (w, src[i]) is in the exclusion edge list (row, col) (strides as in twowl_nonedge_sample). Same hash table and
+ * smallest-slot-wins rounds as twowl_nonedge_sample, with the claim keys (i, w) stored past the N^2 edge keys: the result depends
+ * on (seed, inputs) only. Slots still unfilled after `rounds` rounds hold -1 and are counted in unresolved[0] (a source with fewer
+ * than k allowed nodes, one outside [0, num_nodes), or too few rounds for a source that is adjacent to nearly every node).
+ * P * k < 2^31, num_nodes < 2^31. */
+size_t twowl_tail_negative_sample_workspace_bytes(int64_t n_edges, int64_t P, int64_t k);
+int twowl_tail_negative_sample(const int64_t* row, int64_t s_row, const int64_t* col, int64_t s_col, int64_t n_edges, int64_t num_nodes,
+                               const int64_t* src, int64_t P, int64_t k, uint64_t seed, int32_t rounds, int64_t* out,
+                               int32_t* unresolved, void* ws, size_t ws_bytes, void* stream);
+
 /* Order-preserving column selection of a [2,T] int64 matrix (blockei2 utils.py:48-50; the ei filter of
  * sample_block utils.py:62-63):
  *   mode 0: keep column t iff !mask[t]            mode 1: keep column t iff !mask[row0[t]]
@@ -450,6 +462,25 @@ int twowl_pair_dw_gn(const float* Of, const float* Or, const float* consts, cons
  * score, label: fp32[n]; out: double[3] on the device. Deterministic (radix sort + fixed-order double sums). */
 size_t twowl_auc_workspace_bytes(int64_t n);
 int twowl_auc(const float* score, const float* label, int64_t n, double* out, void* ws, size_t ws_bytes, void* stream);
+
+/* Ranking metrics of the OGB link-prediction evaluators. h_ks is a HOST array of n_k cut-offs, 1 <= n_k <= TWOWL_RANK_MAX_K,
+ * each >= 1. Both are deterministic: integer counts, and (MRR) double sums in a fixed two-level order. */
+#define TWOWL_RANK_MAX_K 16
+
+/* Hits@K against a shared negative set (OGB _eval_hits, ogbl-collab / ogbl-ddi): score, label fp32[n], a positive is
+ * label > 0.5. out (double[n_k + 2], device) = (hits@K_1 .. hits@K_nk, n_pos, n_neg) with hits@K = #(positives with score
+ * > the K-th largest negative score) / n_pos, strict >; 1.0 when n_neg < K; NaN for every K when there is no positive or any
+ * score is NaN. -0.0 and +0.0 are the same score. */
+size_t twowl_hits_at_k_workspace_bytes(int64_t n);
+int twowl_hits_at_k(const float* score, const float* label, int64_t n, const int64_t* h_ks, int32_t n_k, double* out, void* ws,
+                    size_t ws_bytes, void* stream);
+
+/* MRR and hits@k against k negatives per positive (OGB _eval_mrr, ogbl-citation2): pos fp32[P], neg fp32[P*k] row-major (row i
+ * = the k negatives of positive i). rank_i = 0.5 (#(neg_ij > pos_i) + #(neg_ij >= pos_i)) + 1; out (double[n_k + 2], device) =
+ * (mean 1/rank_i, mean(rank_i <= k_1) .. mean(rank_i <= k_nk), P); every metric is NaN when P = 0 or any input is NaN. */
+size_t twowl_rank_metrics_workspace_bytes(int64_t P);
+int twowl_rank_metrics(const float* pos, const float* neg, int64_t P, int64_t k, const int64_t* h_ks, int32_t n_k, double* out,
+                       void* ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------------------------ structured wedge path ------- */
 

@@ -105,6 +105,32 @@ def test(mod, dataset, test=False, curve=True):
     return score, fpr, tpr
 
 
+@torch.no_grad()
+def test_ranking(mod, dataset, ks=(20, 50, 100)):
+    """Ranking evaluation of a link predictor (extension: the OGB link-prediction protocols) -> dict of floats. One full-graph
+    forward exactly like test(), every prediction pair a target, then on the device:
+      * a table from TwoWL.operators.datasets.ranking_dataset (it has `rank_k`): logits [P positives | P x rank_k negatives, row
+        i = positive i's negatives] -> {"mrr": ..., "hits@k": ...} (ops.rank_metrics, OGB's _eval_mrr / ogbl-citation2);
+      * any other dataset, e.g. a val / test split with its shared negatives: labels y[0::2] as in test() ->
+        {"hits@K": ...} (ops.hits_at_k, OGB's _eval_hits / ogbl-collab).
+    The LOGITS are ranked, not sigmoid(logits): in fp32 the sigmoid rounds every logit above about 17 to 1.0, which would create
+    ties the model did not produce and change the ranks. One device->host copy for the whole dict."""
+    mod.eval()
+    n_edges = dataset.ei.shape[1]
+    targets = n_edges + torch.arange(dataset.y.shape[0], device=dataset.x.device)
+    logits = mod(dataset.x, dataset.ei, dataset.pos1, targets, dataset.ei2, True).reshape(-1)
+    ks = [int(k) for k in ks]
+    k = getattr(dataset, "rank_k", None)
+    if k is not None:
+        P = logits.numel() // (1 + int(k))
+        assert P * (1 + int(k)) == logits.numel(), "test_ranking: the logits do not have the [P | P x rank_k] layout"
+        vals = ops.rank_metrics(logits[:P], logits[P:].reshape(P, int(k)), ks).cpu()
+        return {"mrr": float(vals[0]), **{f"hits@{kk}": float(v) for kk, v in zip(ks, vals[1:1 + len(ks)].tolist())}}
+    labels = dataset.y.reshape(-1)[0::2][: logits.shape[0]]
+    vals = ops.hits_at_k(logits, labels, ks).cpu()
+    return {f"hits@{kk}": float(v) for kk, v in zip(ks, vals[:len(ks)].tolist())}
+
+
 def _record_run(record_dir, dsname, tst_score, seconds, fpr, tpr):
     """train.py:108-134: append 'AUC:<auc>   Time:<s>   ' to the dataset's record file; when this run's (unrounded) score is not
     below any recorded (rounded) one, keep its ROC curve in fpr.json / tpr.json in the working directory."""

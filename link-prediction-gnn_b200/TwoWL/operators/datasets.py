@@ -85,6 +85,46 @@ class BaseGraph:
         return self
 
 
+def ranking_dataset(bg: BaseGraph, split: int, num_neg: int, seed=0, pattern=None):
+    """An evaluation table for ranking metrics (extension: OGB's ogbl-citation2 protocol, filtered): split s's P undirected
+    positive pairs (u, v) - the even columns of its doubled positive block, as preprocess slices it - each followed in the table by
+    num_neg negatives (u, w) drawn by ops.sample_tail_negatives, w uniform over the nodes that are neither u nor a positive
+    partner of u in ANY split (bg.edge_pos). On the conventions of preprocess / split(s): x = bg.x[s] (setPosDegreeFeature must have
+    run), ei = bg.edge_indexs[s], pos1 = [ei.T ; double([positives ; negatives in row-major order]).T], y = 1 for the 2P positive
+    rows and 0 for the 2 P num_neg negative rows, ei2 the wedge index of that table (`pattern` as BaseGraph's, default bg.pattern).
+    The returned dataset carries rank_k = num_neg; TwoWL.model.train.test_ranking reads its logits as [P positives | P x num_neg]
+    negatives. split must be 1 (validation) or 2 (test): the training split's positives are edges of its own graph."""
+    from twowl_b200 import ops
+    s, k = int(split), int(num_neg)
+    if s not in (1, 2):
+        raise ValueError(f"ranking_dataset: split must be 1 (validation) or 2 (test), got {split}")
+    if k < 1:
+        raise ValueError(f"ranking_dataset: num_neg must be >= 1, got {num_neg}")
+    if not hasattr(bg, "edge_indexs") or not isinstance(bg.x, (list, tuple)):
+        raise ValueError("ranking_dataset: run bg.preprocess() and bg.setPosDegreeFeature() first")
+    npos = [int(v) for v in bg.num_pos]
+    ep = bg.edge_pos
+    block = ep[:, npos[0]:npos[0] + npos[1]] if s == 1 else ep[:, ep.shape[1] - npos[2]:]
+    pos = block[:, 0::2]                                            # (u, v) once per undirected pair
+    u = pos[0].contiguous()
+    w = ops.sample_tail_negatives(ep[0], ep[1], bg.num_nodes, u, k, seed=seed)
+    neg = torch.stack((u.repeat_interleave(k), w.reshape(-1)))
+    pred = double(torch.cat((pos, neg), dim=1))
+    ei = bg.edge_indexs[s]
+    pos1 = torch.cat((ei.t(), pred.t()), dim=0)
+    dev = ep.device
+    y = torch.cat((torch.ones((2 * pos.shape[1], 1), dtype=torch.float, device=dev),
+                   torch.zeros((2 * neg.shape[1], 1), dtype=torch.float, device=dev)))
+    pattern = bg.pattern if pattern is None else pattern
+    if pattern in ("2wl_l", "2wl_l_implicit"):
+        ei2 = (get_ei2_implicit if pattern == "2wl_l_implicit" else get_ei2)(bg.num_nodes, ei, pred)
+    else:
+        ei2 = None
+    ds = dataset(bg.x[s], bg.node_attr, ei, bg.edge_attrs[s], pos1, y, ei2)
+    ds.rank_k = k
+    return ds
+
+
 class _Data:
     """Stand-in for torch_geometric.data.Data(edge_index=...) as used by load() (datasets.py:165)."""
 

@@ -11,6 +11,10 @@
 //            slot draws again in round r + 1
 // The winner of a key is the SMALLEST slot that proposed it - a function of (seed, edges) only, so the output is reproducible
 // whatever the thread timing; only the cell a key lands in depends on the race, never who owns it. HBM-bound integer work.
+//
+// The same table and rounds draw per-source negatives for ranking evaluation (OGB's "filtered" tail corruption): slot j of row
+// i = j / k draws a node w uniform over [0, N), drops it when w == src[i] or the undirected edge {src[i], w} is in the table, and
+// otherwise claims the key N^2 + i N + w - past every edge key, so one table holds both - so that a row never holds w twice.
 #include "common.cuh"
 
 namespace twowl {
@@ -98,7 +102,7 @@ __global__ void __launch_bounds__(kSmpThreads) k_smp_resolve(int64_t count, int6
     if (own && *own == (int)i) {
       *own = -1;                               // final: no later round may take this key
       done[i] = 1;
-      out_row[i] = key / N;
+      if (out_row) out_row[i] = key / N;
       out_col[i] = key % N;
     } else {
       ++left;
@@ -106,6 +110,27 @@ __global__ void __launch_bounds__(kSmpThreads) k_smp_resolve(int64_t count, int6
   }
   left = __reduce_add_sync(0xffffffffu, left);
   if ((threadIdx.x & 31) == 0 && left) atomicAdd(unresolved, left);
+}
+
+// slot j of row i = j / k: candidate w uniform over [0,N); key N^2 + i N + w unless w is src[i] or a neighbour of it (then -1)
+__global__ void __launch_bounds__(kSmpThreads) k_tail_propose(uint64_t seed, int round, int64_t count, int64_t k, int64_t N,
+                                                              const int64_t* __restrict__ src, const uint8_t* __restrict__ done,
+                                                              long long* __restrict__ cand, long long* __restrict__ keys,
+                                                              int* __restrict__ owners, uint64_t mask) {
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < count; j += (int64_t)gridDim.x * blockDim.x) {
+    if (done[j]) continue;
+    const int64_t i = j / k, u = src[i];
+    const uint64_t a = smp_mix(seed + 0x9E3779B97F4A7C15ull * (uint64_t)(2 * j + 1) + ((uint64_t)round << 40));
+    const int64_t w = (int64_t)__umul64hi(a, (uint64_t)N);
+    long long key = -1;
+    if (u >= 0 && u < N && w != u) {
+      const long long edge = (long long)(u < w ? u * N + w : w * N + u);
+      // every key below N^2 in the table is an edge, inserted by an earlier kernel; the concurrent claims only fill empty cells
+      if (!smp_find(keys, owners, mask, edge)) key = (long long)(N * N + i * N + w);
+    }
+    cand[j] = key;
+    if (key >= 0) smp_claim(keys, owners, mask, key, (int)j);
+  }
 }
 
 static uint64_t smp_capacity(int64_t n_edges, int64_t count) {
@@ -157,5 +182,48 @@ extern "C" int twowl_nonedge_sample(const int64_t* row, int64_t s_row, const int
     TW_LAUNCH_CHECK();
   }
   if (done_out) TW_CUDA(cudaMemcpyAsync(done_out, done, (size_t)count, cudaMemcpyDeviceToDevice, s));
+  return 0;
+}
+
+extern "C" size_t twowl_tail_negative_sample_workspace_bytes(int64_t n_edges, int64_t P, int64_t k) {
+  const int64_t count = (P > 0 && k > 0) ? P * k : 0;
+  return twowl_nonedge_sample_workspace_bytes(n_edges, count);
+}
+
+extern "C" int twowl_tail_negative_sample(const int64_t* row, int64_t s_row, const int64_t* col, int64_t s_col, int64_t n_edges,
+                                          int64_t num_nodes, const int64_t* src, int64_t P, int64_t k, uint64_t seed, int32_t rounds,
+                                          int64_t* out, int32_t* unresolved, void* ws, size_t ws_bytes, void* stream) {
+  TW_CHECK_ARG(n_edges >= 0 && P >= 0 && k >= 1 && num_nodes > 0 && rounds > 0, "tail_negative_sample: bad sizes");
+  TW_CHECK_ARG(P < 0x7fffffffLL && k < 0x7fffffffLL && P * k < 0x7fffffffLL && num_nodes < (1LL << 31),
+               "tail_negative_sample: P * k and num_nodes must be below 2^31");
+  TW_CHECK_ARG(unresolved != nullptr && (P == 0 || (src && out)) && (n_edges == 0 || (row && col)),
+               "tail_negative_sample: null pointer");
+  TW_CHECK_WS(ws_bytes, twowl_tail_negative_sample_workspace_bytes(n_edges, P, k));
+  cudaStream_t s = (cudaStream_t)stream;
+  TW_CUDA(cudaMemsetAsync(unresolved, 0, sizeof(int32_t), s));
+  const int64_t count = P * k;
+  if (count == 0) return 0;
+  const uint64_t cap = smp_capacity(n_edges, count), mask = cap - 1;
+  Carver c(ws);
+  long long* keys = c.take<long long>(cap);
+  int* owners = c.take<int>(cap);
+  long long* cand = c.take<long long>((size_t)count);
+  uint8_t* done = c.take<uint8_t>((size_t)count);
+  TW_CUDA(cudaMemsetAsync(keys, 0xFF, cap * sizeof(long long), s));
+  TW_CUDA(cudaMemsetAsync(owners, 0x7F, cap * sizeof(int), s));
+  TW_CUDA(cudaMemsetAsync(done, 0, (size_t)count, s));
+  TW_CUDA(cudaMemsetAsync(out, 0xFF, (size_t)count * sizeof(int64_t), s));     // -1 = unfilled
+  if (n_edges > 0) {
+    k_smp_insert_edges<<<grid_for(n_edges, kSmpThreads), kSmpThreads, 0, s>>>(row, s_row, col, s_col, n_edges, num_nodes, 1, keys,
+                                                                            owners, mask);
+    TW_LAUNCH_CHECK();
+  }
+  for (int r = 0; r < rounds; ++r) {
+    TW_CUDA(cudaMemsetAsync(unresolved, 0, sizeof(int32_t), s));
+    k_tail_propose<<<grid_for(count, kSmpThreads), kSmpThreads, 0, s>>>(seed, r, count, k, num_nodes, src, done, cand, keys, owners, mask);
+    k_smp_resolve<<<grid_for(count, kSmpThreads), kSmpThreads, 0, s>>>(count, num_nodes, done, cand, keys, owners, mask, nullptr, out,
+                                                                       unresolved);
+    TW_LAUNCH_CHECK();
+  }
   return 0;
 }

@@ -244,6 +244,35 @@ def sample_non_edges(row: torch.Tensor, col: torch.Tensor, num_nodes: int, count
     return out_row, out_col
 
 
+def sample_tail_negatives(row: torch.Tensor, col: torch.Tensor, num_nodes: int, src: torch.Tensor, k: int,
+                          seed: Optional[int] = None, rounds: int = 16) -> torch.Tensor:
+    """k distinct negatives per source for ranking evaluation -> int64 [P, k]: row i is uniform over the nodes w != src[i] such that
+    neither (src[i], w) nor (w, src[i]) is an edge (row[e], col[e]) - OGB's filtered setting when the edges are every known
+    positive. Deterministic under `seed` (drawn from torch's default generator when None). One host read: raises ValueError if a
+    row could not be filled, i.e. a source has fewer than k allowed nodes (or is adjacent to nearly all of them: more `rounds`)."""
+    _need_cuda(row, col, src)
+    row, col = row.reshape(-1), col.reshape(-1)
+    assert row.dtype == torch.int64 and col.dtype == torch.int64 and row.numel() == col.numel()
+    src = src.reshape(-1).to(torch.int64).contiguous()
+    dev = src.device
+    n_edges, P, k = row.numel(), src.numel(), int(k)
+    out = torch.empty((P, k), dtype=torch.int64, device=dev)
+    unresolved = torch.empty(1, dtype=torch.int32, device=dev)
+    if seed is None:
+        seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+    nb = lib.twowl_tail_negative_sample_workspace_bytes(n_edges, P, k)
+    ws = _ws(nb, dev)
+    (pr, sr), (pc, sc) = (_row(row), _row(col)) if n_edges else ((0, 1), (0, 1))
+    check(lib.twowl_tail_negative_sample(pr, sr, pc, sc, n_edges, int(num_nodes), src.data_ptr(), P, k, int(seed), int(rounds),
+                                         out.data_ptr(), unresolved.data_ptr(), ws.data_ptr(), nb, _stream()), "tail_negative_sample")
+    _count(1 + 2 * int(rounds))
+    left = int(unresolved.item())
+    if left:
+        raise ValueError(f"sample_tail_negatives: {left} of {P * k} slots unfilled after {int(rounds)} rounds - a source has fewer "
+                         f"than k={k} allowed nodes, lies outside [0, {int(num_nodes)}), or needs more rounds")
+    return out
+
+
 def select_columns(mat: torch.Tensor, mask: torch.Tensor, mode: int) -> torch.Tensor:
     """Order-preserving column selection of an int64 [2,T] matrix (any strides).
     mode 0: keep column t iff !mask[t]; mode 1: keep iff !mask[mat[0,t]]."""
@@ -1106,4 +1135,54 @@ def auc(score: torch.Tensor, label: torch.Tensor) -> torch.Tensor:
     ws = _ws(nb, score.device)
     check(lib.twowl_auc(score.data_ptr(), label.data_ptr(), n, out.data_ptr(), ws.data_ptr(), nb, _stream()), "auc")
     _count(4 + 3 * 4)
+    return out
+
+
+RANK_MAX_K = 16   # TWOWL_RANK_MAX_K of include/twowl.h
+
+
+def _rank_ks(ks):
+    """The cut-off list as the host int64 array the ranking entry points take."""
+    ks = [int(k) for k in ks]
+    if not 1 <= len(ks) <= RANK_MAX_K or min(ks) < 1:
+        raise ValueError(f"ks must hold 1..{RANK_MAX_K} cut-offs, each >= 1: {ks}")
+    return (ctypes.c_int64 * len(ks))(*ks), len(ks)
+
+
+def hits_at_k(score: torch.Tensor, label: torch.Tensor, ks) -> torch.Tensor:
+    """Hits@K against a shared negative set on the device, OGB's _eval_hits (ogbl-collab, ogbl-ddi) -> float64[len(ks) + 2] =
+    (hits@K for each K, n_pos, n_neg), no host sync. hits@K = fraction of the positives (label > 0.5) scored strictly above the
+    K-th largest negative; 1.0 when there are fewer than K negatives; NaN when there is no positive or any score is NaN."""
+    _need_cuda(score, label)
+    score = score.detach().reshape(-1).float().contiguous()
+    label = label.detach().reshape(-1).float().contiguous()
+    n = score.numel()
+    assert label.numel() == n, "hits_at_k: score / label size mismatch"
+    h_ks, n_k = _rank_ks(ks)
+    out = torch.empty(n_k + 2, dtype=torch.float64, device=score.device)
+    nb = lib.twowl_hits_at_k_workspace_bytes(n)
+    ws = _ws(nb, score.device)
+    check(lib.twowl_hits_at_k(score.data_ptr(), label.data_ptr(), n, h_ks, n_k, out.data_ptr(), ws.data_ptr(), nb, _stream()),
+          "hits_at_k")
+    _count(5 + 3 * 4)
+    return out
+
+
+def rank_metrics(pos: torch.Tensor, neg: torch.Tensor, ks) -> torch.Tensor:
+    """MRR and hits@k of each positive against its own negatives on the device, OGB's _eval_mrr (ogbl-citation2): pos [P],
+    neg [P, k] -> float64[len(ks) + 2] = (MRR, hits@k for each k, P), no host sync. A positive's rank is 1 + the number of its
+    negatives scored above it, ties counting half; NaN when P = 0 or any score is NaN. Two runs give the same bits."""
+    _need_cuda(pos, neg)
+    pos = pos.detach().reshape(-1).float().contiguous()
+    P = pos.numel()
+    assert neg.dim() == 2 and neg.shape[0] == P and neg.shape[1] >= 1, "rank_metrics: neg must be [P, k], k >= 1"
+    k = neg.shape[1]
+    neg = neg.detach().float().contiguous()
+    h_ks, n_k = _rank_ks(ks)
+    out = torch.empty(n_k + 2, dtype=torch.float64, device=pos.device)
+    nb = lib.twowl_rank_metrics_workspace_bytes(P)
+    ws = _ws(nb, pos.device)
+    check(lib.twowl_rank_metrics(pos.data_ptr(), neg.data_ptr(), P, k, h_ks, n_k, out.data_ptr(), ws.data_ptr(), nb, _stream()),
+          "rank_metrics")
+    _count(3)
     return out
