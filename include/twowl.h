@@ -482,6 +482,38 @@ size_t twowl_rank_metrics_workspace_bytes(int64_t P);
 int twowl_rank_metrics(const float* pos, const float* neg, int64_t P, int64_t k, const int64_t* h_ks, int32_t n_k, double* out,
                        void* ws, size_t ws_bytes, void* stream);
 
+/* ------------------------------------------------------------------ link-prediction heuristics -- */
+
+/* The edge list (row, col) (int64[n_edges] each, element strides) read as an undirected simple graph:
+ * N(x) = {y != x : (x, y) or (y, x) is an edge}. Out: ptr (int64[num_nodes+1]; ptr[num_nodes] = nnz) and adj (int32, capacity
+ * 2 * n_edges; the first nnz entries used), every row sorted ascending with no duplicates or self loops. bad[0] (int32, zeroed by
+ * the call) = the number of endpoints outside [0, num_nodes); such edges are dropped. The caller reads nnz and bad together.
+ * n_edges < 2^30, num_nodes < 2^31 - 1. */
+size_t twowl_simple_adjacency_workspace_bytes(int64_t n_edges);
+int twowl_simple_adjacency(const int64_t* row, int64_t s_row, const int64_t* col, int64_t s_col, int64_t n_edges, int64_t num_nodes,
+                           int64_t* ptr, int32_t* adj, int32_t* bad, void* ws, size_t ws_bytes, void* stream);
+
+/* Neighbourhood heuristics of query pairs (u[i], v[i]) (int64[P] each, element strides) over a simple adjacency (ptr, adj) of
+ * twowl_simple_adjacency, in two calls with one host read between them:
+ *   twowl_link_plan:       chunk_off (int64[P+1]) = exclusive scan of the chunks of each pair: a pair whose probe count
+ *                          w = min(d(u), d(v)) exceeds TWOWL_HEUR_LONG is cut into ceil(w / TWOWL_HEUR_CHUNK) chunks;
+ *                          info (int64[3], device) = (ids outside [0, num_nodes), chunks, total probes over the valid pairs).
+ *   twowl_link_heuristics: out (fp32[4*P]) = rows cn, jaccard, aa, ra, with c = |N(u) ∩ N(v)|:
+ *                          cn = c; jaccard = c / (d(u) + d(v) - c) as an fp32 quotient, 0 when the denominator is 0;
+ *                          aa = sum over the common w of 1 / ln d(w) (0 for d(w) <= 1); ra = sum of 1 / d(w); aa and ra summed
+ *                          in double and rounded once. A pair with an id outside [0, num_nodes) gets NaN. n_chunks = info[1],
+ *                          which sizes the workspace (the chunks' partial sums).
+ * Bitwise repeatable (no floating-point atomics), and score(u, v) == score(v, u) bit for bit. P < 2^31; adj may be NULL when nnz = 0. */
+#define TWOWL_HEUR_LONG 64
+#define TWOWL_HEUR_CHUNK 64
+size_t twowl_link_plan_workspace_bytes(int64_t P);
+int twowl_link_plan(const int64_t* ptr, int64_t num_nodes, const int64_t* u, int64_t s_u, const int64_t* v, int64_t s_v, int64_t P,
+                    int64_t* chunk_off, int64_t* info, void* ws, size_t ws_bytes, void* stream);
+size_t twowl_link_heuristics_workspace_bytes(int64_t n_chunks);
+int twowl_link_heuristics(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* u, int64_t s_u, const int64_t* v,
+                          int64_t s_v, int64_t P, const int64_t* chunk_off, int64_t n_chunks, float* out, void* ws, size_t ws_bytes,
+                          void* stream);
+
 /* ------------------------------------------------------------------ structured wedge path ------- */
 
 /* When ei2 is the full wedge join of (pos_edge, pred_edge) minus the wedges whose source edge is blocked

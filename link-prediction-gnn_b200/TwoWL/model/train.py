@@ -118,17 +118,40 @@ def test_ranking(mod, dataset, ks=(20, 50, 100)):
     mod.eval()
     n_edges = dataset.ei.shape[1]
     targets = n_edges + torch.arange(dataset.y.shape[0], device=dataset.x.device)
-    logits = mod(dataset.x, dataset.ei, dataset.pos1, targets, dataset.ei2, True).reshape(-1)
+    logits = mod(dataset.x, dataset.ei, dataset.pos1, targets, dataset.ei2, True)
+    return rank_scores(logits, dataset, ks)
+
+
+@torch.no_grad()
+def rank_scores(scores, dataset, ks=(20, 50, 100)):
+    """The ranking half of test_ranking for any score of the dataset's prediction pairs - one per undirected pair, in the order
+    of test(): a model's logits, or a heuristic of heuristic_scores(dataset). Same dict and protocols as test_ranking."""
+    logits = scores.reshape(-1)
     ks = [int(k) for k in ks]
     k = getattr(dataset, "rank_k", None)
     if k is not None:
         P = logits.numel() // (1 + int(k))
-        assert P * (1 + int(k)) == logits.numel(), "test_ranking: the logits do not have the [P | P x rank_k] layout"
+        assert P * (1 + int(k)) == logits.numel(), "rank_scores: the scores do not have the [P | P x rank_k] layout"
         vals = ops.rank_metrics(logits[:P], logits[P:].reshape(P, int(k)), ks).cpu()
         return {"mrr": float(vals[0]), **{f"hits@{kk}": float(v) for kk, v in zip(ks, vals[1:1 + len(ks)].tolist())}}
     labels = dataset.y.reshape(-1)[0::2][: logits.shape[0]]
     vals = ops.hits_at_k(logits, labels, ks).cpu()
     return {f"hits@{kk}": float(v) for kk, v in zip(ks, vals[:len(ks)].tolist())}
+
+
+@torch.no_grad()
+def heuristic_scores(dataset):
+    """Neighbourhood link-prediction heuristics of the dataset's prediction pairs (extension: the baselines OGB's leaderboards
+    list) -> {"cn", "jaccard", "aa", "ra"}: fp32 [P] each, one score per undirected pair pos1[E::2] in the order of test() /
+    test_ranking(), P = y.shape[0] // 2. The graph is the split's message-passing graph dataset.ei read as undirected and
+    simple (twowl_b200.graph.simple_adjacency, built once per edge tensor); scores are computed on the device
+    (ops.link_heuristics). rank_scores(heuristic_scores(ds)["aa"], ds) then ranks a heuristic like a model."""
+    from twowl_b200 import graph
+    n_edges = dataset.ei.shape[1]
+    ptr, adj = graph.simple_adjacency(dataset.ei, dataset.x.shape[0])
+    pairs = dataset.pos1[n_edges::2][: dataset.y.shape[0] // 2]
+    scores = ops.link_heuristics(ptr, adj, pairs[:, 0], pairs[:, 1])
+    return dict(zip(ops.HEURISTICS, scores.unbind(0)))
 
 
 def _record_run(record_dir, dsname, tst_score, seconds, fpr, tpr):

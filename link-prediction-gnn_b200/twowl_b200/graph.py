@@ -120,6 +120,15 @@ def node_graph(edge1, n: int, _base: bool = False) -> NodeGraph:
     return (_cache if _base else _step_cache).get(edge1, ("node", n), build)
 
 
+def simple_adjacency(ei: torch.Tensor, n: int):
+    """(ptr, adj) of ops.simple_adjacency for an int64 [2,E] edge tensor - the undirected simple graph the link heuristics
+    intersect - cached per tensor, so that several heuristics or tables over one split build it once."""
+    def build():
+        e = _i64(ei)
+        return ops.simple_adjacency(e[0], e[1], n)
+    return _cache.get(ei, ("simple", n), build)
+
+
 # ------------------------------------------------------------------------------ pair table (pos)
 
 @dataclass

@@ -1186,3 +1186,62 @@ def rank_metrics(pos: torch.Tensor, neg: torch.Tensor, ks) -> torch.Tensor:
           "rank_metrics")
     _count(3)
     return out
+
+
+# ------------------------------------------------------------------------------ link-prediction heuristics
+
+HEURISTICS = ("cn", "jaccard", "aa", "ra")   # the rows of link_heuristics
+
+
+def simple_adjacency(row: torch.Tensor, col: torch.Tensor, num_nodes: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The edges (row[e], col[e]) as an undirected simple graph -> (ptr int64 [N+1], adj int32 [nnz]): N(x) = adj[ptr[x]:ptr[x+1]]
+    = every y != x joined to x by an edge in either direction, sorted ascending, each once. One host read (nnz and the bad-id
+    count together); raises ValueError when an endpoint lies outside [0, num_nodes)."""
+    _need_cuda(row, col)
+    row, col = row.reshape(-1), col.reshape(-1)
+    assert row.dtype == torch.int64 and col.dtype == torch.int64 and row.numel() == col.numel(), \
+        "simple_adjacency: row / col must be int64 of one length"
+    dev, E, n = row.device, row.numel(), int(num_nodes)
+    ptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    adj = torch.empty(max(2 * E, 1), dtype=torch.int32, device=dev)
+    bad = torch.empty(1, dtype=torch.int32, device=dev)
+    nb = lib.twowl_simple_adjacency_workspace_bytes(E)
+    ws = _ws(nb, dev)
+    (pr, sr), (pc, sc) = (_row(row), _row(col)) if E else ((0, 1), (0, 1))
+    check(lib.twowl_simple_adjacency(pr, sr, pc, sc, E, n, ptr.data_ptr(), adj.data_ptr(), bad.data_ptr(), ws.data_ptr(), nb,
+                                     _stream()), "simple_adjacency")
+    _count(6 + 2 * 3 * 3)
+    nnz, nbad = torch.cat((ptr[n:], bad.to(torch.int64))).tolist()
+    if nbad:
+        raise ValueError(f"simple_adjacency: {nbad} edge endpoint(s) outside [0, {n})")
+    return ptr, adj[:nnz].clone()
+
+
+def link_heuristics(ptr: torch.Tensor, adj: torch.Tensor, u: torch.Tensor, v: torch.Tensor) -> torch.Tensor:
+    """Neighbourhood scores of the query pairs (u[i], v[i]) over a simple adjacency (simple_adjacency) -> fp32 [4, P], rows in
+    HEURISTICS order: common neighbours c = |N(u) ∩ N(v)|, Jaccard c / (d(u) + d(v) - c) (0 when that is 0), Adamic-Adar
+    sum 1 / ln d(w) (terms with d(w) <= 1 count 0) and resource allocation sum 1 / d(w) over the common neighbours w. Bitwise
+    repeatable and symmetric in (u, v). One host read; raises IndexError when a query id lies outside [0, N)."""
+    _need_cuda(ptr, adj, u, v)
+    assert ptr.dim() == 1 and ptr.dtype == torch.int64 and ptr.is_contiguous(), "link_heuristics: ptr must be contiguous int64 [N+1]"
+    assert adj.dim() == 1 and adj.dtype == torch.int32 and adj.is_contiguous(), "link_heuristics: adj must be contiguous int32"
+    u, v = u.reshape(-1).to(torch.int64), v.reshape(-1).to(torch.int64)
+    assert u.numel() == v.numel(), "link_heuristics: u / v size mismatch"
+    dev, n, P = ptr.device, ptr.numel() - 1, u.numel()
+    (pu, su), (pv, sv) = (_row(u), _row(v)) if P else ((0, 1), (0, 1))
+    chunk_off = torch.empty(P + 1, dtype=torch.int64, device=dev)
+    info = torch.empty(3, dtype=torch.int64, device=dev)
+    nb = lib.twowl_link_plan_workspace_bytes(P)
+    ws = _ws(nb, dev)
+    check(lib.twowl_link_plan(ptr.data_ptr(), n, pu, su, pv, sv, P, chunk_off.data_ptr(), info.data_ptr(), ws.data_ptr(), nb,
+                              _stream()), "link_plan")
+    nbad, n_chunks, _ = info.tolist()
+    if nbad:
+        raise IndexError(f"link_heuristics: {nbad} query id(s) outside [0, {n})")
+    out = torch.empty((4, P), dtype=torch.float32, device=dev)
+    nb = lib.twowl_link_heuristics_workspace_bytes(n_chunks)
+    ws = _ws(nb, dev)
+    check(lib.twowl_link_heuristics(ptr.data_ptr(), adj.data_ptr(), n, pu, su, pv, sv, P, chunk_off.data_ptr(), n_chunks,
+                                    out.data_ptr(), ws.data_ptr(), nb, _stream()), "link_heuristics")
+    _count(5 + 2)
+    return out
