@@ -417,16 +417,11 @@ typedef struct twowl_conv_args {
   float* stats;               /* [2*Nd] or NULL */
   const float* mean_scale;    /* [Nd], needed with stats */
   float eps;
-  int32_t dual;               /* 1: TWO layers over the same A in one pass (both directions of model.py:77): nsrc = 1, Nd = 2*C,
-                                 W[0] = [W_f; W_r] stacked ([2C, Kd], w_kn = 0), bias / mean_scale / stats / moments 2C wide; output
-                                 columns [0,C) use row_scale[0], gather 0 and go to out[M,C]; columns [C,2C) use row_scale[1],
-                                 gather 1 and go to out2[M,C]; the gathered tables are [rows, C]. A is read once. C % 32 == 0. */
-  float* out2;                /* [M, Nd/2], dual launches */
   double* moments;            /* [2*Nd] or NULL (needs stats): the raw column (sum, sum of squares) of `out` over this call's
                                  M rows - what a row-sharded caller sums over ranks before twowl_graphnorm_stats_from_moments */
   int32_t pair_sum_out;       /* 1: `out` is [M/2, Nd] and holds result[2k] + result[2k+1] - rows 2k / 2k+1 are the two directions
                                  of one pair (utils.py:81-90) and the pair-init backward (model.py:75) only consumes their sum
-                                 (twowl_seg_args.pair_sum = 2). M even, ngather = 2, no stats, no dual. */
+                                 (twowl_seg_args.pair_sum = 2). M even, ngather = 2, no stats. */
 } twowl_conv_args;
 int twowl_pair_conv_supported(int32_t Kd, int32_t Nd, int32_t nsrc);
 size_t twowl_pair_conv_workspace_bytes(int64_t M, int32_t Nd);

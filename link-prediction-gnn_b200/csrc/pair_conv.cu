@@ -53,8 +53,6 @@ struct ConvParams {
   int ngather;
   const float* bias;
   float* out;
-  float* out2;         // dual: the second direction's output
-  int dual;            // 0, or Nd/2: columns [0, dual) and [dual, Nd) are two layers sharing A (row scale / gather / output d)
   int group;           // K-slabs per pipeline stage (1 or 2)
   double* stats_part;  // [gridDim.x][2][Nsub] column (sum, sum of squares) of this CTA's window of `out`, or NULL
   int tmem_cols;
@@ -169,7 +167,7 @@ struct PcRing {
 // tile run side by side, so the re-reads of its A slabs are L2 hits.
 // PSUM (compile time, its own instantiation - a runtime flag changed the register allocation of every other one and cost the
 // forward launches 1 ms each): out has M/2 rows, out[k] = result[2k] + result[2k+1]
-template <int NG, bool DUAL, bool PSUM = false>
+template <int NG, bool PSUM = false>
 __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
                                                              const __grid_constant__ CUtensorMap tmA1) {
   extern __shared__ uint8_t pc_smem_raw[];
@@ -429,28 +427,25 @@ __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p,
 #pragma unroll
       for (int s = 0; s < 2; ++s) {
         const float* __restrict__ rsv = s ? p.rs[1] : p.rs[0];
-        rss[s] = ((s < p.nsrc || DUAL) && rsv && myrow < p.M) ? __ldg(rsv + myrow) : 1.f;
+        rss[s] = (s < p.nsrc && rsv && myrow < p.M) ? __ldg(rsv + myrow) : 1.f;
       }
     };
     auto load_idx = [&](int64_t tile_, int (&ixx)[NGA][8], float (&cff)[NGA][8], float (&rss)[2]) {
       load_ix(tile_, ixx);
       load_cf(tile_, cff, rss);
     };
-    // dual: the 32-column block belongs to direction dd = (first column >= dual); only that direction's table is gathered,
-    // from its own column range, and the tables / outputs are dual columns wide.
-    const int pdual = DUAL ? p.dual : 0;   // compile-time zero in the single-direction instantiations
-    const int Tld = DUAL ? pdual : Nd;
+    // row stride of the gathered tables and of `out`; a variable of its own because the lambdas capture it: writing Nd in its
+    // place changes the register allocation of the three non-PSUM instantiations
+    const int Tld = Nd;
     auto gather = [&](const int (&ixx)[NGA][8], int c0_, float4 (&g4)[NGA][8]) {
       const int lcol_ = c0_ + lchunk * 4, col_ = n0 + lcol_;
       const bool ok = lcol_ < Nsub && col_ < Nd;
-      const int dd = (DUAL && n0 + c0_ >= pdual) ? 1 : 0;
-      const int tcol = col_ - dd * pdual;
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
 #pragma unroll
         for (int g = 0; g < NGA; ++g) {
-          g4[g][i] = (NG > g && ixx[g][i] >= 0 && ok && (!DUAL || g == dd))
-                         ? pc_ldg_keep(reinterpret_cast<const float4*>(p.T[g] + (size_t)ixx[g][i] * Tld + tcol), keep_policy) : f4_zero();
+          g4[g][i] = (NG > g && ixx[g][i] >= 0 && ok)
+                         ? pc_ldg_keep(reinterpret_cast<const float4*>(p.T[g] + (size_t)ixx[g][i] * Tld + col_), keep_policy) : f4_zero();
         }
       }
     };
@@ -466,7 +461,6 @@ __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p,
         const int lcol = c0 + lchunk * 4;        // column inside this CTA's window
         const int col = n0 + lcol;               // column of `out`
         const bool cok = lcol < Nsub && col < Nd;
-        const int dd = (DUAL && n0 + c0 >= pdual) ? 1 : 0;   // direction of this column block (dual launches)
         // gathered rows first: they do not depend on the accumulator, so their latency hides behind the wait for it
         gather(ix, c0, gv);
         if (!waited) {
@@ -486,7 +480,7 @@ __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p,
           pc_tmem_wait_ld();
           float o[8];
 #pragma unroll
-          for (int e = 0; e < 8; ++e) o[e] = (dd ? rsc[1] : rsc[0]) * __uint_as_float(v0[e]);
+          for (int e = 0; e < 8; ++e) o[e] = rsc[0] * __uint_as_float(v0[e]);
           if (p.nsrc > 1) {
 #pragma unroll
             for (int e = 0; e < 8; ++e) o[e] = fmaf(rsc[1], __uint_as_float(v1[e]), o[e]);
@@ -506,7 +500,7 @@ __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p,
           if (live) {
 #pragma unroll
             for (int g = 0; g < NGA; ++g)
-              if (NG > g && (!DUAL || g == dd)) f4_fma(o, cf[g][i], gv[g][i]);
+              if (NG > g) f4_fma(o, cf[g][i], gv[g][i]);
             f4_add(o, bias4);
           }
           if constexpr (PSUM) {
@@ -522,7 +516,7 @@ __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p,
             }
           } else if (live) {
             // written once, read by a later kernel: evict first
-            __stcs(reinterpret_cast<float4*>((dd ? p.out2 : p.out) + row * Tld + (col - dd * pdual)), o);
+            __stcs(reinterpret_cast<float4*>(p.out + row * Tld + col), o);
             f4_add(bsum, o);
             bsq.x = fmaf(o.x, o.x, bsq.x), bsq.y = fmaf(o.y, o.y, bsq.y), bsq.z = fmaf(o.z, o.z, bsq.z), bsq.w = fmaf(o.w, o.w, bsq.w);
           }
@@ -598,19 +592,6 @@ __global__ void k_pc_stats_final(const double* __restrict__ part, int nparts, in
   stats[C + c] = (float)(1.0 / sqrt(var + (1.0 - a) * (1.0 - a) * mean * mean + (double)eps));
 }
 
-// tuning knobs from the environment (TWOWL_PC_STAGES, TWOWL_PC_NSPLIT), read ONCE per process - not on every launch
-struct PcEnv {
-  int stages = 0, nsplit = 0;
-  PcEnv() {
-    if (const char* e = getenv("TWOWL_PC_STAGES")) stages = atoi(e);
-    if (const char* e = getenv("TWOWL_PC_NSPLIT")) nsplit = atoi(e);
-  }
-};
-static const PcEnv& pc_env() {
-  static const PcEnv env;
-  return env;
-}
-
 // How one launch is cut: column windows of Nsub (multiple of 16) output columns per CTA, raw / lo ring depths.
 struct PcConfig {
   int nsplit = 0, Nsub = 0, stages = 0, lo_stages = 0, tmem_cols = 0, group = kPcGroup;
@@ -629,13 +610,12 @@ static int pc_tmem_cols(int Nsub, int nsrc) {
 }
 // Fewest column windows that fit at all: every extra window re-reads (and re-splits) the whole A tile, which costs far more than
 // a shallower ring (measured at C = 128, M = 15 M: 2 windows with 2 raw stages 5.3 ms, 4 windows with 3 stages 8.2 ms, 8 windows
-// 15.2 ms). The ring is then grown to what the remaining shared memory holds. force_nsplit > 0 pins the split (tuning / tests).
-static PcConfig pc_config(int Kd, int Nd, int nsrc, bool with_stats, int force_nsplit = 0) {
+// 15.2 ms). The ring is then grown to what the remaining shared memory holds.
+static PcConfig pc_config(int Kd, int Nd, int nsrc, bool with_stats) {
   PcConfig best;
   if (Kd < 4 || Kd > 1024 || (Kd % 4) || Nd < 4 || Nd > 1024 || (Nd % 4) || nsrc < 1 || nsrc > 2) return best;
   const size_t cap = 227 * 1024;
   for (int ns = 1; ns <= 32 && !best.nsplit; ns *= 2) {
-    if (force_nsplit > 0 && ns != force_nsplit) continue;
     const int Nsub = (int)(cdiv(cdiv(Nd, ns), 16) * 16);
     if (Nsub > 256 || (ns > 1 && (int64_t)(ns - 1) * Nsub >= Nd)) continue;
     if (pc_tmem_cols(Nsub, nsrc) > 512) continue;
@@ -646,14 +626,12 @@ static PcConfig pc_config(int Kd, int Nd, int nsrc, bool with_stats, int force_n
       if (pc_smem_bytes(Kd, Nsub, nsrc, with_stats, st, lo, grp) > cap) continue;
     }
     while (st < kPcMaxStages && pc_smem_bytes(Kd, Nsub, nsrc, with_stats, st + 1, lo, grp) <= cap) ++st;
-    if (pc_env().stages > 0) st = pc_env().stages < st ? (pc_env().stages < 2 ? 2 : pc_env().stages) : st;   // tuning knob
     best.nsplit = ns, best.Nsub = Nsub, best.stages = st, best.lo_stages = lo, best.group = grp;
     best.tmem_cols = pc_tmem_cols(Nsub, nsrc);
     best.smem = pc_smem_bytes(Kd, Nsub, nsrc, with_stats, st, lo, grp);
   }
   return best;
 }
-static int pc_force_nsplit() { return pc_env().nsplit; }
 static bool pc_supported(int Kd, int Nd, int nsrc) { return pc_config(Kd, Nd, nsrc, nsrc == 1).nsplit > 0; }
 static int pc_grid(int64_t M, int nsplit) {
   const int64_t ntiles = cdiv(M, kPcTileM);
@@ -667,10 +645,10 @@ static int pc_make_tmap(CUtensorMap* tm, const float* A, int64_t M, int Kd) {
   return make_tmap_2d_f32(tm, A, M, Kd, 32, kPcTileM, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-template <int NG, bool DUAL = false, bool PSUM = false>
+template <int NG, bool PSUM = false>
 static int pc_launch(const ConvParams& p, size_t smem, const CUtensorMap& t0, const CUtensorMap& t1, cudaStream_t s) {
-  TW_CUDA(cudaFuncSetAttribute(k_pair_conv<NG, DUAL, PSUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_pair_conv<NG, DUAL, PSUM><<<pc_grid(p.M, p.nsplit), kPcThreads, smem, s>>>(p, t0, t1);
+  TW_CUDA(cudaFuncSetAttribute(k_pair_conv<NG, PSUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_pair_conv<NG, PSUM><<<pc_grid(p.M, p.nsplit), kPcThreads, smem, s>>>(p, t0, t1);
   TW_LAUNCH_CHECK();
   return 0;
 }
@@ -707,7 +685,7 @@ extern "C" int twowl_pair_conv(const twowl_conv_args* a, void* ws, size_t ws_byt
   TW_CHECK_ARG(a != nullptr && a->nsrc >= 1 && a->nsrc <= 2 && a->ngather >= 0 && a->ngather <= 2, "pair_conv: bad nsrc/ngather");
   TW_CHECK_ARG(a->M >= 0, "pair_conv: negative M");
   const bool want_stats = a->stats != nullptr;
-  const PcConfig cfg = pc_config(a->Kd, a->Nd, a->nsrc, want_stats, pc_force_nsplit());
+  const PcConfig cfg = pc_config(a->Kd, a->Nd, a->nsrc, want_stats);
   TW_CHECK_ARG(cfg.nsplit > 0, "pair_conv: Kd=%d Nd=%d nsrc=%d%s unsupported (widths %% 4, <= 1024, shared memory)", a->Kd, a->Nd,
                a->nsrc, want_stats ? " with statistics" : "");
   ConvParams p;
@@ -721,15 +699,9 @@ extern "C" int twowl_pair_conv(const twowl_conv_args* a, void* ws, size_t ws_byt
     p.T[g] = a->T[g], p.tidx[g] = a->tidx[g], p.tcoef[g] = a->tcoef[g];
   }
   TW_CHECK_ARG(aligned16(a->out) && aligned16(a->bias), "pair_conv: out/bias must be 16-byte aligned");
-  if (a->dual) {
-    TW_CHECK_ARG(a->nsrc == 1 && a->ngather == 2 && a->Nd % 64 == 0 && a->out2 && aligned16(a->out2) && a->row_scale[0] && a->row_scale[1],
-                 "pair_conv: a dual launch needs one source, two gathers, two row scales, out2, and Nd/2 a multiple of 32");
-    p.rs[1] = a->row_scale[1];
-    p.out2 = a->out2, p.dual = a->Nd / 2;
-  }
   if (a->pair_sum_out) {
-    TW_CHECK_ARG(!a->dual && !want_stats && a->M % 2 == 0 && a->ngather == 2,
-                 "pair_conv: pair_sum_out is built for the pair layer's input gradient: two gathers, an even M, no statistics, no dual launch");
+    TW_CHECK_ARG(!want_stats && a->M % 2 == 0 && a->ngather == 2,
+                 "pair_conv: pair_sum_out is built for the pair layer's input gradient: two gathers, an even M, no statistics");
   }
   p.nsrc = a->nsrc, p.ngather = a->ngather, p.M = a->M, p.Kd = a->Kd, p.Nd = a->Nd, p.bias = a->bias, p.out = a->out;
   p.Nsub = cfg.Nsub, p.nsplit = cfg.nsplit, p.stages = cfg.stages, p.lo_stages = cfg.lo_stages, p.tmem_cols = cfg.tmem_cols, p.group = cfg.group;
@@ -746,8 +718,7 @@ extern "C" int twowl_pair_conv(const twowl_conv_args* a, void* ws, size_t ws_byt
     const int rc_t = pc_make_tmap(&tm[i], a->A[i], a->M, a->Kd);
     if (rc_t) return rc_t;
   }
-  const int rc = a->dual           ? pc_launch<2, true>(p, cfg.smem, tm[0], tm[1], s)
-                 : a->pair_sum_out ? pc_launch<2, false, true>(p, cfg.smem, tm[0], tm[1], s)
+  const int rc = a->pair_sum_out   ? pc_launch<2, true>(p, cfg.smem, tm[0], tm[1], s)
                  : a->ngather == 0 ? pc_launch<0>(p, cfg.smem, tm[0], tm[1], s)
                  : a->ngather == 1 ? pc_launch<1>(p, cfg.smem, tm[0], tm[1], s)
                                    : pc_launch<2>(p, cfg.smem, tm[0], tm[1], s);

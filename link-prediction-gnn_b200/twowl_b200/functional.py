@@ -327,13 +327,9 @@ readout.register_autograd(_ro_bwd, setup_context=_ro_setup)
 
 def _pair_convs_fwd(h, pf, pr, SHf, SHr, centre, dinv, selfw, eps):
     """O_d = selfw_d * (h W_d^T) + dinv_d * (SH_d W_d^T)[centre_d] + bias_d and its GraphNorm statistics, both directions:
-    -> [(O_f, stats_f, SH_f), (O_r, stats_r, SH_r)]. One pass over h when the dual launch covers the width."""
+    -> [(O_f, stats_f, SH_f), (O_r, stats_r, SH_r)]."""
     (wf, bf, gmf), (wr, br, gmr) = pf, pr
     Sf, Sr = ops.linear_fwd(SHf, wf), ops.linear_fwd(SHr, wr)
-    if ops.PAIR_CONV_DUAL and wf.shape == wr.shape and ops.pair_conv_dual_supported(h.shape[1], wf.shape[0]):
-        Of, Or, sf, sr = ops.pair_conv_dual(h, wf, wr, selfw[0], selfw[1], (Sf, centre[0], dinv[0]), (Sr, centre[1], dinv[1]), bf, br,
-                                            gmf, gmr, eps)
-        return [(Of, sf, SHf), (Or, sr, SHr)]
     outs = []
     for d, (w, b, gm, S, SH) in enumerate(((wf, bf, gmf, Sf, SHf), (wr, br, gmr, Sr, SHr))):
         O, st = ops.pair_conv([h], [w], [0], row_scale=[selfw[d]], gathers=[(S, centre[d], dinv[d])], bias=b,

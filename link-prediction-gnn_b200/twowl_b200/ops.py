@@ -905,55 +905,6 @@ def pair_conv(A, W, w_kn, *, row_scale=None, gathers=(), bias=None, stats_mean_s
     return out if stats is None else (out, stats)
 
 
-# both directions of a pair layer in one pass over H (twowl_conv_args.dual). Off by default: bit-identical to the two launches
-# and 20 GB less traffic at R-MAT scale, but at 128 output columns every epilogue warp serves two column blocks per tile and the
-# second block's gather latency is exposed: 19.3 ms against 2 x 8.2 ms measured (DESIGN 4)
-PAIR_CONV_DUAL = os.environ.get("TWOWL_PAIR_CONV_DUAL", "0") != "0"
-
-
-def pair_conv_dual_supported(Kd: int, C: int) -> bool:
-    return C % 32 == 0 and bool(lib.twowl_pair_conv_supported(Kd, 2 * C, 1))
-
-
-def pair_conv_dual(A, Wf, Wr, rs_f, rs_r, gather_f, gather_r, bias_f, bias_r, ms_f, ms_r, eps: float = 1e-5, want_moments: bool = False):
-    """Both directions of one pair layer (model.py:77) in ONE pass over A: O_d = rs_d * (A W_d^T) + coef_d * T_d[idx_d] + bias_d
-    and the GraphNorm statistics of both. gather_d = (T_d [rows, C], idx_d int32 [M], coef_d [M]).
-    -> (O_f, O_r, stats_f [2C], stats_r [2C]) or, with want_moments, (O_f, O_r, moments_f, moments_r float64 [2C])."""
-    M, Kd = A.shape
-    C = Wf.shape[0]
-    dev = A.device
-    _need_cuda(A, Wf, Wr)
-    A = A.contiguous()
-    W = torch.cat((Wf, Wr)).contiguous()
-    bias = torch.cat((bias_f, bias_r))
-    ms = torch.cat((ms_f, ms_r))
-    Of = torch.empty((M, C), dtype=torch.float32, device=dev)
-    Or = torch.empty((M, C), dtype=torch.float32, device=dev)
-    a = ConvArgs(nsrc=1, ngather=2, Kd=Kd, Nd=2 * C, M=M, bias=bias.data_ptr(), out=Of.data_ptr(), out2=Or.data_ptr(), dual=1,
-                 eps=float(eps))
-    a.A[0], a.W[0], a.w_kn[0] = A.data_ptr(), W.data_ptr(), 0
-    a.row_scale[0], a.row_scale[1] = rs_f.data_ptr(), rs_r.data_ptr()
-    for g, (T, idx, coef) in enumerate((gather_f, gather_r)):
-        a.T[g], a.tidx[g], a.tcoef[g] = T.data_ptr(), idx.data_ptr(), coef.data_ptr()
-    stats = torch.empty(4 * C, dtype=torch.float32, device=dev)
-    nb = lib.twowl_pair_conv_workspace_bytes(M, 2 * C)
-    ws = _ws(nb, dev)
-    a.stats, a.mean_scale = stats.data_ptr(), ms.data_ptr()
-    moments = None
-    if want_moments:
-        moments = torch.zeros(4 * C, dtype=torch.float64, device=dev)
-        a.moments = moments.data_ptr()
-    nbytes = M * (4 * Kd + 2 * (4 * C + 4 * C + 16))
-    with _P("pair_conv", nbytes):
-        check(lib.twowl_pair_conv(ctypes.byref(a), ws.data_ptr(), nb, _stream()), "pair_conv (dual)")
-    _count(2)
-    if moments is not None:   # [sum(2C) | sumsq(2C)] -> per direction [sum(C) | sumsq(C)]
-        m = moments.view(2, 2, C)
-        return Of, Or, m[:, 0].reshape(-1), m[:, 1].reshape(-1)
-    st = stats.view(2, 2, C)      # [mean(2C) | inv_std(2C)] -> per direction [mean(C) | inv_std(C)]
-    return Of, Or, st[:, 0].reshape(-1), st[:, 1].reshape(-1)
-
-
 def pair_dw_supported(C: int) -> bool:
     return bool(lib.twowl_pair_dw_supported(C))
 

@@ -44,7 +44,6 @@ depth1 >= 1, depth2 >= 1 on the structured wedge path with the doubled pair layo
 """
 from __future__ import annotations
 
-import os
 from dataclasses import dataclass
 from typing import Optional, Tuple
 
@@ -129,7 +128,7 @@ class RowShard:
         self.steps = 0
         # node ranges of the pipelined table exchanges (8 GPUs, R-MAT 1M/16M: 2 ranges 18.5 ms per step, 4 ranges 19.1 ms - every
         # range is three more launches over short lists)
-        self.chunks = int(os.environ.get("TWOWL_ROWSHARD_CHUNKS", "2"))
+        self.chunks = 2
         _last_shard = self
 
     def _account(self, what: str, t: torch.Tensor):
@@ -419,17 +418,12 @@ def _layer_forward(shard, loc, rows, blocked_l, R_total, n_node, eps, H, pf, pr)
                                                              out=SH[1], out2=SH[0], rows=(lo, hi)),
                            (SH[0], SH[1]), "SH [2,N,C]")
     Sf, Sr = ops.linear_fwd(SH[0], wf), ops.linear_fwd(SH[1], wr)
-    if ops.PAIR_CONV_DUAL and ops.pair_conv_dual_supported(H.shape[1], wf.shape[0]):
-        Of, Or, mf, mr = ops.pair_conv_dual(H, wf, wr, selfw[0], selfw[1], (Sf, centre[0], dinv[0]), (Sr, centre[1], dinv[1]), bf, br,
-                                            gmf, gmr, eps, want_moments=True)
-        Os, moms = [Of, Or], [mf, mr]
-    else:
-        Os, moms = [], []
-        for d, (w, b, gm, S) in enumerate(((wf, bf, gmf, Sf), (wr, br, gmr, Sr))):
-            O, mom = ops.pair_conv([H], [w], [0], row_scale=[selfw[d]], gathers=[(S, centre[d], dinv[d])], bias=b,
-                                   stats_mean_scale=gm, eps=eps, want_moments=True)
-            Os.append(O)
-            moms.append(mom)
+    Os, moms = [], []
+    for d, (w, b, gm, S) in enumerate(((wf, bf, gmf, Sf), (wr, br, gmr, Sr))):
+        O, mom = ops.pair_conv([H], [w], [0], row_scale=[selfw[d]], gathers=[(S, centre[d], dinv[d])], bias=b,
+                               stats_mean_scale=gm, eps=eps, want_moments=True)
+        Os.append(O)
+        moms.append(mom)
     mom = shard.all_reduce(torch.stack(moms), "GraphNorm moments [2,2C] f64")
     sf = ops.graphnorm_stats_from_moments(mom[0], R_total, gmf, eps)
     sr = ops.graphnorm_stats_from_moments(mom[1], R_total, gmr, eps)

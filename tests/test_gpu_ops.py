@@ -542,9 +542,10 @@ def test_pair_conv_tcgen05_vs_fp64(U, M, Kd, Nd, nsrc, ngather, stats):
     for w_kn in (1, 0):
         Wd = [c(w) if w_kn else c(w.t()) for w in W]
         ms = torch.rand(Nd) + 0.5
-        res = ops.pair_conv([c(a) for a in A], Wd, [w_kn] * nsrc, row_scale=[c(r) for r in rs],
-                            gathers=[(c(T[g]), idx[g].int().cuda(), c(coef[g])) for g in range(ngather)], bias=c(bias),
-                            stats_mean_scale=ms.cuda() if stats else None, eps=1e-5)
+        args = ([c(a) for a in A], Wd, [w_kn] * nsrc)
+        kw = dict(row_scale=[c(r) for r in rs], gathers=[(c(T[g]), idx[g].int().cuda(), c(coef[g])) for g in range(ngather)],
+                  bias=c(bias), stats_mean_scale=ms.cuda() if stats else None, eps=1e-5)
+        res = ops.pair_conv(*args, **kw)
         out = res[0] if stats else res
         assert_close(out, ref, absum=absum, nterms=nterms, mma=True, what=f"pair_conv out w_kn={w_kn}")
         if stats:
@@ -557,6 +558,11 @@ def test_pair_conv_tcgen05_vs_fp64(U, M, Kd, Nd, nsrc, ngather, stats):
             dvar = 2 * (dev_ * absum).mean(0) + 2 * dev_.mean(0) * ms.double() * absum.mean(0)
             inv = (var + 1e-5).rsqrt()
             assert_close(res[1][Nd:], inv, absum=inv * dvar / (2 * (var + 1e-5)), nterms=nterms, mma=True, what="pair_conv inv_std")
+            # the raw column moments a row-sharded caller sums over ranks
+            _, mom = ops.pair_conv(*args, **kw, want_moments=True)
+            assert_close(mom[:Nd], ref.sum(0), absum=absum.sum(0), nterms=nterms, mma=True, what="pair_conv moment sum")
+            assert_close(mom[Nd:], (ref ** 2).sum(0), absum=(2 * ref.abs() * absum).sum(0), nterms=nterms, mma=True,
+                         what="pair_conv moment sumsq")
 
 
 @pytest.mark.parametrize("M,C", [(2, 64), (126, 32), (130, 64), (40002, 64), (20002, 128), (3002, 24), (9002, 256)])
@@ -610,50 +616,6 @@ def test_pair_conv_statistics_with_a_large_mean(U, ratio, M):
     assert_close(st[:Nd], mean, rtol=1e-6, atol=1e-6, what="mean")
     rel = ((st[Nd:].double().cpu() - inv) / inv).abs().max()
     assert float(rel) <= 1e-5 + ratio ** 2 * 2.0 ** -22, (float(rel), ratio)
-
-
-@pytest.mark.parametrize("M,Kd,C", [(3, 64, 64), (129, 32, 32), (5000, 64, 64), (70001, 64, 64), (30011, 128, 128), (9000, 24, 32),
-                                    (4000, 256, 256)])
-def test_pair_conv_dual_vs_fp64(U, M, Kd, C):
-    """Both directions of a pair layer in one pass over A (twowl_conv_args.dual): outputs, statistics and raw moments of each
-    direction against fp64, and against two single-direction launches."""
-    from twowl_b200 import ops
-    torch.manual_seed(M + C)
-    NT = 777
-    A = r32(torch.randn(M, Kd, dtype=torch.float64))
-    W = [r32(torch.randn(C, Kd, dtype=torch.float64) / Kd ** 0.5) for _ in range(2)]
-    T = [r32(torch.randn(NT, C, dtype=torch.float64)) for _ in range(2)]
-    idx = [torch.randint(0, NT, (M,)) for _ in range(2)]
-    idx[1][::7] = -1                                     # rows without a gathered term
-    coef = [r32(torch.rand(M, dtype=torch.float64)) for _ in range(2)]
-    rs = [r32(torch.rand(M, dtype=torch.float64) * (torch.rand(M) > 0.2)) for _ in range(2)]
-    bias = [r32(torch.randn(C, dtype=torch.float64)) for _ in range(2)]
-    ms = [r32(torch.rand(C, dtype=torch.float64) + 0.5) for _ in range(2)]
-    c = lambda t: t.float().cuda().contiguous()          # noqa: E731
-    ci = lambda t: t.to(torch.int32).cuda()              # noqa: E731
-    assert ops.pair_conv_dual_supported(Kd, C)
-    args = (c(A), c(W[0]), c(W[1]), c(rs[0]), c(rs[1]), (c(T[0]), ci(idx[0]), c(coef[0])), (c(T[1]), ci(idx[1]), c(coef[1])), c(bias[0]),
-            c(bias[1]), c(ms[0]), c(ms[1]))
-    Of, Or, sf, sr = ops.pair_conv_dual(*args)
-    _, _, mf, mr = ops.pair_conv_dual(*args, want_moments=True)
-    for d, (O, st, mom) in enumerate(((Of, sf, mf), (Or, sr, mr))):
-        g = T[d][idx[d].clamp(min=0)] * (idx[d] >= 0).double().unsqueeze(1)
-        ref = rs[d].unsqueeze(1) * (A @ W[d].t()) + coef[d].unsqueeze(1) * g + bias[d]
-        absum = rs[d].unsqueeze(1) * (A.abs() @ W[d].abs().t()) + coef[d].unsqueeze(1) * g.abs() + bias[d].abs()
-        kw = dict(nterms=Kd + 5, mma=True)              # fp32 summation + split-tf32 product bounds over the absolute terms
-        assert_close(O, ref, absum=absum, what=f"dual out {d}", **kw)
-        mean = ref.mean(0)
-        var = ((ref - ms[d] * mean) ** 2).mean(0)
-        assert_close(st[:C], mean, absum=absum.mean(0), what=f"dual mean {d}", **kw)
-        dev_ = (ref - mean * ms[d]).abs()               # first-order propagation of the elements' bounds into inv_std
-        dvar = 2 * (dev_ * absum).mean(0) + 2 * dev_.mean(0) * ms[d] * absum.mean(0)
-        inv = (var + 1e-5).rsqrt()
-        assert_close(st[C:], inv, absum=inv * dvar / (2 * (var + 1e-5)), what=f"dual inv_std {d}", **kw)
-        assert_close(mom[:C], ref.sum(0), absum=absum.sum(0), what=f"dual moment sum {d}", **kw)
-        assert_close(mom[C:], (ref ** 2).sum(0), absum=(2 * ref.abs() * absum).sum(0), what=f"dual moment sumsq {d}", **kw)
-        one, st1 = ops.pair_conv([c(A)], [c(W[d])], [0], row_scale=[c(rs[d])], gathers=[(c(T[d]), ci(idx[d]), c(coef[d]))], bias=c(bias[d]),
-                                 stats_mean_scale=c(ms[d]))
-        assert torch.equal(one, O), f"dual launch differs from the single-direction launch, direction {d}"
 
 
 @pytest.mark.parametrize("M,C", [(1, 64), (63, 32), (64, 64), (65, 64), (5000, 32), (70001, 64), (400000, 64), (1, 128), (33, 128),
