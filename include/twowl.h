@@ -208,7 +208,9 @@ typedef struct twowl_seg_args {
   int64_t long_cap;
   int32_t pair_sum;              /* 1: gather X[s] + X[s ^ 1] (the two directions 2k / 2k+1 of one pair, utils.py:81-90);
                                     2: X has ONE row per pair that already holds that sum (twowl_conv_args.pair_sum_out): gather
-                                    X[s >> 1] - the same terms in the same order, half the rows read */
+                                    X[s >> 1] - the same terms in the same order, half the rows read. With the dual output
+                                    (no X2, no X_mate), 2 means X has ONE row per pair, X[k] = H[2k] = H[2k+1]: entry s loads
+                                    X[s >> 1] once and adds it to both outputs - one 256-byte row where the 2-row block is 512 */
   const uint8_t* entry_mask;     /* indexed by CSR ENTRY k (not by col[k]) or NULL: entries removed from a cached CSR */
   /* dual output (out2 != NULL; plain gather, flip = row_flip = 0): one pass over the 2-row blocks (s, s^1) gives
    *   out[m]  = sum src_scale[s]    * X[s]        (edge2_r's in-list sum of the pair layer, model.py:77)
@@ -243,8 +245,10 @@ int twowl_seg_plan(const int64_t* ptr, int64_t M, int64_t nnz, int32_t* counts /
 int twowl_gather_rows(const float* W, int64_t rows_w, const int64_t* idx, int64_t stride, int64_t n, int32_t C,
                       float* out, void* stream);
 
-/* pair init (model.py:75): out[p] = X[src[p]] * X[dst[p]]. */
-int twowl_pair_init_fwd(const float* X, const int32_t* src, const int32_t* dst, int64_t R, int32_t C, float* out,
+/* pair init (model.py:75): out[p] = X[src[p]] * X[dst[p]], [R, C].
+ * pairs = 1: (src, dst) is a mated table (rows 2k / 2k+1 are (u,v) / (v,u), utils.py:81-90, R even), whose two rows of a pair
+ * have the same product bit for bit (fp32 multiplication commutes): out is [R/2, C], out[k] = X[src[2k]] * X[dst[2k]]. */
+int twowl_pair_init_fwd(const float* X, const int32_t* src, const int32_t* dst, int64_t R, int32_t C, int32_t pairs, float* out,
                         void* stream);
 
 /* readout (model.py:78-83): pred[l] = sum_c H[idx[2l],c] * H[idx[2l+1],c] * w[c] + b.
@@ -422,6 +426,10 @@ typedef struct twowl_conv_args {
   int32_t pair_sum_out;       /* 1: `out` is [M/2, Nd] and holds result[2k] + result[2k+1] - rows 2k / 2k+1 are the two directions
                                  of one pair (utils.py:81-90) and the pair-init backward (model.py:75) only consumes their sum
                                  (twowl_seg_args.pair_sum = 2). M even, ngather = 2, no stats. */
+  int32_t a_pairs;            /* 1: A[0] is [M/2, Kd], ONE row per pair, and output row r uses A row r >> 1 - the pair features
+                                 of the depth-1 pair layer, whose rows 2k / 2k+1 are the same bits (twowl_pair_init_fwd with
+                                 pairs = 1). Everything else (row scales, gathers, bias, out, stats) keeps its M rows. M even,
+                                 nsrc = 1, ngather = 1. */
 } twowl_conv_args;
 int twowl_pair_conv_supported(int32_t Kd, int32_t Nd, int32_t nsrc);
 size_t twowl_pair_conv_workspace_bytes(int64_t M, int32_t Nd);
@@ -446,8 +454,10 @@ int twowl_pair_dw_ld(const float* dOf, const float* dOr, const float* rsf, const
  * pass (2 reads + 2 writes of [M,C]) disappears. ws as twowl_pair_dw. */
 int twowl_pair_dw_gn(const float* Of, const float* Or, const float* consts, const float* G, const int32_t* head,
                      const int32_t* next, float p_drop, uint64_t seed_f, uint64_t seed_r, int32_t relu, const float* rsf,
-                     const float* rsr, const float* H, int64_t M, int32_t C, float* dOf, float* dOr, float* dWf, float* dWr,
-                     void* ws, size_t ws_bytes, void* stream);
+                     const float* rsr, const float* H, int32_t h_pairs, int64_t M, int32_t C, float* dOf, float* dOr, float* dWf,
+                     float* dWr, void* ws, size_t ws_bytes, void* stream);
+/* h_pairs = 1: H is [M/2, C], one row per pair, standing for pair-table rows 2k and 2k+1 (the depth-1 pair layer's H, see
+ * twowl_conv_args.a_pairs). M even. The sums see the same terms in the same order: bit-identical to the full-height H. */
 
 /* ------------------------------------------------------------------ metrics -------------------- */
 

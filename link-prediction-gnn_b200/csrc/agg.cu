@@ -41,7 +41,8 @@ struct SegParams {
   float* out;
   int accumulate;
   int pair_sum;
-  int x_shift;                 // 1: X holds ONE row per pair (already X[2k] + X[2k+1]): entry s gathers X[s >> 1]
+  int x_shift;                 // 1: X holds ONE row per pair: entry s gathers X[s >> 1] (times X2: the row is already
+                               // X[2k] + X[2k+1]; dual: the row is H[2k] = H[2k+1], the two directions' shared pair features)
   const uint8_t* entry_mask;
   // dual mode (MODE & 4): one pass over the 2-row blocks (s, s^1) feeds TWO outputs: out += src_scale[s] * X[s],
   // out2 += src_scale2[s^1] * X[s^1] - both directions of the pair layer's in-list sum, H read as 512-byte blocks
@@ -94,7 +95,8 @@ struct GroupCtx {
 // Software-pipelined two blocks deep so that no load is consumed in the iteration that issues it: while block b is
 // gathered and accumulated, the col entries of block b+2 and the (col-dependent) scale / second-factor indices of
 // block b+1 are in flight.
-// MODE: 0 = plain gather, 1 = times X2[mul_idx], 3 = (X[s] + X[s^1]) times X2[mul_idx], 4 = dual (X[s] -> acc, X[s^1] -> acc2)
+// MODE: 0 = plain gather, 1 = times X2[mul_idx], 3 = (X[s] + X[s^1]) times X2[mul_idx], 4 = dual (X[s] -> acc, X[s^1] -> acc2),
+// 12 = dual over ONE row per pair (x_shift: X[s >> 1] is both X[s] and X[s^1], loaded once, added to acc and to acc2)
 // (compile-time, so that the plain path keeps its registers for gathers in flight)
 template <int G, int VEC, int MODE>
 __device__ __forceinline__ void seg_accumulate(const SegParams& p, const GroupCtx<G>& g, const SegPolicies& pol, int64_t m, int64_t kb,
@@ -159,6 +161,9 @@ __device__ __forceinline__ void seg_accumulate(const SegParams& p, const GroupCt
             x[u][v] = on ? seg_ldg(X4 + (int64_t)((MODE & 2) ? sj[u] : (sj[u] >> p.x_shift)) * g.cv + c4, pol.stream) : f4_zero();
             if (MODE & 2) xm[u][v] = on ? seg_ldg(Xm4 + (int64_t)(sj[u] ^ 1) * g.cv + c4, pol.stream) : f4_zero();
             y[u][v] = on ? seg_ldg(X24 + (int64_t)m2j[u] * g.cv + c4, pol.keep) : f4_zero();
+          } else if (MODE & 8) {
+            x[u][v] = on ? ldg_cached(X4 + (int64_t)(sj[u] >> 1) * g.cv + c4) : f4_zero();
+            xm[u][v] = x[u][v];
           } else {
             x[u][v] = on ? ldg_cached(X4 + (int64_t)sj[u] * g.cv + c4) : f4_zero();
             if (MODE & 6) xm[u][v] = on ? ldg_cached(Xm4 + (int64_t)(sj[u] ^ 1) * g.cv + c4) : f4_zero();
@@ -404,7 +409,8 @@ static void launch_seg_mode(const SegParams& p, int64_t chunk_cap, int64_t long_
 }
 template <int G, int VEC>
 static void launch_seg(const SegParams& p, int64_t chunk_cap, int64_t long_cap, cudaStream_t s) {
-  if (p.out2) launch_seg_mode<G, VEC, 4>(p, chunk_cap, long_cap, s);
+  if (p.out2 && p.x_shift) launch_seg_mode<G, VEC, 12>(p, chunk_cap, long_cap, s);
+  else if (p.out2) launch_seg_mode<G, VEC, 4>(p, chunk_cap, long_cap, s);
   else if (!p.X2) launch_seg_mode<G, VEC, 0>(p, chunk_cap, long_cap, s);
   else if (!p.pair_sum) launch_seg_mode<G, VEC, 1>(p, chunk_cap, long_cap, s);
   else launch_seg_mode<G, VEC, 3>(p, chunk_cap, long_cap, s);
@@ -529,7 +535,9 @@ extern "C" int twowl_seg_reduce(const twowl_seg_args* a, void* stream) {
                "seg_reduce: feature pointers must be 16-byte aligned");
   TW_CHECK_ARG(!(a->row_flip && (a->M & 1)), "seg_reduce: row_flip needs an even row count");
   TW_CHECK_ARG((a->X2 == nullptr) == (a->mul_idx == nullptr), "seg_reduce: X2 and mul_idx go together");
-  TW_CHECK_ARG(!a->pair_sum || a->X2 != nullptr, "seg_reduce: pair_sum is only built together with X2");
+  TW_CHECK_ARG(!a->pair_sum || a->X2 != nullptr || (a->pair_sum == 2 && a->out2),
+               "seg_reduce: pair_sum is only built together with X2 (or, = 2, with the dual output)");
+  TW_CHECK_ARG(!(a->pair_sum == 2 && a->X_mate), "seg_reduce: X_mate does not go with a one-row-per-pair X (pair_sum = 2)");
   TW_CHECK_ARG(a->pair_sum >= 0 && a->pair_sum <= 2, "seg_reduce: pair_sum = %d (0, 1 or 2)", a->pair_sum);
   TW_CHECK_ARG(!a->out2 || (!a->X2 && !a->flip && !a->row_flip && !a->accumulate && aligned16(a->out2) && aligned16(a->partial2)),
                "seg_reduce: dual output goes with a plain, unflipped, non-accumulating gather");

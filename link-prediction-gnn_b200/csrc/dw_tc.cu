@@ -148,7 +148,11 @@ __device__ __forceinline__ float dw_lo(float x) { return x - __uint_as_float(__f
 
 // C = width of dO_f, dO_r and H (32, 64 or 128). One stage:
 //   A_hi: AG groups of 32 M-elements ([f cols | r cols | zero padding when C = 32]), A_lo: the same, B_hi: C/32 groups, B_lo
-template <int C, bool GN>
+// HP (H at half height, twowl_pair_dw_gn with h_pairs = 1): H holds ONE row per pair, H[k] = rows 2k and 2k+1 of the pair
+// table. TMA lands the tile's TK/2 rows in a staging area (Hs, C/32 groups of TK/2 rows) and the split warps write each of them
+// twice, to K-rows 2k and 2k+1 of B_hi (raw) and B_lo (split): the MMAs see the same operands in the same K order as with the
+// full-height H, so the sums are bit-identical (adding mates before the MMA would halve its work but change the rounding).
+template <int C, bool GN, bool HP = false>
 __global__ void __launch_bounds__(kDwThreads, 1) k_dw_tc(const DwParams p, const __grid_constant__ CUtensorMap tmF,
                                                          const __grid_constant__ CUtensorMap tmR, const __grid_constant__ CUtensorMap tmH) {
   constexpr int GS = C / 32;                          // 32-column groups per source
@@ -158,8 +162,9 @@ __global__ void __launch_bounds__(kDwThreads, 1) k_dw_tc(const DwParams p, const
   constexpr uint32_t kDwLbo = (kDwTileK / 4) * kDwSbo;   // next group of 32 mn-elements
   constexpr uint32_t kAHalf = (uint32_t)AG * kDwLbo;  // hi (or lo) part of the A stage
   constexpr uint32_t kBHalf = (uint32_t)GS * kDwLbo;
-  constexpr uint32_t kStage = 2u * kAHalf + 2u * kBHalf;
-  constexpr uint32_t kTxBytes = 3u * GS * kDwLbo;     // raw bytes landing per tile
+  constexpr uint32_t kHs = HP ? (uint32_t)GS * (kDwLbo / 2) : 0u;   // staging of the half-height H tile
+  constexpr uint32_t kStage = 2u * kAHalf + 2u * kBHalf + kHs;
+  constexpr uint32_t kTxBytes = 2u * GS * kDwLbo + (HP ? kHs : (uint32_t)GS * kDwLbo);   // raw bytes landing per tile
   extern __shared__ uint8_t dw_smem_raw[];
   // 1024-byte alignment by OFFSET from the shared array: a pointer rebuilt from an integer would be generic (LD.E / ST.E)
   uint8_t* smem = dw_smem_raw + ((1024u - (dw_smem_u32(dw_smem_raw) & 1023u)) & 1023u);
@@ -232,7 +237,10 @@ __global__ void __launch_bounds__(kDwThreads, 1) k_dw_tc(const DwParams p, const
         for (int g = 0; g < GS; ++g) {
           dw_tma_load_2d(Ahi + (size_t)g * kDwLbo, &tmF, g * 32, row, &raw_full[st], policy);
           dw_tma_load_2d(Ahi + (size_t)(GS + g) * kDwLbo, &tmR, g * 32, row, &raw_full[st], policy);
-          dw_tma_load_2d(Bhi + (size_t)g * kDwLbo, &tmH, g * 32, row, &raw_full[st], policy);
+          if (HP)
+            dw_tma_load_2d(Bhi + 2 * kBHalf + (size_t)g * (kDwLbo / 2), &tmH, g * 32, row / 2, &raw_full[st], policy);
+          else
+            dw_tma_load_2d(Bhi + (size_t)g * kDwLbo, &tmH, g * 32, row, &raw_full[st], policy);
         }
       }
       __syncwarp();
@@ -424,11 +432,34 @@ __global__ void __launch_bounds__(kDwThreads, 1) k_dw_tc(const DwParams p, const
           }
         }
       }
+      if constexpr (HP) {
+        // staging chunk i: group g, pair row k (byte k * 128 of the group), 32-byte unit us = logical unit u ^ (k & 3), half hh;
+        // K-rows 2k and 2k+1 of B take it at their own swizzle phase
+        constexpr int kHsGroupChunks = (int)(kDwLbo / 32);
+        const float4* Hs = reinterpret_cast<const float4*>(smem + st * kStage + 2 * kAHalf + 2 * kBHalf);
+        float4* Bh = reinterpret_cast<float4*>(smem + st * kStage + 2 * kAHalf);
+#pragma unroll
+        for (int j = 0; j < kBIter / 2; ++j) {
+          const int i = j * kSplitThreads + t;
+          const float4 v = Hs[i];
+          const float4 lo = make_float4(dw_lo(v.x), dw_lo(v.y), dw_lo(v.z), dw_lo(v.w));
+          const int g = i / kHsGroupChunks, o = i % kHsGroupChunks;   // o: 16-byte chunk inside the group's staging
+          const int k = o >> 3, u = ((o >> 1) & 3) ^ (k & 3), hh = o & 1;
+#pragma unroll
+          for (int e = 0; e < 2; ++e) {
+            const int kk = 2 * k + e;
+            const int c = g * (int)(kDwLbo / 16) + kk * 8 + ((u ^ (kk & 3)) << 1) + hh;
+            Bh[c] = v;
+            Blo[c] = lo;
+          }
+        }
+      } else {
 #pragma unroll 4
-      for (int j = 0; j < kBIter; ++j) {
-        const int i = j * kSplitThreads + t;
-        const float4 v = Bhi[i];
-        Blo[i] = make_float4(dw_lo(v.x), dw_lo(v.y), dw_lo(v.z), dw_lo(v.w));
+        for (int j = 0; j < kBIter; ++j) {
+          const int i = j * kSplitThreads + t;
+          const float4 v = Bhi[i];
+          Blo[i] = make_float4(dw_lo(v.x), dw_lo(v.y), dw_lo(v.z), dw_lo(v.w));
+        }
       }
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       dw_mbar_arrive(&split_done[st]);
@@ -535,22 +566,24 @@ static int dw_grid(int64_t M, int C) {
   const int64_t ntiles = cdiv(M, dw_tile_k(C));
   return (int)(ntiles < kNumSMs ? ntiles : kNumSMs);
 }
-template <int C>
+template <int C, bool HP>
 static size_t dw_smem() {
   const size_t lbo = (size_t)(dw_tile_k(C) / 4) * kDwSbo;
-  const size_t stage = 2 * (dw_nacc(C) == 1 ? 4 : 2 * (C / 32)) * lbo + 2 * (C / 32) * lbo;
+  const size_t stage = 2 * (dw_nacc(C) == 1 ? 4 : 2 * (C / 32)) * lbo + 2 * (C / 32) * lbo + (HP ? (C / 32) * lbo / 2 : 0);
   return (size_t)kDwStages * stage + 128 + 4 * C * sizeof(float) + 1024;
 }
 
-template <int C, bool GN>
+template <int C, bool GN, bool HP = false>
 static int dw_launch(const DwParams& p, const float* Af, const float* Ar, const float* H, cudaStream_t s, int64_t ldA = 0, int64_t ldH = 0) {
   CUtensorMap tf, tr, th;
   if (int rc = make_tmap_2d_f32(&tf, Af, p.M, C, 32, dw_tile_k(C), CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, ldA)) return rc;
   if (int rc = make_tmap_2d_f32(&tr, Ar, p.M, C, 32, dw_tile_k(C), CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, ldA)) return rc;
-  if (int rc = make_tmap_2d_f32(&th, H, p.M, C, 32, dw_tile_k(C), CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, ldH)) return rc;
-  const size_t smem = dw_smem<C>();
-  TW_CUDA(cudaFuncSetAttribute(k_dw_tc<C, GN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_dw_tc<C, GN><<<dw_grid(p.M, C), kDwThreads, smem, s>>>(p, tf, tr, th);
+  if (int rc = make_tmap_2d_f32(&th, H, HP ? p.M / 2 : p.M, C, 32, HP ? dw_tile_k(C) / 2 : dw_tile_k(C), CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
+                                ldH))
+    return rc;
+  const size_t smem = dw_smem<C, HP>();
+  TW_CUDA(cudaFuncSetAttribute(k_dw_tc<C, GN, HP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_dw_tc<C, GN, HP><<<dw_grid(p.M, C), kDwThreads, smem, s>>>(p, tf, tr, th);
   TW_LAUNCH_CHECK();
   return 0;
 }
@@ -561,12 +594,12 @@ using namespace twowl;
 
 extern "C" int twowl_pair_dw_supported(int32_t C) { return (C == 32 || C == 64 || C == 128) ? 1 : 0; }
 
-template <bool GN>
+template <bool GN, bool HP = false>
 static int dw_dispatch(const DwParams& p, int C, const float* Af, const float* Ar, const float* H, float* dWf, float* dWr, cudaStream_t s,
                        int64_t ldA = 0, int64_t ldH = 0) {
-  const int rc = C == 32   ? dw_launch<32, GN>(p, Af, Ar, H, s, ldA, ldH)
-                 : C == 64 ? dw_launch<64, GN>(p, Af, Ar, H, s, ldA, ldH)
-                           : dw_launch<128, GN>(p, Af, Ar, H, s, ldA, ldH);
+  const int rc = C == 32   ? dw_launch<32, GN, HP>(p, Af, Ar, H, s, ldA, ldH)
+                 : C == 64 ? dw_launch<64, GN, HP>(p, Af, Ar, H, s, ldA, ldH)
+                           : dw_launch<128, GN, HP>(p, Af, Ar, H, s, ldA, ldH);
   if (rc) return rc;
   if (dw_nacc(C) == 1)
     k_dw_tc_final<double><<<(int)cdiv(2 * C * C, 256), 256, 0, s>>>(reinterpret_cast<const double*>(p.part), dw_grid(p.M, C), C,
@@ -612,10 +645,11 @@ extern "C" int twowl_pair_dw_ld(const float* dOf, const float* dOr, const float*
 
 extern "C" int twowl_pair_dw_gn(const float* Of, const float* Or, const float* consts, const float* G, const int32_t* head,
                                 const int32_t* next, float p_drop, uint64_t seed_f, uint64_t seed_r, int32_t relu, const float* rsf,
-                                const float* rsr, const float* H, int64_t M, int32_t C, float* dOf, float* dOr, float* dWf, float* dWr,
-                                void* ws, size_t ws_bytes, void* stream) {
+                                const float* rsr, const float* H, int32_t h_pairs, int64_t M, int32_t C, float* dOf, float* dOr,
+                                float* dWf, float* dWr, void* ws, size_t ws_bytes, void* stream) {
   TW_CHECK_ARG(twowl_pair_dw_supported(C), "pair_dw_gn: C=%d unsupported (32, 64 or 128)", C);
   TW_CHECK_ARG(M > 0 && M < 0x7fffffffLL, "pair_dw_gn: needs 0 < M < 2^31");
+  TW_CHECK_ARG(h_pairs == 0 || (h_pairs == 1 && M % 2 == 0), "pair_dw_gn: h_pairs = %d needs 0, or 1 with an even M", h_pairs);
   TW_CHECK_ARG(aligned16(Of) && aligned16(Or) && aligned16(H) && aligned16(dOf) && aligned16(dOr) && aligned16(consts) && aligned16(G) &&
                    rsf && rsr && head && next,
                "pair_dw_gn: bad pointers");
@@ -627,5 +661,6 @@ extern "C" int twowl_pair_dw_gn(const float* Of, const float* Or, const float* c
   p.consts = consts, p.G = G, p.head = head, p.next = next, p.dOf = dOf, p.dOr = dOr;
   p.thresh = p_drop > 0.f ? drop_thresh(p_drop) : 0u, p.inv_keep = 1.f / (1.f - p_drop);
   p.seed_f = seed_f, p.seed_r = seed_r, p.relu = relu;
-  return dw_dispatch<true>(p, C, Of, Or, H, dWf, dWr, (cudaStream_t)stream);
+  return h_pairs ? dw_dispatch<true, true>(p, C, Of, Or, H, dWf, dWr, (cudaStream_t)stream)
+                 : dw_dispatch<true>(p, C, Of, Or, H, dWf, dWr, (cudaStream_t)stream);
 }

@@ -167,7 +167,12 @@ struct PcRing {
 // tile run side by side, so the re-reads of its A slabs are L2 hits.
 // PSUM (compile time, its own instantiation - a runtime flag changed the register allocation of every other one and cost the
 // forward launches 1 ms each): out has M/2 rows, out[k] = result[2k] + result[2k+1]
-template <int NG, bool PSUM = false>
+// APAIR (compile time, likewise; nsrc = 1): A has M/2 rows, one per pair, and output row r uses A row r >> 1 - the depth-1 pair
+// layer's H, whose rows 2k / 2k+1 are the same bits (twowl_conv_args.a_pairs). The 64 pairs of a 128-row tile land as four
+// 16-row boxes at rows 0 / 32 / 64 / 96 of the stage, so TMEM lanes 32q..32q+15 hold the products of pairs 16q..16q+15 and
+// epilogue lane l of quarter q takes its row's values from lane l >> 1. Rows 16..31 of each quarter hold stale data whose
+// products land in TMEM lanes nobody reads; the MMA, the epilogue's rows, gathers, stores and statistics are unchanged.
+template <int NG, bool PSUM = false, bool APAIR = false>
 __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
                                                              const __grid_constant__ CUtensorMap tmA1) {
   extern __shared__ uint8_t pc_smem_raw[];
@@ -279,9 +284,17 @@ __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p,
           const int ns = KB - kb < G ? KB - kb : G;
           pc_mbar_wait(&raw_empty[r.slot], r.phase ^ 1u);
           if (pc_elect_one()) {
-            pc_mbar_expect_tx(&raw_full[r.slot], (uint32_t)ns * kPcSlab);
-            for (int j = 0; j < ns; ++j)
-              pc_tma_load_2d(As + (size_t)r.slot * kStage + (size_t)j * kPcSlab, tm, (kb + j) * 32, row0, &raw_full[r.slot], policy);
+            if constexpr (APAIR) {
+              pc_mbar_expect_tx(&raw_full[r.slot], (uint32_t)ns * (kPcSlab / 2));
+              for (int j = 0; j < ns; ++j)
+                for (int q = 0; q < 4; ++q)
+                  pc_tma_load_2d(As + (size_t)r.slot * kStage + (size_t)j * kPcSlab + q * 4096, tm, (kb + j) * 32, (row0 >> 1) + q * 16,
+                                 &raw_full[r.slot], policy);
+            } else {
+              pc_mbar_expect_tx(&raw_full[r.slot], (uint32_t)ns * kPcSlab);
+              for (int j = 0; j < ns; ++j)
+                pc_tma_load_2d(As + (size_t)r.slot * kStage + (size_t)j * kPcSlab, tm, (kb + j) * 32, row0, &raw_full[r.slot], policy);
+            }
           }
           __syncwarp();
           r.next(S);
@@ -478,6 +491,10 @@ __global__ void __launch_bounds__(kPcThreads, 1) k_pair_conv(const ConvParams p,
           pc_tmem_ld8(taddr + c0 + q2 * 8, v0);
           if (p.nsrc > 1) pc_tmem_ld8(taddr + Nsp + c0 + q2 * 8, v1);
           pc_tmem_wait_ld();
+          if constexpr (APAIR) {
+#pragma unroll
+            for (int e = 0; e < 8; ++e) v0[e] = __shfl_sync(0xffffffffu, v0[e], lane >> 1);
+          }
           float o[8];
 #pragma unroll
           for (int e = 0; e < 8; ++e) o[e] = rsc[0] * __uint_as_float(v0[e]);
@@ -645,10 +662,10 @@ static int pc_make_tmap(CUtensorMap* tm, const float* A, int64_t M, int Kd) {
   return make_tmap_2d_f32(tm, A, M, Kd, 32, kPcTileM, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-template <int NG, bool PSUM = false>
+template <int NG, bool PSUM = false, bool APAIR = false>
 static int pc_launch(const ConvParams& p, size_t smem, const CUtensorMap& t0, const CUtensorMap& t1, cudaStream_t s) {
-  TW_CUDA(cudaFuncSetAttribute(k_pair_conv<NG, PSUM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_pair_conv<NG, PSUM><<<pc_grid(p.M, p.nsplit), kPcThreads, smem, s>>>(p, t0, t1);
+  TW_CUDA(cudaFuncSetAttribute(k_pair_conv<NG, PSUM, APAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_pair_conv<NG, PSUM, APAIR><<<pc_grid(p.M, p.nsplit), kPcThreads, smem, s>>>(p, t0, t1);
   TW_LAUNCH_CHECK();
   return 0;
 }
@@ -703,6 +720,11 @@ extern "C" int twowl_pair_conv(const twowl_conv_args* a, void* ws, size_t ws_byt
     TW_CHECK_ARG(!want_stats && a->M % 2 == 0 && a->ngather == 2,
                  "pair_conv: pair_sum_out is built for the pair layer's input gradient: two gathers, an even M, no statistics");
   }
+  TW_CHECK_ARG(a->a_pairs == 0 || a->a_pairs == 1, "pair_conv: a_pairs = %d (0 or 1)", a->a_pairs);
+  if (a->a_pairs) {
+    TW_CHECK_ARG(a->nsrc == 1 && a->ngather == 1 && a->M % 2 == 0 && !a->pair_sum_out,
+                 "pair_conv: a_pairs is built for the depth-1 pair layer's forward: one source, one gather, an even M");
+  }
   p.nsrc = a->nsrc, p.ngather = a->ngather, p.M = a->M, p.Kd = a->Kd, p.Nd = a->Nd, p.bias = a->bias, p.out = a->out;
   p.Nsub = cfg.Nsub, p.nsplit = cfg.nsplit, p.stages = cfg.stages, p.lo_stages = cfg.lo_stages, p.tmem_cols = cfg.tmem_cols, p.group = cfg.group;
   cudaStream_t s = (cudaStream_t)stream;
@@ -715,10 +737,13 @@ extern "C" int twowl_pair_conv(const twowl_conv_args* a, void* ws, size_t ws_byt
   CUtensorMap tm[2];
   memset(tm, 0, sizeof(tm));
   for (int i = 0; i < a->nsrc; ++i) {
-    const int rc_t = pc_make_tmap(&tm[i], a->A[i], a->M, a->Kd);
+    // a_pairs: A has one row per pair, fetched as 16-row boxes (four per 128-row output tile)
+    const int rc_t = a->a_pairs ? make_tmap_2d_f32(&tm[i], a->A[i], a->M / 2, a->Kd, 32, 16, CU_TENSOR_MAP_SWIZZLE_128B)
+                                : pc_make_tmap(&tm[i], a->A[i], a->M, a->Kd);
     if (rc_t) return rc_t;
   }
-  const int rc = a->pair_sum_out   ? pc_launch<2, true>(p, cfg.smem, tm[0], tm[1], s)
+  const int rc = a->a_pairs        ? pc_launch<1, false, true>(p, cfg.smem, tm[0], tm[1], s)
+                 : a->pair_sum_out ? pc_launch<2, true>(p, cfg.smem, tm[0], tm[1], s)
                  : a->ngather == 0 ? pc_launch<0>(p, cfg.smem, tm[0], tm[1], s)
                  : a->ngather == 1 ? pc_launch<1>(p, cfg.smem, tm[0], tm[1], s)
                                    : pc_launch<2>(p, cfg.smem, tm[0], tm[1], s);

@@ -41,16 +41,17 @@ __global__ void __launch_bounds__(kRowThreads) k_gather_rows(const float* __rest
   }
 }
 
+// out[r] = X[src[r << sh]] * X[dst[r << sh]] for r < R (sh = 1: one row per mated pair, see twowl_pair_init_fwd)
 __global__ void __launch_bounds__(kRowThreads) k_pair_init(const float* __restrict__ X, const int32_t* __restrict__ src,
-                                                           const int32_t* __restrict__ dst, int64_t R, int C,
+                                                           const int32_t* __restrict__ dst, int64_t R, int C, int sh,
                                                            float* __restrict__ out) {
   const RowSlots rs(C);
   if (rs.slot < 0) return;
   const float4* __restrict__ X4 = reinterpret_cast<const float4*>(X);
   float4* __restrict__ o4 = reinterpret_cast<float4*>(out);
   for (int64_t r = (int64_t)blockIdx.x * rs.slots + rs.slot; r < R; r += (int64_t)gridDim.x * rs.slots) {
-    const float4 a = ldg_cached(X4 + (int64_t)src[r] * rs.cv + rs.c4);
-    const float4 b = ldg_cached(X4 + (int64_t)dst[r] * rs.cv + rs.c4);
+    const float4 a = ldg_cached(X4 + (int64_t)src[r << sh] * rs.cv + rs.c4);
+    const float4 b = ldg_cached(X4 + (int64_t)dst[r << sh] * rs.cv + rs.c4);
     stg_stream(o4 + r * rs.cv + rs.c4, f4_mul(a, b));
   }
 }
@@ -294,12 +295,14 @@ extern "C" int twowl_gather_rows(const float* W, int64_t rows_w, const int64_t* 
   return 0;
 }
 
-extern "C" int twowl_pair_init_fwd(const float* X, const int32_t* src, const int32_t* dst, int64_t R, int32_t C, float* out,
-                                   void* stream) {
+extern "C" int twowl_pair_init_fwd(const float* X, const int32_t* src, const int32_t* dst, int64_t R, int32_t C, int32_t pairs,
+                                   float* out, void* stream) {
   if (int rc = check_c("pair_init_fwd", C)) return rc;
   TW_CHECK_ARG(aligned16(X) && aligned16(out), "pair_init_fwd: X/out must be 16-byte aligned");
-  if (R <= 0) return 0;
-  k_pair_init<<<row_grid(R, C), kRowThreads, 0, (cudaStream_t)stream>>>(X, src, dst, R, C, out);
+  TW_CHECK_ARG(pairs == 0 || (pairs == 1 && R % 2 == 0), "pair_init_fwd: pairs = %d needs 0, or 1 with an even R", pairs);
+  const int64_t rows = R >> pairs;
+  if (rows <= 0) return 0;
+  k_pair_init<<<row_grid(rows, C), kRowThreads, 0, (cudaStream_t)stream>>>(X, src, dst, rows, C, pairs, out);
   TW_LAUNCH_CHECK();
   return 0;
 }

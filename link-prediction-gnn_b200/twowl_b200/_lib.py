@@ -46,7 +46,7 @@ class ConvArgs(ctypes.Structure):
         ("W", ctypes.c_void_p * 2), ("w_kn", ctypes.c_int32 * 2), ("T", ctypes.c_void_p * 2),
         ("tidx", ctypes.c_void_p * 2), ("tcoef", ctypes.c_void_p * 2), ("bias", ctypes.c_void_p),
         ("out", ctypes.c_void_p), ("stats", ctypes.c_void_p), ("mean_scale", ctypes.c_void_p), ("eps", ctypes.c_float),
-        ("moments", ctypes.c_void_p), ("pair_sum_out", ctypes.c_int32),
+        ("moments", ctypes.c_void_p), ("pair_sum_out", ctypes.c_int32), ("a_pairs", ctypes.c_int32),
     ]
 
 

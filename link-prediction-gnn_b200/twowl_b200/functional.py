@@ -325,15 +325,15 @@ readout.register_autograd(_ro_bwd, setup_context=_ro_setup)
 # and the two GraphNorm(+Dropout+ReLU) applications summed. The backward is hand-written from the same pieces.
 
 
-def _pair_convs_fwd(h, pf, pr, SHf, SHr, centre, dinv, selfw, eps):
+def _pair_convs_fwd(h, pf, pr, SHf, SHr, centre, dinv, selfw, eps, h_pairs=False):
     """O_d = selfw_d * (h W_d^T) + dinv_d * (SH_d W_d^T)[centre_d] + bias_d and its GraphNorm statistics, both directions:
-    -> [(O_f, stats_f, SH_f), (O_r, stats_r, SH_r)]."""
+    -> [(O_f, stats_f, SH_f), (O_r, stats_r, SH_r)]. h_pairs: h holds one row per pair (row r of O uses h[r >> 1])."""
     (wf, bf, gmf), (wr, br, gmr) = pf, pr
     Sf, Sr = ops.linear_fwd(SHf, wf), ops.linear_fwd(SHr, wr)
     outs = []
     for d, (w, b, gm, S, SH) in enumerate(((wf, bf, gmf, Sf, SHf), (wr, br, gmr, Sr, SHr))):
         O, st = ops.pair_conv([h], [w], [0], row_scale=[selfw[d]], gathers=[(S, centre[d], dinv[d])], bias=b,
-                              stats_mean_scale=gm, eps=eps)
+                              stats_mean_scale=gm, eps=eps, a_pairs=h_pairs)
         outs.append((O, st, SH))
     return outs
 
@@ -437,11 +437,13 @@ def pair_layer_readout(h: Tensor, wf: Tensor, bf: Tensor, gwf: Tensor, gbf: Tens
 
 
 def _plr_forward(h, wf, bf, gwf, gbf, gmf, wr, br, gwr, gbr, gmr, idx, pw, pb, in_ptr, in_ids, in_plan, centre, dinv, selfw, blocked,
-                 n_node, eps, p_drop, seed_f, seed_r):
-    # both directions' in-list sums from one pass over the mated 2-row blocks of h: SH_r gathers h[a], SH_f h[a^1]
+                 n_node, eps, p_drop, seed_f, seed_r, h_pairs=False):
+    """h_pairs: h is [R/2, C], one row per pair, standing for rows 2k and 2k+1 of the mated pair table (pair_init_layer_readout)."""
+    # both directions' in-list sums from one pass over the mated 2-row blocks of h: SH_r gathers h[a], SH_f h[a^1] (h_pairs: the
+    # one row h[a >> 1] feeds both)
     SHr, SHf = ops.seg_reduce(in_ptr, in_ids, n_node, h, plan=in_plan, src_scale=dinv[1], skip_mask=blocked, dual=True,
-                              src_scale2=dinv[0])
-    outs = _pair_convs_fwd(h, (wf, bf, gmf), (wr, br, gmr), SHf, SHr, centre, dinv, selfw, eps)
+                              src_scale2=dinv[0], x_pairs=h_pairs)
+    outs = _pair_convs_fwd(h, (wf, bf, gmf), (wr, br, gmr), SHf, SHr, centre, dinv, selfw, eps, h_pairs)
     pred = ops.gn2_readout_fwd(outs[0][0], outs[1][0], outs[0][1], outs[1][1], (gwf, gbf, gmf), (gwr, gbr, gmr), p_drop, seed_f,
                                seed_r, True, idx, pw.contiguous(), pb)
     return pred, outs[0][0], outs[1][0], outs[0][1], outs[1][1], outs[0][2], outs[1][2]
@@ -475,11 +477,13 @@ def _plr_bwd(ctx, g, *_unused):
 
 def _plr_backward(g, saved, n_node, p_drop, seed_f, seed_r, pair_sum_out=False):
     """Backward of the fused last pair layer + readout from d pred: -> (dh, per-direction parameter gradients, d pred.weight,
-    d pred.bias). pair_sum_out: dh is [R/2, C], the sum of the two directions' rows of every pair."""
+    d pred.bias). pair_sum_out: dh is [R/2, C], the sum of the two directions' rows of every pair. h may hold one row per pair
+    ([R/2, C], pair_init_layer_readout): only pair_dw_gn reads it then."""
     (h, wf, bf, gwf, gbf, gmf, wr, br, gwr, gbr, gmr, idx, pw, out_ptr, out_ids, out_plan, dinv, selfw, bnode, Of, Or, sf, sr,
      SHf, SHr) = saved
     C = wf.shape[0]
-    if ops.pair_dw_supported(C) and h.shape[1] == C:
+    h_pairs = h.shape[0] != Of.shape[0]
+    if h_pairs or (ops.pair_dw_supported(C) and h.shape[1] == C):
         # the dense GraphNorm-backward pass rides on the weight-gradient kernel's shared-memory pass (twowl_pair_dw_gn)
         G, head, nxt, consts, dpf, dpr, dpw, dpb = ops.gn2_readout_bwd_prepare(Of, Or, sf, sr, (gwf, gbf, gmf), (gwr, gbr, gmr),
                                                                                p_drop, seed_f, seed_r, True, idx, pw.contiguous(),
@@ -495,7 +499,7 @@ def _plr_backward(g, saved, n_node, p_drop, seed_f, seed_r, pair_sum_out=False):
         dWs = None
     dh_out = None
     if inplace:      # h is not read by that launch: dH (or its pair sums, in the first half of the buffer) may take its place
-        dh_out = h.view(-1)[:(h.shape[0] // 2) * h.shape[1]].view(h.shape[0] // 2, h.shape[1]) if pair_sum_out else h
+        dh_out = h.view(-1)[:(h.shape[0] // 2) * h.shape[1]].view(h.shape[0] // 2, h.shape[1]) if pair_sum_out and not h_pairs else h
     dh, res = _pl_bwd_core(h, wf, wr, out_ptr, out_ids, out_plan, dinv, selfw, bnode, SHf, SHr, n_node, [dOf, dOr], [dpf, dpr],
                            dWs=dWs, dh_out=dh_out, pair_sum_out=pair_sum_out)
     return dh, res, dpw.reshape(pw.shape), dpb
@@ -518,17 +522,26 @@ def pair_init_layer_readout(x: Tensor, src: Tensor, dst: Tensor, ptr_s: Tensor, 
                             out_ptr: Tensor, out_ids: Tensor, out_plan: Tensor, centre: Tensor, dinv: Tensor, selfw: Tensor,
                             bnode: Tensor, blocked: Optional[Tensor], n_node: int, eps: float, p_drop: float, seed_f: int,
                             seed_r: int) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
-    """-> (pred [L,1], H, O_f, O_r, stats_f, stats_r, SH_f, SH_r); only pred is differentiable, the rest is saved state."""
-    h = ops.pair_init_fwd(x.contiguous(), src, dst)
+    """-> (pred [L,1], H, O_f, O_r, stats_f, stats_r, SH_f, SH_r); only pred is differentiable, the rest is saved state.
+    H is private to the op, and on the mated table its rows 2k and 2k+1 are the same bits: where the weight-gradient kernel
+    covers the width it is kept at half height, ONE row per pair ([R/2, C]), and every consumer reads that row for both."""
+    h_pairs = _plr_h_pairs(x.shape[1], wf.shape[0])
+    h = ops.pair_init_fwd(x.contiguous(), src, dst, pairs=h_pairs)
     return (h,) + _plr_forward(h, wf, bf, gwf, gbf, gmf, wr, br, gwr, gbr, gmr, idx, pw, pb, in_ptr, in_ids, in_plan, centre, dinv,
-                               selfw, blocked, n_node, eps, p_drop, seed_f, seed_r)
+                               selfw, blocked, n_node, eps, p_drop, seed_f, seed_r, h_pairs)
+
+
+def _plr_h_pairs(Cin: int, C: int) -> bool:
+    """Whether pair_init_layer_readout keeps H at half height: the widths pair_dw_gn covers (other widths compute the weight
+    gradient from a full-height H)."""
+    return Cin == C and ops.pair_dw_supported(C)
 
 
 @pair_init_layer_readout.register_fake
 def _(x, src, dst, ptr_s, ids_s, plan_s, wf, bf, gwf, gbf, gmf, wr, br, gwr, gbr, gmr, idx, pw, pb, in_ptr, in_ids, in_plan, out_ptr,
       out_ids, out_plan, centre, dinv, selfw, bnode, blocked, n_node, eps, p_drop, seed_f, seed_r):
     C = wf.shape[0]
-    h = x.new_empty((src.numel(), x.shape[1]))
+    h = x.new_empty((src.numel() // 2 if _plr_h_pairs(x.shape[1], C) else src.numel(), x.shape[1]))
     o = x.new_empty((src.numel(), C))
     return (h, x.new_empty((idx.numel() // 2, 1)), o, torch.empty_like(o), x.new_empty((2 * C,)), x.new_empty((2 * C,)),
             x.new_empty((n_node, x.shape[1])), x.new_empty((n_node, x.shape[1])))

@@ -457,7 +457,7 @@ def seg_reduce(ptr, col, M: int, X, *, plan=None, flip=0, row_flip=0, src_scale=
         if X_mate is not None:      # the mates' rows come from a second matrix of the same shape (dO_r next to dO_f)
             assert X_mate.shape == X.shape and X_mate.is_contiguous() and X_mate.dtype == torch.float32
             a.X_mate = X_mate.data_ptr()
-    nbytes = col.numel() * (4 * C * (1 + int(pair_sum) + int(X2 is not None) + int(dual)) + 8 + 4 * int(dual)) + \
+    nbytes = col.numel() * (4 * C * (1 + int(pair_sum) + int(X2 is not None) + int(dual and not x_pairs)) + 8 + 4 * int(dual)) + \
         M * (4 * C + 8) * (1 + int(dual))
     if rows is not None:      # a node block: its share of the entries is not known on the host - charged by its share of the rows
         nbytes = nbytes * (int(rows[1]) - int(rows[0])) // max(M, 1)
@@ -479,12 +479,14 @@ def gather_rows(W: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def pair_init_fwd(X, src32, dst32) -> torch.Tensor:
+def pair_init_fwd(X, src32, dst32, pairs: bool = False) -> torch.Tensor:
+    """H[p] = X[src[p]] * X[dst[p]]; pairs=True on a mated table: ONE row per pair, H[k] = X[src[2k]] * X[dst[2k]] ([R/2, C])."""
     _need_cuda(X, src32, dst32)
     R = src32.numel()
-    out = torch.empty((R, X.shape[1]), dtype=torch.float32, device=X.device)
-    with _P("pair_init_fwd", R * (12 * X.shape[1] + 8)):
-        check(lib.twowl_pair_init_fwd(X.data_ptr(), src32.data_ptr(), dst32.data_ptr(), R, X.shape[1], out.data_ptr(),
+    rows = R // 2 if pairs else R
+    out = torch.empty((rows, X.shape[1]), dtype=torch.float32, device=X.device)
+    with _P("pair_init_fwd", rows * (12 * X.shape[1] + 8)):
+        check(lib.twowl_pair_init_fwd(X.data_ptr(), src32.data_ptr(), dst32.data_ptr(), R, X.shape[1], int(pairs), out.data_ptr(),
                                       _stream()), "pair_init_fwd")
     _count()
     return out
@@ -857,14 +859,17 @@ def pair_conv_supported(Kd: int, Nd: int, nsrc: int) -> bool:
 
 
 def pair_conv(A, W, w_kn, *, row_scale=None, gathers=(), bias=None, stats_mean_scale=None, eps: float = 1e-5,
-              want_moments: bool = False, out=None, pair_sum_out: bool = False):
+              want_moments: bool = False, out=None, pair_sum_out: bool = False, a_pairs: bool = False):
     """out = sum_s (row_scale_s * A_s) B_s^T + sum_g coef_g * T_g[idx_g] + bias on tcgen05 (3xTF32).
     A, W, w_kn, row_scale: sequences of length nsrc; gathers: sequence of (T, idx int32, coef).
     Returns out, or (out, stats[2*Nd]) when stats_mean_scale is given (GraphNorm mean / inv_std of out), or
     (out, moments float64[2*Nd]) with want_moments (raw column sum / sum of squares, for a row-sharded caller).
-    pair_sum_out: out is [M/2, Nd] and holds out[2k] + out[2k+1] (what the pair-init backward consumes: seg_reduce(x_pairs=True))."""
+    pair_sum_out: out is [M/2, Nd] and holds out[2k] + out[2k+1] (what the pair-init backward consumes: seg_reduce(x_pairs=True)).
+    a_pairs: A[0] holds ONE row per pair ([M/2, Kd], pair_init_fwd(pairs=True)) and output row r uses row r >> 1; out keeps M rows."""
     nsrc = len(A)
     M, Kd = A[0].shape
+    if a_pairs:
+        M *= 2
     Nd = W[0].shape[1] if w_kn[0] else W[0].shape[0]
     dev = A[0].device
     _need_cuda(*A, *W)
@@ -876,7 +881,7 @@ def pair_conv(A, W, w_kn, *, row_scale=None, gathers=(), bias=None, stats_mean_s
     else:   # a caller-owned [M, Nd] buffer that is none of this launch's inputs (the in-place backward, see INPLACE_BACKWARD)
         assert out.shape == (Mo, Nd) and out.is_contiguous() and all(out.data_ptr() != x.data_ptr() for x in A)
     a = ConvArgs(nsrc=nsrc, ngather=len(gathers), Kd=Kd, Nd=Nd, M=M, bias=_p(bias), out=out.data_ptr(), eps=float(eps),
-                 pair_sum_out=int(pair_sum_out))
+                 pair_sum_out=int(pair_sum_out), a_pairs=int(a_pairs))
     keep = []
     for s in range(nsrc):
         x = A[s].contiguous()
@@ -896,7 +901,7 @@ def pair_conv(A, W, w_kn, *, row_scale=None, gathers=(), bias=None, stats_mean_s
         assert stats is not None, "pair_conv: moments need stats_mean_scale"
         moments = torch.zeros(2 * Nd, dtype=torch.float64, device=dev)   # zeros: an empty row block contributes nothing
         a.moments = moments.data_ptr()
-    nbytes = M * (4 * Kd * nsrc + 8 * len(gathers) + (4 * Nd + 8) * len(gathers)) + Mo * 4 * Nd
+    nbytes = (M // 2 if a_pairs else M) * 4 * Kd * nsrc + M * (8 * len(gathers) + (4 * Nd + 8) * len(gathers)) + Mo * 4 * Nd
     with _P("pair_conv", nbytes):
         check(lib.twowl_pair_conv(ctypes.byref(a), _p(ws), nb, _stream()), "pair_conv")
     _count(1 if stats is None else 2)
@@ -963,18 +968,21 @@ INPLACE_BACKWARD = os.environ.get("TWOWL_INPLACE_BACKWARD", "0") != "0"
 
 def pair_dw_gn(Of, Or, consts, G, head, nxt, p_drop: float, seed_f: int, seed_r: int, relu: bool, rsf, rsr, H, inplace: bool = False):
     """pair_dw with the gradients made on the fly from the last pair layer's outputs (after gn2_readout_bwd_prepare):
-    -> (dOf, dOr [M,C], dWf, dWr [C,C]). One pass: reads Of, Or, H, writes dOf, dOr (over Of, Or with inplace=True)."""
+    -> (dOf, dOr [M,C], dWf, dWr [C,C]). One pass: reads Of, Or, H, writes dOf, dOr (over Of, Or with inplace=True).
+    H may hold ONE row per pair ([M/2, C], pair_init_fwd(pairs=True)): it then stands for rows 2k and 2k+1."""
     _need_cuda(Of, Or, H)
-    M, C = H.shape
+    M, C = Of.shape
+    h_pairs = H.shape[0] != M
+    assert H.shape == ((M // 2, C) if h_pairs else (M, C)) and (M % 2 == 0 or not h_pairs), "pair_dw_gn: H is [M, C] or [M/2, C]"
     dOf, dOr = (Of, Or) if inplace else (torch.empty_like(Of), torch.empty_like(Or))
     dWf = torch.empty((C, C), dtype=torch.float32, device=H.device)
     dWr = torch.empty((C, C), dtype=torch.float32, device=H.device)
     nb = lib.twowl_pair_dw_workspace_bytes(M, C)
     ws = _ws(nb, H.device)
-    with _P("pair_dw_gn", 20 * M * C + 12 * M):
+    with _P("pair_dw_gn", (18 if h_pairs else 20) * M * C + 12 * M):
         check(lib.twowl_pair_dw_gn(Of.data_ptr(), Or.data_ptr(), consts.data_ptr(), G.data_ptr(), head.data_ptr(), nxt.data_ptr(),
                                    float(p_drop), int(seed_f), int(seed_r), int(relu), rsf.data_ptr(), rsr.data_ptr(), H.data_ptr(),
-                                   M, C, dOf.data_ptr(), dOr.data_ptr(), dWf.data_ptr(), dWr.data_ptr(), ws.data_ptr(), nb,
+                                   int(h_pairs), M, C, dOf.data_ptr(), dOr.data_ptr(), dWf.data_ptr(), dWr.data_ptr(), ws.data_ptr(), nb,
                                    _stream()), "pair_dw_gn")
     _count(2)
     return dOf, dOr, dWf, dWr
