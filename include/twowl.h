@@ -519,6 +519,27 @@ int twowl_link_heuristics(const int64_t* ptr, const int32_t* adj, int64_t num_no
                           int64_t s_v, int64_t P, const int64_t* chunk_off, int64_t n_chunks, float* out, void* ws, size_t ws_bytes,
                           void* stream);
 
+/* Link recommendation over a simple adjacency (ptr, adj) of twowl_simple_adjacency: for each source s = src[q] (int64[Q], element
+ * stride), the top k of its candidates C(s) = {v != s : v not in N(s), N(s) ∩ N(v) non-empty} by one of the four scores above.
+ * With c = |N(s) ∩ N(v)|: cn = c; jaccard = c / (d(s) + d(v) - c) as an fp32 quotient; aa and ra add the same terms as
+ * twowl_link_heuristics, but in double over the common w in ascending id order, one at a time, rounded once to fp32.
+ * Two calls, with one host read between them:
+ *   twowl_recommend_plan: exp_off (int64[Q+1]) = exclusive scan of the expansions X(s) = sum of d(w) over w in N(s) (0 for a bad
+ *                         id); info (int64[2], device) = (ids outside [0, num_nodes), exp_off[Q]).
+ *   twowl_recommend:      the queries [q_begin, q_end), a batch of n_entries = exp_off[q_end] - exp_off[q_begin] < 2^31
+ *                         expansion entries (the caller's copy of exp_off; the workspace is sized by it). Writes rows
+ *                         [q_begin, q_end) of ids (int64[Q*k]) and scores (fp32[4*Q*k], rows cn, jaccard, aa, ra): row q holds
+ *                         the top min(k, |C(s)|) candidates ordered by score `by` (0 cn, 1 jaccard, 2 aa, 3 ra) descending,
+ *                         ties by id ascending, then -1 / NaN. Every source id must be valid (the plan counts bad ones).
+ * Bitwise repeatable (no floating-point atomics) and independent of the batching. adj may be NULL when nnz = 0. */
+size_t twowl_recommend_plan_workspace_bytes(int64_t Q);
+int twowl_recommend_plan(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* src, int64_t s_src, int64_t Q,
+                         int64_t* exp_off, int64_t* info, void* ws, size_t ws_bytes, void* stream);
+size_t twowl_recommend_workspace_bytes(int64_t n_entries, int64_t n_queries);
+int twowl_recommend(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* src, int64_t s_src, int64_t Q,
+                    int64_t q_begin, int64_t q_end, const int64_t* exp_off, int64_t n_entries, int32_t by, int64_t k, int64_t* ids,
+                    float* scores, void* ws, size_t ws_bytes, void* stream);
+
 /* ------------------------------------------------------------------ structured wedge path ------- */
 
 /* When ei2 is the full wedge join of (pos_edge, pred_edge) minus the wedges whose source edge is blocked

@@ -154,6 +154,35 @@ def heuristic_scores(dataset):
     return dict(zip(ops.HEURISTICS, scores.unbind(0)))
 
 
+@torch.no_grad()
+def recommend(dataset, src, k=100, by="aa"):
+    """Link recommendation (extension: the retrieval half of a re-ranking pipeline) -> (ids int64 [Q, k], scores fp32 [4, Q, k]):
+    each source's top-k two-hop non-neighbours by the heuristic `by`, over the split's message-passing graph dataset.ei read as
+    undirected and simple, exactly as heuristic_scores reads it (ops.recommend_links; -1 / NaN pad a row with fewer candidates).
+    TwoWL.operators.datasets.candidate_dataset turns the result into a table that rerank() scores with the model."""
+    from twowl_b200 import graph
+    ptr, adj = graph.simple_adjacency(dataset.ei, dataset.x.shape[0])
+    return ops.recommend_links(ptr, adj, src, k, by)
+
+
+@torch.no_grad()
+def rerank(mod, dataset):
+    """Re-rank a candidate table of TwoWL.operators.datasets.candidate_dataset with the model -> (ids int64 [Q, k], logits fp32
+    [Q, k]). One full-graph forward exactly like test(), every prediction pair a target; each row is then ordered by logit
+    descending, ties keeping the heuristic's order, with the padding (-1) last at -inf.
+    The logits depend on the whole candidate table, not only on the pair: GraphNorm's statistics run over all pair rows of the
+    table (SURVEY §3.4), just as test()'s scores depend on the split. Score one table per set of sources you compare."""
+    mod.eval()
+    n_edges = dataset.ei.shape[1]
+    targets = n_edges + torch.arange(dataset.y.shape[0], device=dataset.x.device)
+    logits = mod(dataset.x, dataset.ei, dataset.pos1, targets, dataset.ei2, True).reshape(-1)
+    mask = dataset.cand_mask
+    table = torch.full(mask.shape, float("-inf"), dtype=logits.dtype, device=logits.device)
+    table[mask] = logits
+    order = torch.sort(table, dim=1, descending=True, stable=True).indices
+    return dataset.cand_ids.gather(1, order), table.gather(1, order)
+
+
 def _record_run(record_dir, dsname, tst_score, seconds, fpr, tpr):
     """train.py:108-134: append 'AUC:<auc>   Time:<s>   ' to the dataset's record file; when this run's (unrounded) score is not
     below any recorded (rounded) one, keep its ROC curve in fpr.json / tpr.json in the working directory."""

@@ -109,19 +109,48 @@ def ranking_dataset(bg: BaseGraph, split: int, num_neg: int, seed=0, pattern=Non
     u = pos[0].contiguous()
     w = ops.sample_tail_negatives(ep[0], ep[1], bg.num_nodes, u, k, seed=seed)
     neg = torch.stack((u.repeat_interleave(k), w.reshape(-1)))
-    pred = double(torch.cat((pos, neg), dim=1))
-    ei = bg.edge_indexs[s]
-    pos1 = torch.cat((ei.t(), pred.t()), dim=0)
     dev = ep.device
     y = torch.cat((torch.ones((2 * pos.shape[1], 1), dtype=torch.float, device=dev),
                    torch.zeros((2 * neg.shape[1], 1), dtype=torch.float, device=dev)))
+    ds = _eval_table(bg, s, torch.cat((pos, neg), dim=1), y, pattern)
+    ds.rank_k = k
+    return ds
+
+
+def _eval_table(bg: BaseGraph, s: int, pairs, y, pattern):
+    """The evaluation dataset of split s's graph with the prediction pairs `pairs` ([2, P], one column per undirected pair):
+    x = bg.x[s], ei = bg.edge_indexs[s], pos1 = [ei.T ; double(pairs).T], labels y ([2P, 1]), ei2 the wedge index of that
+    table for `pattern` (default bg.pattern)."""
+    pred = double(pairs)
+    ei = bg.edge_indexs[s]
+    pos1 = torch.cat((ei.t(), pred.t()), dim=0)
     pattern = bg.pattern if pattern is None else pattern
     if pattern in ("2wl_l", "2wl_l_implicit"):
         ei2 = (get_ei2_implicit if pattern == "2wl_l_implicit" else get_ei2)(bg.num_nodes, ei, pred)
     else:
         ei2 = None
-    ds = dataset(bg.x[s], bg.node_attr, ei, bg.edge_attrs[s], pos1, y, ei2)
-    ds.rank_k = k
+    return dataset(bg.x[s], bg.node_attr, ei, bg.edge_attrs[s], pos1, y, ei2)
+
+
+def candidate_dataset(bg: BaseGraph, split: int, src, ids, pattern=None):
+    """An evaluation table of recommended links (extension: the re-ranking half of link recommendation): the prediction pairs
+    are the valid (src[i], ids[i, j]) of TwoWL.model.train.recommend (ids >= 0), in row-major order, each doubled as preprocess
+    doubles them, on split s's graph and conventions (x = bg.x[s], ei = bg.edge_indexs[s], ei2 for `pattern`, default
+    bg.pattern) - the layout ranking_dataset builds. y is all zeros: there are no labels. The dataset carries cand_ids (ids) and
+    cand_mask ([Q, k] bool, the valid entries); TwoWL.model.train.rerank scores it. split may be 0, 1 or 2."""
+    s = int(split)
+    if s not in (0, 1, 2):
+        raise ValueError(f"candidate_dataset: split must be 0, 1 or 2, got {split}")
+    if not hasattr(bg, "edge_indexs") or not isinstance(bg.x, (list, tuple)):
+        raise ValueError("candidate_dataset: run bg.preprocess() and bg.setPosDegreeFeature() first")
+    src = src.reshape(-1).to(torch.int64)
+    if ids.dim() != 2 or ids.shape[0] != src.numel():
+        raise ValueError(f"candidate_dataset: ids must be [Q, k] with Q = {src.numel()} sources, got {tuple(ids.shape)}")
+    mask = ids >= 0
+    pairs = torch.stack((src.unsqueeze(1).expand_as(ids)[mask], ids[mask]))
+    y = torch.zeros((2 * pairs.shape[1], 1), dtype=torch.float, device=ids.device)
+    ds = _eval_table(bg, s, pairs, y, pattern)
+    ds.cand_ids, ds.cand_mask = ids, mask
     return ds
 
 

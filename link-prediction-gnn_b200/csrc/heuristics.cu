@@ -127,18 +127,21 @@ struct HeurAcc {
   double aa, ra;
 };
 
+// adds the terms of one common neighbour of degree d >= 1: Adamic-Adar 1 / ln d (0 for d = 1) and resource allocation 1 / d.
+// The pair scores (probe) and the recommendations (k_rec_runs) both add them here, so the two ops see the same term bits.
+__device__ __forceinline__ void heur_add(int64_t d, HeurAcc& acc) {
+  acc.cnt += 1;
+  acc.aa += d > 1 ? 1.0 / log((double)d) : 0.0;
+  acc.ra += 1.0 / (double)d;
+}
+
 // probes S[j] for j = j0, j0 + step, ... < j1 into L[lo, hi). S is sorted, so each probe starts where the last one ended.
 __device__ __forceinline__ void probe(const int64_t* __restrict__ ptr, const int32_t* __restrict__ S, int j0, int j1, int step,
                                       const int32_t* __restrict__ L, int lo, int hi, HeurAcc& acc) {
   for (int j = j0; j < j1; j += step) {
     const int32_t x = __ldg(S + j);
     lo = lower_bound_i32(L, lo, hi, x);
-    if (lo < hi && __ldg(L + lo) == x) {
-      const int64_t d = __ldg(ptr + x + 1) - __ldg(ptr + x);   // >= 1: x is a neighbour
-      acc.cnt += 1;
-      acc.aa += d > 1 ? 1.0 / log((double)d) : 0.0;
-      acc.ra += 1.0 / (double)d;
-    }
+    if (lo < hi && __ldg(L + lo) == x) heur_add(__ldg(ptr + x + 1) - __ldg(ptr + x), acc);   // d >= 1: x is a neighbour
   }
 }
 
@@ -258,6 +261,269 @@ __global__ void __launch_bounds__(kHeurThreads) k_lh_pairs(const int64_t* __rest
   }
 }
 
+// ---------------------------------------------------------------- link recommendation ---------------
+// The candidates of a source s are its two-hop non-neighbours. One batch of queries [q_begin, q_end), with M expansion entries:
+//   expand   for j in the batch, w in N(s_j) ascending, v in N(w) ascending: entry e = (v, w), at the query's offset. The
+//            batch's neighbour lists are cut into tiles of kRecTile; a CTA takes a tile, scans its degrees and writes the
+//            tile's entries flat, so a hub's row and a hub neighbour's long list both spread over the whole CTA.
+//   sort     stably by v, then stably by the query: entries ordered by (query, v, e), so each (query, v) run lists its
+//            common neighbours w in ascending order.
+//   runs     the head of a run drops v = s and v in N(s) (binary search), else sums its w terms in order, one thread per
+//            run, and keys the run by its chosen score (descending: the complement of the fp32 bits, every score > 0).
+//   top-k    stably by that key, then stably by the query: each query's runs in (score descending, v ascending) order.
+//            Query j's rows are the first k entries of its segment, found by binary search.
+// Every position is a uint32, so a batch holds fewer than 2^31 entries. No floating-point atomics; the order of every sum is
+// fixed by the sorts, which are stable: the result is bitwise repeatable and does not depend on how queries are batched.
+constexpr int kRecThreads = 256;
+constexpr int kRecTile = kRecThreads;                  // neighbours of a source per expansion tile
+constexpr uint32_t kRecDead = 0xffffffffu;             // score key of an entry that is not a kept run head
+
+__device__ __forceinline__ int64_t deg_of(const int64_t* __restrict__ ptr, int64_t x) { return __ldg(ptr + x + 1) - __ldg(ptr + x); }
+
+// largest i in [0, n) with off[i] - base <= x, given off[0] - base <= x
+__device__ __forceinline__ int64_t last_le(const int64_t* __restrict__ off, int64_t n, int64_t base, int64_t x) {
+  int64_t lo = 0, hi = n - 1;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi + 1) >> 1;
+    if (off[mid] - base <= x)
+      lo = mid;
+    else
+      hi = mid - 1;
+  }
+  return lo;
+}
+
+// first position in [0, n) of the ascending keys with keys[pos] >= x
+__device__ __forceinline__ int64_t lower_bound_u32(const uint32_t* __restrict__ keys, int64_t n, uint32_t x) {
+  int64_t lo = 0, hi = n;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (keys[mid] < x)
+      lo = mid + 1;
+    else
+      hi = mid;
+  }
+  return lo;
+}
+
+__device__ __forceinline__ int64_t warp_sum_l(int64_t v) {
+#pragma unroll
+  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+// exclusive scan of one value per thread over the CTA; *total = the CTA's sum. sm: kRecThreads / 32 + 1 slots.
+__device__ __forceinline__ int64_t block_exclusive_scan_l(int64_t v, int64_t* total, int64_t* sm) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int64_t inc = v;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int64_t o = __shfl_up_sync(0xffffffffu, inc, d);
+    if (lane >= d) inc += o;
+  }
+  if (lane == 31) sm[warp] = inc;
+  __syncthreads();
+  if (warp == 0) {
+    const int64_t w = lane < kRecThreads / 32 ? sm[lane] : 0;
+    int64_t winc = w;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int64_t o = __shfl_up_sync(0xffffffffu, winc, d);
+      if (lane >= d) winc += o;
+    }
+    if (lane < kRecThreads / 32) sm[lane] = winc - w;
+    if (lane == kRecThreads / 32 - 1) sm[kRecThreads / 32] = winc;
+  }
+  __syncthreads();
+  const int64_t res = sm[warp] + inc - v;
+  *total = sm[kRecThreads / 32];
+  __syncthreads();
+  return res;
+}
+
+// one warp per query: xcount[q] = X(s) = sum of d(w) over w in N(s), 0 for a bad id; info[0] += bad ids
+__global__ void __launch_bounds__(kRecThreads) k_rec_plan(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj, int64_t N,
+                                                          const int64_t* __restrict__ src, int64_t s_src, int64_t Q,
+                                                          int64_t* __restrict__ xcount, unsigned long long* __restrict__ info) {
+  const int lane = threadIdx.x & 31;
+  for (int64_t q = (int64_t)blockIdx.x * (kRecThreads / 32) + (threadIdx.x >> 5); q < Q; q += (int64_t)gridDim.x * (kRecThreads / 32)) {
+    const int64_t s = src[q * s_src];
+    const bool ok = id_ok(s, N);
+    int64_t x = 0;
+    if (ok)
+      for (int64_t i = ptr[s] + lane, e = ptr[s + 1]; i < e; i += 32) x += deg_of(ptr, __ldg(adj + i));
+    x = warp_sum_l(x);
+    if (lane == 0) {
+      xcount[q] = x;
+      if (!ok) atomicAdd(info, 1ull);
+    }
+  }
+}
+
+// tile_cnt[j] = ceil(d(s_j) / kRecTile) for the batch's queries
+__global__ void __launch_bounds__(kRecThreads) k_rec_tiles(const int64_t* __restrict__ ptr, const int64_t* __restrict__ src, int64_t s_src,
+                                                           int64_t Qb, int64_t* __restrict__ tile_cnt) {
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < Qb; j += (int64_t)gridDim.x * blockDim.x)
+    tile_cnt[j] = (deg_of(ptr, src[j * s_src]) + kRecTile - 1) / kRecTile;
+}
+
+struct RecTile {
+  int64_t s, first;   // the source, and the position in N(s) of the tile's first neighbour
+  int n;              // neighbours in the tile
+};
+
+// tile `it` < tile_off[Qb]: query = the last j with tile_off[j] <= it
+__device__ __forceinline__ RecTile rec_tile(const int64_t* __restrict__ ptr, const int64_t* __restrict__ src, int64_t s_src, int64_t Qb,
+                                            const int64_t* __restrict__ tile_off, int64_t it) {
+  const int64_t j = last_le(tile_off, Qb, 0, it);
+  RecTile t;
+  t.s = src[j * s_src];
+  t.first = (it - tile_off[j]) * kRecTile;
+  const int64_t rest = deg_of(ptr, t.s) - t.first;
+  t.n = (int)(rest < kRecTile ? rest : kRecTile);
+  return t;
+}
+
+// one CTA per tile: tile_sum[it] = the number of entries the tile expands to (0 for it >= the batch's tile count)
+__global__ void __launch_bounds__(kRecThreads) k_rec_tile_sums(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj,
+                                                               const int64_t* __restrict__ src, int64_t s_src, int64_t Qb,
+                                                               const int64_t* __restrict__ tile_off, int64_t n_items,
+                                                               int64_t* __restrict__ tile_sum) {
+  __shared__ int64_t sm[kRecThreads / 32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t n_tiles = tile_off[Qb];
+  for (int64_t it = blockIdx.x; it < n_items; it += gridDim.x) {
+    int64_t x = 0;
+    if (it < n_tiles) {
+      const RecTile t = rec_tile(ptr, src, s_src, Qb, tile_off, it);
+      if ((int)threadIdx.x < t.n) x = deg_of(ptr, __ldg(adj + ptr[t.s] + t.first + threadIdx.x));
+    }
+    x = warp_sum_l(x);
+    if (lane == 0) sm[warp] = x;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      int64_t tot = 0;
+#pragma unroll
+      for (int w = 0; w < kRecThreads / 32; ++w) tot += sm[w];
+      tile_sum[it] = tot;
+    }
+    __syncthreads();
+  }
+}
+
+// one CTA per tile: entry base + x of the tile = (v, w) with w the tile's neighbour whose list covers x; key = v, val = entry
+__global__ void __launch_bounds__(kRecThreads) k_rec_expand(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj,
+                                                            const int64_t* __restrict__ src, int64_t s_src, int64_t Qb,
+                                                            const int64_t* __restrict__ tile_off, const int64_t* __restrict__ tile_base,
+                                                            uint32_t* __restrict__ key, uint32_t* __restrict__ val,
+                                                            uint32_t* __restrict__ V, uint32_t* __restrict__ W) {
+  __shared__ int64_t off[kRecThreads], nb[kRecThreads], sm[kRecThreads / 32 + 1];
+  __shared__ int32_t wid[kRecThreads];
+  const int64_t n_tiles = tile_off[Qb];
+  for (int64_t it = blockIdx.x; it < n_tiles; it += gridDim.x) {
+    const RecTile t = rec_tile(ptr, src, s_src, Qb, tile_off, it);
+    int64_t dw = 0;
+    if ((int)threadIdx.x < t.n) {
+      const int32_t w = __ldg(adj + ptr[t.s] + t.first + threadIdx.x);
+      wid[threadIdx.x] = w;
+      nb[threadIdx.x] = ptr[w];
+      dw = ptr[w + 1] - nb[threadIdx.x];
+    }
+    int64_t total;
+    off[threadIdx.x] = block_exclusive_scan_l(dw, &total, sm);   // ends in a barrier: off / wid / nb are visible
+    __syncthreads();
+    const int64_t base = tile_base[it];
+    for (int64_t x = threadIdx.x; x < total; x += kRecThreads) {
+      int lo = 0, hi = kRecThreads - 1;                           // the last neighbour whose offset is <= x (it has d > 0)
+      while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (off[mid] <= x)
+          lo = mid;
+        else
+          hi = mid - 1;
+      }
+      const uint32_t v = (uint32_t)__ldg(adj + nb[lo] + (x - off[lo]));
+      const int64_t e = base + x;
+      key[e] = v, V[e] = v, W[e] = (uint32_t)wid[lo], val[e] = (uint32_t)e;
+    }
+    __syncthreads();
+  }
+}
+
+// after the sort by v (val = entry): key = the entry's batch-local query (the last j with exp_off[j] - exp_off[0] <= entry)
+__global__ void __launch_bounds__(kRecThreads) k_rec_qkeys(const uint32_t* __restrict__ ent, int64_t M, const int64_t* __restrict__ exp_off,
+                                                           int64_t Qb, uint32_t* __restrict__ key, uint32_t* __restrict__ val) {
+  const int64_t base = exp_off[0];
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < M; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint32_t e = ent[i];
+    key[i] = (uint32_t)last_le(exp_off, Qb, base, e);
+    val[i] = e;
+  }
+}
+
+// entries in (query, v, e) order: qk = query, ent = entry. A kept run head r gets the run's scores sc[r] and the key of the
+// chosen score; every other position the key kRecDead. key / val feed the sort by score (val = position).
+__global__ void __launch_bounds__(kRecThreads) k_rec_runs(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj,
+                                                          const int64_t* __restrict__ src, int64_t s_src, const uint32_t* __restrict__ qk,
+                                                          const uint32_t* __restrict__ ent, const uint32_t* __restrict__ V,
+                                                          const uint32_t* __restrict__ W, int64_t M, int by, float4* __restrict__ sc,
+                                                          uint32_t* __restrict__ key, uint32_t* __restrict__ val) {
+  for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < M; r += (int64_t)gridDim.x * blockDim.x) {
+    const uint32_t j = qk[r], v = V[ent[r]];
+    uint32_t k = kRecDead;
+    if (r == 0 || qk[r - 1] != j || V[ent[r - 1]] != v) {
+      const int64_t s = src[(int64_t)j * s_src];
+      const int64_t ps = ptr[s], ds = ptr[s + 1] - ps;
+      const int lo = lower_bound_i32(adj + ps, 0, (int)ds, (int32_t)v);
+      if ((int64_t)v != s && !(lo < ds && __ldg(adj + ps + lo) == (int32_t)v)) {
+        HeurAcc acc{0, 0.0, 0.0};
+        for (int64_t q = r; q < M && qk[q] == j && V[ent[q]] == v; ++q) heur_add(deg_of(ptr, W[ent[q]]), acc);   // w ascending
+        const int64_t den = ds + deg_of(ptr, v) - acc.cnt;
+        const float cn = (float)acc.cnt;
+        const float4 o = make_float4(cn, den > 0 ? __fdiv_rn(cn, (float)den) : 0.f, __double2float_rn(acc.aa),
+                                     __double2float_rn(acc.ra));
+        sc[r] = o;
+        k = ~__float_as_uint(by == 0 ? o.x : by == 1 ? o.y : by == 2 ? o.z : o.w);
+      }
+    }
+    key[r] = k;
+    val[r] = (uint32_t)r;
+  }
+}
+
+// after the sort by score key (skey, pos): key = the query of a kept run, Qb (last) for the rest; val = position
+__global__ void __launch_bounds__(kRecThreads) k_rec_jkeys(const uint32_t* __restrict__ skey, const uint32_t* __restrict__ pos,
+                                                           const uint32_t* __restrict__ qk, int64_t M, uint32_t Qb,
+                                                           uint32_t* __restrict__ key, uint32_t* __restrict__ val) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < M; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint32_t p = pos[i];
+    key[i] = skey[i] != kRecDead ? qk[p] : Qb;
+    val[i] = p;
+  }
+}
+
+// one thread per output slot (j, t): the t-th run of query j's segment in the final order, or padding (-1, NaN)
+__global__ void __launch_bounds__(kRecThreads) k_rec_out(const uint32_t* __restrict__ fkey, const uint32_t* __restrict__ fpos, int64_t M,
+                                                         const uint32_t* __restrict__ ent, const uint32_t* __restrict__ V,
+                                                         const float4* __restrict__ sc, int64_t Qb, int64_t k, int64_t q_begin, int64_t QK,
+                                                         int64_t* __restrict__ ids, float* __restrict__ scores) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < Qb * k; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t j = i / k, t = i - j * k;
+    const int64_t lo = lower_bound_u32(fkey, M, (uint32_t)j), hi = lower_bound_u32(fkey, M, (uint32_t)j + 1);
+    const int64_t o = q_begin * k + i;
+    if (lo + t < hi) {
+      const uint32_t r = fpos[lo + t];
+      const float4 s = sc[r];
+      ids[o] = V[ent[r]];
+      scores[o] = s.x, scores[QK + o] = s.y, scores[2 * QK + o] = s.z, scores[3 * QK + o] = s.w;
+    } else {
+      const float nan = __int_as_float(0x7fc00000);
+      ids[o] = -1;
+      scores[o] = nan, scores[QK + o] = nan, scores[2 * QK + o] = nan, scores[3 * QK + o] = nan;
+    }
+  }
+}
+
 }  // namespace twowl
 
 using namespace twowl;
@@ -352,6 +618,94 @@ extern "C" int twowl_link_heuristics(const int64_t* ptr, const int32_t* adj, int
     TW_LAUNCH_CHECK();
   }
   k_lh_pairs<<<grid_for(P, kHeurGroups), kHeurThreads, 0, s>>>(ptr, adj, num_nodes, u, s_u, v, s_v, P, chunk_off, p_cnt, p_aa, p_ra, out);
+  TW_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" size_t twowl_recommend_plan_workspace_bytes(int64_t Q) { return scan_workspace_bytes(Q > 0 ? Q : 1); }
+
+extern "C" int twowl_recommend_plan(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* src, int64_t s_src, int64_t Q,
+                                    int64_t* exp_off, int64_t* info, void* ws, size_t ws_bytes, void* stream) {
+  TW_CHECK_ARG(Q >= 0 && Q < 0x7fffffffLL && num_nodes >= 0 && num_nodes < 0x7fffffffLL,
+               "recommend_plan: bad sizes (0 <= Q < 2^31, 0 <= num_nodes < 2^31 - 1)");
+  TW_CHECK_ARG(ptr && exp_off && info && (Q == 0 || src), "recommend_plan: null pointer");   // adj: NULL when nnz = 0
+  TW_CHECK_WS(ws_bytes, twowl_recommend_plan_workspace_bytes(Q));
+  cudaStream_t s = (cudaStream_t)stream;
+  TW_CUDA(cudaMemsetAsync(info, 0, 2 * sizeof(int64_t), s));
+  if (Q > 0) {
+    k_rec_plan<<<grid_for(Q, kRecThreads / 32), kRecThreads, 0, s>>>(ptr, adj, num_nodes, src, s_src, Q, exp_off,
+                                                                     reinterpret_cast<unsigned long long*>(info));
+    TW_LAUNCH_CHECK();
+  }
+  if (int rc = scan_exclusive_i64(exp_off, exp_off, Q, ws, s)) return rc;
+  TW_CUDA(cudaMemcpyAsync(info + 1, exp_off + Q, sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
+  return 0;
+}
+
+// expansion tiles of a batch: at most one partial tile per query plus M / kRecTile full ones (each neighbour w has d(w) >= 1)
+static int64_t rec_items(int64_t M, int64_t Qb) { return Qb + cdiv(M, kRecTile); }
+
+extern "C" size_t twowl_recommend_workspace_bytes(int64_t n_entries, int64_t n_queries) {
+  const int64_t M = n_entries > 0 ? n_entries : 1, Qb = n_queries > 0 ? n_queries : 1, T = rec_items(M, Qb);
+  return 7 * align_up((size_t)M * sizeof(uint32_t)) + align_up((size_t)M * sizeof(float4)) + align_up(radix_workspace_bytes(M)) +
+         align_up((size_t)(Qb + 1) * sizeof(int64_t)) + align_up(scan_workspace_bytes(Qb)) + align_up((size_t)(T + 1) * sizeof(int64_t)) +
+         align_up(scan_workspace_bytes(T));
+}
+
+extern "C" int twowl_recommend(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* src, int64_t s_src, int64_t Q,
+                               int64_t q_begin, int64_t q_end, const int64_t* exp_off, int64_t n_entries, int32_t by, int64_t k,
+                               int64_t* ids, float* scores, void* ws, size_t ws_bytes, void* stream) {
+  TW_CHECK_ARG(Q >= 0 && Q < 0x7fffffffLL && num_nodes >= 0 && num_nodes < 0x7fffffffLL && 0 <= q_begin && q_begin <= q_end && q_end <= Q,
+               "recommend: bad sizes (0 <= q_begin <= q_end <= Q < 2^31, 0 <= num_nodes < 2^31 - 1)");
+  TW_CHECK_ARG(k >= 1 && k < 0x7fffffffLL && Q * k < (1LL << 60), "recommend: k must be in [1, 2^31) with Q * k < 2^60");
+  TW_CHECK_ARG(by >= 0 && by < 4, "recommend: by must be 0 (cn), 1 (jaccard), 2 (aa) or 3 (ra)");
+  TW_CHECK_ARG(n_entries >= 0 && n_entries < 0x80000000LL, "recommend: a batch must expand to 0 <= n_entries < 2^31 entries");
+  TW_CHECK_ARG(ptr && exp_off && ids && scores && (q_begin == q_end || src) && (n_entries == 0 || adj), "recommend: null pointer");
+  const int64_t Qb = q_end - q_begin, M = n_entries;
+  TW_CHECK_WS(ws_bytes, twowl_recommend_workspace_bytes(M, Qb));
+  if (Qb == 0) return 0;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t* bsrc = src + q_begin * s_src;
+  const int64_t* boff = exp_off + q_begin;
+  Carver c(ws);
+  uint32_t* A = c.take<uint32_t>(M);
+  uint32_t* B = c.take<uint32_t>(M);
+  uint32_t* C = c.take<uint32_t>(M);
+  uint32_t* D = c.take<uint32_t>(M);
+  uint32_t* V = c.take<uint32_t>(M);
+  uint32_t* W = c.take<uint32_t>(M);
+  uint32_t* F = c.take<uint32_t>(M);
+  float4* SC = c.take<float4>(M);
+  void* rws = c.take<char>(radix_workspace_bytes(M));
+  int64_t* tile_off = c.take<int64_t>(Qb + 1);
+  void* tws = c.take<char>(scan_workspace_bytes(Qb));
+  const int64_t T = rec_items(M, Qb);
+  int64_t* tile_base = c.take<int64_t>(T + 1);
+  void* bws = c.take<char>(scan_workspace_bytes(T));
+  if (M > 0) {
+    k_rec_tiles<<<grid_for(Qb, kRecThreads), kRecThreads, 0, s>>>(ptr, bsrc, s_src, Qb, tile_off);
+    TW_LAUNCH_CHECK();
+    if (int rc = scan_exclusive_i64(tile_off, tile_off, Qb, tws, s)) return rc;
+    k_rec_tile_sums<<<grid_for(T, 1), kRecThreads, 0, s>>>(ptr, adj, bsrc, s_src, Qb, tile_off, T, tile_base);
+    TW_LAUNCH_CHECK();
+    if (int rc = scan_exclusive_i64(tile_base, tile_base, T, bws, s)) return rc;
+    k_rec_expand<<<grid_for(T, 1), kRecThreads, 0, s>>>(ptr, adj, bsrc, s_src, Qb, tile_off, tile_base, A, B, V, W);
+    TW_LAUNCH_CHECK();
+    const int grid = grid_for(M, kRecThreads);
+    // (query, v, entry) order: stably by v, then stably by the query
+    if (int rc = radix_sort_pairs(A, B, C, D, M, bits_for_value(num_nodes - 1), rws, s)) return rc;   // C = v, D = entry
+    k_rec_qkeys<<<grid, kRecThreads, 0, s>>>(D, M, boff, Qb, A, B);
+    TW_LAUNCH_CHECK();
+    if (int rc = radix_sort_pairs(A, B, C, D, M, bits_for_value(Qb - 1), rws, s)) return rc;          // C = query, D = entry
+    k_rec_runs<<<grid, kRecThreads, 0, s>>>(ptr, adj, bsrc, s_src, C, D, V, W, M, by, SC, A, B);
+    TW_LAUNCH_CHECK();
+    // (query, score descending, v) order: stably by the score key, then stably by the query (the rest last)
+    if (int rc = radix_sort_pairs(A, B, W, F, M, 32, rws, s)) return rc;                                // W = score key, F = position
+    k_rec_jkeys<<<grid, kRecThreads, 0, s>>>(W, F, C, M, (uint32_t)Qb, A, B);
+    TW_LAUNCH_CHECK();
+    if (int rc = radix_sort_pairs(A, B, W, F, M, bits_for_value(Qb), rws, s)) return rc;              // W = query, F = position
+  }
+  k_rec_out<<<grid_for(Qb * k, kRecThreads), kRecThreads, 0, s>>>(W, F, M, D, V, SC, Qb, k, q_begin, Q * k, ids, scores);
   TW_LAUNCH_CHECK();
   return 0;
 }

@@ -11,6 +11,7 @@ import ctypes
 import os
 from typing import Optional, Tuple
 
+import numpy as np
 import torch
 
 from ._lib import ConvArgs, SegArgs, check, lib
@@ -1204,3 +1205,72 @@ def link_heuristics(ptr: torch.Tensor, adj: torch.Tensor, u: torch.Tensor, v: to
                                     out.data_ptr(), ws.data_ptr(), nb, _stream()), "link_heuristics")
     _count(5 + 2)
     return out
+
+
+RECOMMEND_MAX_ENTRIES = 1 << 26   # default expansion budget of one batch: 44 B of workspace per entry, about 3 GB
+
+
+def _sort_launches(bits: int) -> int:
+    """Launches of one radix_sort_pairs: histogram, 3-kernel scan and scatter per 8-bit pass, two copies after an even count."""
+    p = max(1, (max(1, bits) + 7) // 8)
+    return 5 * p + 2 * (1 - p % 2)
+
+
+def recommend_links(ptr: torch.Tensor, adj: torch.Tensor, src: torch.Tensor, k: int, by: str = "aa",
+                    max_entries: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Each source's top-k link candidates over a simple adjacency (simple_adjacency) -> (ids int64 [Q, k], scores fp32 [4, Q, k]).
+
+    The candidates of s are its two-hop non-neighbours {v != s : v not in N(s), N(s) ∩ N(v) non-empty}; any other node scores 0
+    under every heuristic. Row q holds the top min(k, #candidates) of src[q] ordered by the heuristic `by` (one of HEURISTICS)
+    descending, ties by id ascending, then -1 ids and NaN scores. scores[j] is heuristic HEURISTICS[j] of each returned pair, as
+    link_heuristics defines it, except that aa and ra are summed in double over the common neighbours in ascending id order, one
+    at a time: a sequential numpy sum reproduces cn, jaccard and ra bit for bit.
+
+    The work of a source is its expansion X(s) = sum of d(w) over w in N(s). The queries run in consecutive batches of at most
+    max_entries expansion entries (default RECOMMEND_MAX_ENTRIES); a source that expands to more runs alone. The result is
+    bitwise repeatable and does not depend on max_entries. One host read (the plan); raises IndexError when a source id lies
+    outside [0, N) and ValueError for an unknown `by` or k < 1."""
+    if by not in HEURISTICS:
+        raise ValueError(f"recommend_links: by must be one of {HEURISTICS}, got {by!r}")
+    k = int(k)
+    if k < 1:
+        raise ValueError(f"recommend_links: k must be >= 1, got {k}")
+    budget = RECOMMEND_MAX_ENTRIES if max_entries is None else max(1, int(max_entries))
+    _need_cuda(ptr, adj, src)
+    assert ptr.dim() == 1 and ptr.dtype == torch.int64 and ptr.is_contiguous(), "recommend_links: ptr must be contiguous int64 [N+1]"
+    assert adj.dim() == 1 and adj.dtype == torch.int32 and adj.is_contiguous(), "recommend_links: adj must be contiguous int32"
+    src = src.reshape(-1).to(torch.int64)
+    dev, n, Q = ptr.device, ptr.numel() - 1, src.numel()
+    ps, ss = _row(src) if Q else (0, 1)
+    exp_off = torch.empty(Q + 1, dtype=torch.int64, device=dev)
+    info = torch.empty(2, dtype=torch.int64, device=dev)
+    nb = lib.twowl_recommend_plan_workspace_bytes(Q)
+    ws = _ws(nb, dev)
+    check(lib.twowl_recommend_plan(ptr.data_ptr(), adj.data_ptr(), n, ps, ss, Q, exp_off.data_ptr(), info.data_ptr(), ws.data_ptr(),
+                                   nb, _stream()), "recommend_plan")
+    _count(6)
+    host = torch.cat((info, exp_off)).cpu().numpy()
+    if host[0]:
+        raise IndexError(f"recommend_links: {int(host[0])} source id(s) outside [0, {n})")
+    off = host[2:]
+    batches, q = [], 0
+    while q < Q:   # consecutive queries while the expansion stays within the budget; at least one query per batch
+        e = min(Q, max(q + 1, int(np.searchsorted(off, off[q] + budget, side="right")) - 1))
+        batches.append((q, e, int(off[e] - off[q])))
+        q = e
+    ids = torch.empty((Q, k), dtype=torch.int64, device=dev)
+    scores = torch.empty((4, Q, k), dtype=torch.float32, device=dev)
+    if not batches:
+        return ids, scores
+    nb = lib.twowl_recommend_workspace_bytes(max(b[2] for b in batches), max(b[1] - b[0] for b in batches))
+    ws = _ws(nb, dev)
+    j_by = HEURISTICS.index(by)
+    for q0, q1, m in batches:
+        check(lib.twowl_recommend(ptr.data_ptr(), adj.data_ptr(), n, ps, ss, Q, q0, q1, exp_off.data_ptr(), m, j_by, k, ids.data_ptr(),
+                                  scores.data_ptr(), ws.data_ptr(), nb, _stream()), "recommend")
+        if m:   # expansion (9 launches), three small kernels between and after the four sorts
+            qb = q1 - q0
+            _count(12 + _sort_launches((n - 1).bit_length()) + _sort_launches((qb - 1).bit_length()) + _sort_launches(32)
+                   + _sort_launches(qb.bit_length()))
+        _count(1)
+    return ids, scores
