@@ -540,6 +540,35 @@ int twowl_recommend(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, c
                     int64_t q_begin, int64_t q_end, const int64_t* exp_off, int64_t n_entries, int32_t by, int64_t k, int64_t* ids,
                     float* scores, void* ws, size_t ws_bytes, void* stream);
 
+/* Global link-prediction heuristics over a simple adjacency (ptr, adj) of twowl_simple_adjacency, d(w) = ptr[w+1] - ptr[w]:
+ *   Katz truncated at L steps, katz(s, v) = sum_{l=1..L} beta^l (A^l)[s, v], by Horner: y_0 = 0, y_{t+1} = A diag(beta) (y_t + e_s);
+ *   personalized PageRank, pi_0 = e_s, pi_{t+1} = alpha A D^-1 pi_t + (1 - alpha) e_s (mass at an isolated node is dropped).
+ * A batch of sources is one row-major fp32 [num_nodes, ld] operand Y, column j for source src[j]. One step is twowl_seg_reduce over
+ * (ptr, adj) with its long-row plan and src_scale from twowl_walk_scale, between ping-pong operands, and twowl_walk_restart before
+ * it (Katz, value 1) or after it (PPR, value 1 - alpha). Every call below is asynchronous on `stream` and allocates nothing.
+ *   twowl_walk_scale:   scale (fp32[num_nodes]) = beta (method TWOWL_WALK_KATZ; finite, > 0) or the fp32 quotient alpha / d(w),
+ *                       0 when d(w) = 0 (TWOWL_WALK_PPR; 0 < alpha < 1).
+ *   twowl_walk_restart: Y[src[j], j] += value for j < n_cols (src int64, element stride s_src; ids outside [0, num_nodes) skipped).
+ *   twowl_walk_gather:  out[dst[i]] = Y[v[i], col[i] - c_begin] for every i < P with c_begin <= col[i] < c_end. col, v, dst are
+ *                       contiguous int64[P], col ascending (the pairs ordered by their source's column); NaN for v outside
+ *                       [0, num_nodes).
+ *   twowl_walk_topk:    rows [q_begin, q_begin + n_cols) of ids (int64[Q*k]) and scores (fp32[Q*k]): row q_begin + j holds the
+ *                       candidates v of column j's source s = src[j] - v != s, v not in N(s), Y[v, j] > 0 - the top min(k, #)
+ *                       by score descending, ties by id ascending, then -1 / NaN. Y is clobbered: the rows of s and N(s) are
+ *                       set to 0 in column j. n_cols * min(k, num_nodes) < 2^31; adj may be NULL when nnz = 0.
+ * Bitwise repeatable (no floating-point atomics); a column's result depends on nothing but that column's source. */
+#define TWOWL_WALK_KATZ 0
+#define TWOWL_WALK_PPR 1
+int twowl_walk_scale(const int64_t* ptr, int64_t num_nodes, int32_t method, float damping, float* scale, void* stream);
+int twowl_walk_restart(float* Y, int64_t ld, int64_t num_nodes, const int64_t* src, int64_t s_src, int64_t n_cols, float value,
+                       void* stream);
+int twowl_walk_gather(const float* Y, int64_t ld, int64_t num_nodes, const int64_t* col, const int64_t* v, const int64_t* dst, int64_t P,
+                      int64_t c_begin, int64_t c_end, float* out, void* stream);
+size_t twowl_walk_topk_workspace_bytes(int64_t num_nodes, int64_t n_cols, int64_t k);
+int twowl_walk_topk(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, float* Y, int64_t ld, const int64_t* src, int64_t s_src,
+                    int64_t n_cols, int64_t k, int64_t Q, int64_t q_begin, int64_t* ids, float* scores, void* ws, size_t ws_bytes,
+                    void* stream);
+
 /* ------------------------------------------------------------------ structured wedge path ------- */
 
 /* When ei2 is the full wedge join of (pos_edge, pred_edge) minus the wedges whose source edge is blocked

@@ -155,6 +155,31 @@ def heuristic_scores(dataset):
 
 
 @torch.no_grad()
+def global_heuristic_scores(dataset, by="katz", **params):
+    """A global link-prediction heuristic of the dataset's prediction pairs (extension: the path-based baselines of SEAL's table)
+    -> fp32 [P]: truncated Katz (by="katz") or personalized PageRank (by="ppr") of each undirected pair pos1[E::2], rooted at its
+    first endpoint, in the order of test() / test_ranking(), over the split's graph read exactly as heuristic_scores reads it.
+    params (steps, damping, max_cols) go to ops.global_heuristics. rank_scores(global_heuristic_scores(ds, "ppr"), ds) ranks it
+    like a model."""
+    from twowl_b200 import graph
+    n_edges = dataset.ei.shape[1]
+    ptr, adj = graph.simple_adjacency(dataset.ei, dataset.x.shape[0])
+    pairs = dataset.pos1[n_edges::2][: dataset.y.shape[0] // 2]
+    return ops.global_heuristics(ptr, adj, pairs[:, 0], pairs[:, 1], by=by, **params)
+
+
+@torch.no_grad()
+def recommend_global(dataset, src, k=100, by="ppr", **params):
+    """Link recommendation beyond two hops -> (ids int64 [Q, k], scores fp32 [Q, k]): each source's top-k non-neighbours by
+    personalized PageRank (by="ppr") or truncated Katz (by="katz") over the split's graph, as recommend() reads it
+    (ops.recommend_global; -1 / NaN pad a row with fewer candidates). The ids feed
+    TwoWL.operators.datasets.candidate_dataset and rerank() as recommend()'s do."""
+    from twowl_b200 import graph
+    ptr, adj = graph.simple_adjacency(dataset.ei, dataset.x.shape[0])
+    return ops.recommend_global(ptr, adj, src, k, by=by, **params)
+
+
+@torch.no_grad()
 def recommend(dataset, src, k=100, by="aa"):
     """Link recommendation (extension: the retrieval half of a re-ranking pipeline) -> (ids int64 [Q, k], scores fp32 [4, Q, k]):
     each source's top-k two-hop non-neighbours by the heuristic `by`, over the split's message-passing graph dataset.ei read as

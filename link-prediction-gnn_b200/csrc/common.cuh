@@ -62,6 +62,12 @@ inline uint32_t drop_thresh(float p) {
 }
 inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+// radix-sort key width: the fewest bits (1 to 32) that hold every value in [0, max_value]
+inline int bits_for_value(int64_t max_value) {
+  int b = 1;
+  while (b < 32 && ((int64_t)1 << b) <= max_value) ++b;
+  return b;
+}
 
 // grid for a grid-stride kernel: enough CTAs to cover `work_items` at `per_cta`, capped at a
 // multiple of the SM count so every SM holds the same number of resident CTAs.
@@ -137,6 +143,12 @@ __device__ __forceinline__ uint32_t hash_u32(uint64_t seed, uint64_t idx) {
 // 1/(1-p) if element kept else 0
 __device__ __forceinline__ float drop_scale(uint64_t seed, uint64_t idx, uint32_t thresh, float inv_keep) {
   return hash_u32(seed, idx) >= thresh ? inv_keep : 0.f;
+}
+__device__ __forceinline__ uint32_t auc_key(float x) {
+  // ascending order-preserving map of IEEE-754 floats to uint32 (-0 and +0 share a key; NaNs sort last)
+  if (x == 0.f) x = 0.f;
+  const uint32_t u = __float_as_uint(x);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 __device__ __forceinline__ float4 f4_shfl_xor(const float4& v, int m) {
   return make_float4(__shfl_xor_sync(0xffffffffu, v.x, m), __shfl_xor_sync(0xffffffffu, v.y, m),

@@ -24,12 +24,6 @@ constexpr int kHeurWarps = kHeurThreads / 32;
 constexpr int kHeurLong = TWOWL_HEUR_LONG;
 constexpr int kHeurChunk = TWOWL_HEUR_CHUNK;
 
-static int bits_for_value(int64_t max_value) {
-  int b = 1;
-  while (b < 32 && ((int64_t)1 << b) <= max_value) ++b;
-  return b;
-}
-
 __device__ __forceinline__ int warp_sum_i(int v) { return __reduce_add_sync(0xffffffffu, v); }
 
 // ---------------------------------------------------------------- simple adjacency -----------------

@@ -19,13 +19,6 @@ namespace twowl {
 constexpr int kAucThreads = 256;
 constexpr int kAucMaxCtas = kNumSMs * 4;
 
-__device__ __forceinline__ uint32_t auc_key(float x) {
-  // ascending order-preserving map of IEEE-754 floats to uint32 (-0 and +0 share a key; NaNs sort last)
-  if (x == 0.f) x = 0.f;
-  const uint32_t u = __float_as_uint(x);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 __global__ void __launch_bounds__(kAucThreads) k_auc_keys(const float* __restrict__ score, int64_t n, uint32_t* __restrict__ keys,
                                                           uint32_t* __restrict__ vals) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {

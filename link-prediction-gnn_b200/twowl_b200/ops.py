@@ -1274,3 +1274,169 @@ def recommend_links(ptr: torch.Tensor, adj: torch.Tensor, src: torch.Tensor, k: 
                    + _sort_launches(qb.bit_length()))
         _count(1)
     return ids, scores
+
+
+# ------------------------------------------------------------------------------ global link-prediction heuristics
+
+GLOBAL_HEURISTICS = ("katz", "ppr")
+GLOBAL_DEFAULTS = {"katz": (3, 0.001), "ppr": (20, 0.85)}   # (steps, damping): SEAL's beta and alpha
+WALK_MAX_COLS = 256      # default sources per batch: the operand pair is 2 x N x 256 x 4 bytes, 2 GB at N = 1 M (DESIGN.md §0)
+# seg_reduce hands a row of more than 32 chunks to a whole CTA whose lane-group count depends on the operand width up to 68
+# columns and is fixed from there on: an operand of at least 68 columns gives every column the same bits at every batch width
+_WALK_MIN_WIDTH = 68
+_WALK_MAX_WIDTH = 1024   # seg_reduce's widest operand
+
+
+def _walk_params(fn: str, by: str, steps, damping) -> Tuple[int, float]:
+    if by not in GLOBAL_HEURISTICS:
+        raise ValueError(f"{fn}: by must be one of {GLOBAL_HEURISTICS}, got {by!r}")
+    d_steps, d_damp = GLOBAL_DEFAULTS[by]
+    steps = d_steps if steps is None else int(steps)
+    if steps < 1:
+        raise ValueError(f"{fn}: steps must be >= 1, got {steps}")
+    with np.errstate(over="ignore"):     # the recursion runs on the fp32-rounded parameter; one that overflows fp32 is refused
+        damp = float(np.float32(d_damp if damping is None else damping))
+    if by == "katz" and not (np.isfinite(damp) and damp > 0):
+        raise ValueError(f"{fn}: the Katz damping beta must be finite and > 0, got {damping}")
+    if by == "ppr" and not 0 < damp < 1:
+        raise ValueError(f"{fn}: the PageRank damping alpha must lie in (0, 1), got {damping}")
+    return steps, damp
+
+
+def _walk_cols(fn: str, max_cols) -> int:
+    b = WALK_MAX_COLS if max_cols is None else int(max_cols)
+    if not 1 <= b <= _WALK_MAX_WIDTH:
+        raise ValueError(f"{fn}: max_cols must lie in [1, {_WALK_MAX_WIDTH}], got {b}")
+    return b
+
+
+class _Walk:
+    """The operands of batched walks from up to `cols` sources over a simple adjacency: two fp32 [N, ld] buffers, ld the batch
+    width rounded up to a multiple of 4 and at least _WALK_MIN_WIDTH (columns past a batch's sources stay 0), the long-row plan
+    and the per-node scale."""
+
+    def __init__(self, ptr, adj, by: str, steps: int, damping: float, cols: int):
+        n, dev = ptr.numel() - 1, ptr.device
+        self.ptr, self.adj, self.n, self.by, self.steps, self.damping = ptr, adj, n, by, steps, damping
+        self.ld = min(_WALK_MAX_WIDTH, max(_WALK_MIN_WIDTH, -(-cols // 4) * 4))
+        self.Y = [torch.empty((n, self.ld), dtype=torch.float32, device=dev) for _ in range(2)]
+        self.plan = seg_plan(ptr, n, adj.numel())
+        self.scale = torch.empty(n, dtype=torch.float32, device=dev)
+        check(lib.twowl_walk_scale(ptr.data_ptr(), n, int(by == "ppr"), damping, self.scale.data_ptr(), _stream()), "walk_scale")
+        _count()
+
+    def _restart(self, Y, src, n_cols: int, value: float):
+        ps, ss = _row(src)
+        check(lib.twowl_walk_restart(Y.data_ptr(), self.ld, self.n, ps, ss, n_cols, value, _stream()), "walk_restart")
+        _count()
+
+    def run(self, src: torch.Tensor) -> torch.Tensor:
+        """Scores of every node from each source of src (int64, at most ld ids, all valid) -> Y: column j for src[j]."""
+        Y, Z = self.Y
+        Y.zero_()
+        n_cols = src.numel()
+        ppr = self.by == "ppr"
+        if ppr:
+            self._restart(Y, src, n_cols, 1.0)
+        for _ in range(self.steps):
+            if not ppr:
+                self._restart(Y, src, n_cols, 1.0)
+            seg_reduce(self.ptr, self.adj, self.n, Y, plan=self.plan, src_scale=self.scale, out=Z)
+            if ppr:
+                self._restart(Z, src, n_cols, float(np.float32(1) - np.float32(self.damping)))
+            Y, Z = Z, Y
+        self.Y = [Y, Z]
+        return Y
+
+
+def _check_graph(fn: str, ptr, adj):
+    assert ptr.dim() == 1 and ptr.dtype == torch.int64 and ptr.is_contiguous(), f"{fn}: ptr must be contiguous int64 [N+1]"
+    assert adj.dim() == 1 and adj.dtype == torch.int32 and adj.is_contiguous(), f"{fn}: adj must be contiguous int32"
+
+
+def global_heuristics(ptr: torch.Tensor, adj: torch.Tensor, u: torch.Tensor, v: torch.Tensor, by: str = "katz", steps: Optional[int] = None,
+                      damping: Optional[float] = None, max_cols: Optional[int] = None) -> torch.Tensor:
+    """Global (path-based) scores of the query pairs (u[i], v[i]) over a simple adjacency (simple_adjacency) -> fp32 [P], each
+    rooted at its first endpoint u[i]:
+      by="katz": sum_{l=1..steps} beta^l (A^l)[u, v], truncated Katz (default steps 3, beta = damping = 0.001);
+      by="ppr":  pi_steps[v] of personalized PageRank from u: pi_0 = e_u, pi_{t+1} = alpha A D^-1 pi_t + (1 - alpha) e_u (default
+                 steps 20, alpha = damping = 0.85); mass at an isolated node is dropped.
+    Everything runs in fp32 with the fp32-rounded damping. Katz is symmetric in exact arithmetic, but the fp32 scores of (u, v) and
+    (v, u) come from different walks and may differ in the last bits; PPR is not symmetric. A score whose paths all underflow
+    fp32 (PPR through hubs: (1 / d)^steps) is 0.
+
+    The distinct u are the walks' sources, up to max_cols (default WALK_MAX_COLS, at most 1024) per batch; each batch is `steps`
+    seg_reduce passes over the adjacency on an [N, max(68, max_cols)] operand. The result is bitwise repeatable and does not depend
+    on max_cols. One host read (the bad-id count and the number of distinct u); raises IndexError for an id outside [0, N) and
+    ValueError for an unknown `by`, steps < 1, a Katz damping that is not finite and > 0 or a PageRank damping outside (0, 1)."""
+    steps, damp = _walk_params("global_heuristics", by, steps, damping)
+    cols = _walk_cols("global_heuristics", max_cols)
+    _need_cuda(ptr, adj, u, v)
+    _check_graph("global_heuristics", ptr, adj)
+    u, v = u.reshape(-1).to(torch.int64), v.reshape(-1).to(torch.int64)
+    assert u.numel() == v.numel(), "global_heuristics: u / v size mismatch"
+    dev, n, P = ptr.device, ptr.numel() - 1, u.numel()
+    out = torch.empty(P, dtype=torch.float32, device=dev)
+    if P == 0:
+        return out
+    # the pairs ordered by source once; column c = rank of the source among the distinct u
+    us, order = torch.sort(u, stable=True)
+    new = torch.ones(P, dtype=torch.bool, device=dev)
+    new[1:] = us[1:] != us[:-1]
+    col = torch.cumsum(new, 0) - 1
+    bad = ((u < 0) | (u >= n) | (v < 0) | (v >= n)).sum()
+    nbad, U = torch.stack((bad, col[-1] + 1)).tolist()
+    if nbad:
+        raise IndexError(f"global_heuristics: {nbad} query id(s) outside [0, {n})")
+    sources = torch.zeros(P, dtype=torch.int64, device=dev).scatter_(0, col, us)[:U]
+    vs = v[order].contiguous()
+    walk = _Walk(ptr, adj, by, steps, damp, min(cols, U))
+    for c0 in range(0, U, cols):
+        c1 = min(U, c0 + cols)
+        Y = walk.run(sources[c0:c1])
+        check(lib.twowl_walk_gather(Y.data_ptr(), walk.ld, n, col.data_ptr(), vs.data_ptr(), order.data_ptr(), P, c0, c1, out.data_ptr(),
+                                    _stream()), "walk_gather")
+        _count()
+    return out
+
+
+def recommend_global(ptr: torch.Tensor, adj: torch.Tensor, src: torch.Tensor, k: int, by: str = "ppr", steps: Optional[int] = None,
+                     damping: Optional[float] = None, max_cols: Optional[int] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Each source's top-k link candidates by a global heuristic (see global_heuristics) -> (ids int64 [Q, k], scores fp32 [Q, k]).
+
+    The candidates of s are {v != s : v not in N(s), score(s, v) > 0}, at any distance: every node a walk of at most `steps` edges
+    reaches (Katz), or that keeps an fp32 share of the walk's mass (PPR). Row q holds the top min(k, #candidates) of src[q] by score
+    descending, ties by id ascending, then -1 ids and NaN scores. scores[q, j] is bit-identical to
+    global_heuristics(src[q], ids[q, j]) with the same parameters. One walk per query, in src order, max_cols per batch (duplicates
+    are walked again); the result is bitwise repeatable and independent of max_cols. One host read (the bad-id count); raises
+    IndexError for a source outside [0, N) and ValueError as global_heuristics does or for k < 1."""
+    steps, damp = _walk_params("recommend_global", by, steps, damping)
+    cols = _walk_cols("recommend_global", max_cols)
+    k = int(k)
+    if k < 1:
+        raise ValueError(f"recommend_global: k must be >= 1, got {k}")
+    _need_cuda(ptr, adj, src)
+    _check_graph("recommend_global", ptr, adj)
+    src = src.reshape(-1).to(torch.int64)
+    dev, n, Q = ptr.device, ptr.numel() - 1, src.numel()
+    ids = torch.empty((Q, k), dtype=torch.int64, device=dev)
+    scores = torch.empty((Q, k), dtype=torch.float32, device=dev)
+    if Q == 0:
+        return ids, scores
+    nbad = int(((src < 0) | (src >= n)).sum())
+    if nbad:
+        raise IndexError(f"recommend_global: {nbad} source id(s) outside [0, {n})")
+    walk = _Walk(ptr, adj, by, steps, damp, min(cols, Q))
+    nb = lib.twowl_walk_topk_workspace_bytes(n, min(cols, Q), k)
+    ws = _ws(nb, dev)
+    kk = min(k, n)
+    for q0 in range(0, Q, cols):
+        q1 = min(Q, q0 + cols)
+        Y = walk.run(src[q0:q1])
+        ps, ss = _row(src[q0:q1])
+        check(lib.twowl_walk_topk(ptr.data_ptr(), adj.data_ptr(), n, Y.data_ptr(), walk.ld, ps, ss, q1 - q0, k, Q, q0, ids.data_ptr(),
+                                  scores.data_ptr(), ws.data_ptr(), nb, _stream()), "walk_topk")
+        if kk:   # exclusion, memset, 4 x (histogram, select), count, scan, take, scan, write, two sorts with a key kernel between
+            _count(1 + 1 + 8 + 1 + 3 + 1 + 3 + 1 + _sort_launches(32) + 1 + _sort_launches((q1 - q0 - 1).bit_length()))
+        _count(1)
+    return ids, scores
