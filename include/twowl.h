@@ -569,6 +569,38 @@ int twowl_walk_topk(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, f
                     int64_t n_cols, int64_t k, int64_t Q, int64_t q_begin, int64_t* ids, float* scores, void* ws, size_t ws_bytes,
                     void* stream);
 
+/* node2vec (Grover & Leskovec 2016) over a simple adjacency (ptr, adj) of twowl_simple_adjacency. Every call below is asynchronous
+ * on `stream` and allocates nothing.
+ *   twowl_n2v_walks:  walks (int32[W*length], row i = walk i) from start[i] (int64, element stride s_start): walks[i, 0] = start[i],
+ *                     the first step uniform over N(start), then from cur with predecessor prev the next x in N(cur) with
+ *                     probability proportional to 1/p (x == prev), 1 (x in N(prev)) or 1/q (otherwise). Rejection sampling: x is
+ *                     proposed uniformly (a 32-bit multiply-high, bias at most d(cur) / 2^32) and accepted with probability
+ *                     w(x) / max(1/p, 1, 1/q) (rounded down to a multiple of 2^-32), so a step takes max(w) / min(w) trials at
+ *                     most in expectation; p = q = 1 accepts every proposal (DeepWalk). A walk from an isolated start is
+ *                     [s, -1, -1, ...]; a start outside [0, num_nodes) gives a row of -1. Every draw is hash_u32(seed, .) of
+ *                     (index_base + i, step, trial, draw): a walk depends on (seed, index_base + i, start[i]) alone.
+ *                     p, q finite and > 0 with max(w) / min(w) <= 1024; 1 <= length <= 2^24; index_base + W <= 2^40.
+ *   twowl_n2v_step:   one skip-gram step with negative sampling on emb (fp32[num_nodes*d], row-major), d a multiple of 32 in
+ *                     [32, 512]. walks int32[B*L] (-1 padding), negs int32[B*L*K]; K >= 1, window >= 1, 2 B L (window + K) < 2^31.
+ *                     Positive pairs (walks[b,i], walks[b,i+o]), 1 <= o <= window, i + o < L, both >= 0; negative pairs
+ *                     (walks[b,i], negs[b,i,j]), j < K, for each token i with a positive pair; self pairs kept. An id outside
+ *                     [0, num_nodes) counts as padding. loss[0] (double, device) = mean_pos softplus(-e_a.e_b) + mean_neg
+ *                     softplus(e_a.e_b), 0 when there is no positive pair. The rows in any pair are updated as
+ *                     torch.optim.SparseAdam updates the coalesced gradient (taken from the pre-step table) of an
+ *                     nn.Embedding(sparse=True) (lr, betas, eps in double, as torch holds them); no other row changes. step[0] (int64, device) is the step count: it is read as
+ *                     t - 1 and incremented when the batch has a positive pair. No host read; bitwise repeatable (integer atomics
+ *                     only; each row's gradient summed in a fixed order after a stable radix sort; fixed dot and loss trees).
+ *   twowl_embedding_dot: out[i] = e_u[i] . e_v[i] (u, v int64[P], element strides), the step's dot routine, so (u, v) and (v, u)
+ *                     give the same bits; NaN for an id outside [0, num_nodes). */
+int twowl_n2v_walks(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* start, int64_t s_start, int64_t W,
+                    int64_t length, float p, float q, uint64_t seed, int64_t index_base, int32_t* walks, void* stream);
+size_t twowl_n2v_step_workspace_bytes(int64_t B, int64_t L, int64_t window, int64_t K, int64_t d);
+int twowl_n2v_step(float* emb, float* exp_avg, float* exp_avg_sq, int64_t* step, int64_t num_nodes, int32_t d, const int32_t* walks,
+                   const int32_t* negs, int64_t B, int64_t L, int64_t window, int64_t K, double lr, double beta1, double beta2, double eps,
+                   double* loss, void* ws, size_t ws_bytes, void* stream);
+int twowl_embedding_dot(const float* emb, int64_t num_nodes, int32_t d, const int64_t* u, int64_t s_u, const int64_t* v, int64_t s_v,
+                        int64_t P, float* out, void* stream);
+
 /* ------------------------------------------------------------------ structured wedge path ------- */
 
 /* When ei2 is the full wedge join of (pos_edge, pred_edge) minus the wedges whose source edge is blocked

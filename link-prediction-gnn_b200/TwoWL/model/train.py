@@ -169,6 +169,26 @@ def global_heuristic_scores(dataset, by="katz", **params):
 
 
 @torch.no_grad()
+def node2vec_embedding(dataset, **params):
+    """node2vec embeddings (extension: the reference's learned baseline, SURVEY rows 7-8) -> (emb fp32 [N, dim], losses float64
+    [epochs]), trained on the device by ops.node2vec over the split's graph read exactly as heuristic_scores reads it. params (dim,
+    walk_length, walks_per_node, window, neg, p, q, epochs, batch_walks, lr, seed) go to ops.node2vec."""
+    from twowl_b200 import graph
+    ptr, adj = graph.simple_adjacency(dataset.ei, dataset.x.shape[0])
+    return ops.node2vec(ptr, adj, **params)
+
+
+@torch.no_grad()
+def embedding_scores(dataset, emb):
+    """The link score e_u . e_v of an embedding table (node2vec_embedding) for each prediction pair pos1[E::2], in the order of
+    test() -> fp32 [P] (ops.embedding_dot). rank_scores(embedding_scores(ds, emb), ds) and ops.auc(scores, ds.y[0::2]) rank it
+    like a model."""
+    n_edges = dataset.ei.shape[1]
+    pairs = dataset.pos1[n_edges::2][: dataset.y.shape[0] // 2]
+    return ops.embedding_dot(emb, pairs[:, 0], pairs[:, 1])
+
+
+@torch.no_grad()
 def recommend_global(dataset, src, k=100, by="ppr", **params):
     """Link recommendation beyond two hops -> (ids int64 [Q, k], scores fp32 [Q, k]): each source's top-k non-neighbours by
     personalized PageRank (by="ppr") or truncated Katz (by="katz") over the split's graph, as recommend() reads it

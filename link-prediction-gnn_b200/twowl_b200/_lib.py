@@ -16,7 +16,7 @@ HEADER_PATH = os.path.normpath(os.path.join(_HERE, "..", "..", "include", "twowl
 
 _CTYPES = {
     "int": ctypes.c_int32, "int32_t": ctypes.c_int32, "int64_t": ctypes.c_int64,
-    "uint64_t": ctypes.c_uint64, "size_t": ctypes.c_size_t, "float": ctypes.c_float,
+    "uint64_t": ctypes.c_uint64, "size_t": ctypes.c_size_t, "float": ctypes.c_float, "double": ctypes.c_double,
 }
 
 

@@ -1440,3 +1440,194 @@ def recommend_global(ptr: torch.Tensor, adj: torch.Tensor, src: torch.Tensor, k:
             _count(1 + 1 + 8 + 1 + 3 + 1 + 3 + 1 + _sort_launches(32) + 1 + _sort_launches((q1 - q0 - 1).bit_length()))
         _count(1)
     return ids, scores
+
+
+# ------------------------------------------------------------------------------ node2vec
+
+N2V_MAX_RATIO = 1024.0   # max(1/p, 1, 1/q) / min(1/p, 1, 1/q): the expected number of rejection trials per walk step
+N2V_MAX_DIM = 512
+
+
+def _n2v_pq(fn: str, p, q) -> Tuple[float, float]:
+    p, q = float(p), float(q)
+    if not (np.isfinite(p) and np.isfinite(q) and p > 0 and q > 0):
+        raise ValueError(f"{fn}: p and q must be finite and > 0, got p={p}, q={q}")
+    w = (1.0 / p, 1.0, 1.0 / q)
+    if max(w) / min(w) > N2V_MAX_RATIO:
+        raise ValueError(f"{fn}: max(1/p, 1, 1/q) / min(1/p, 1, 1/q) must be <= {N2V_MAX_RATIO:g} (the expected rejection trials "
+                         f"per step), got p={p}, q={q}")
+    return p, q
+
+
+def _n2v_dim(fn: str, d: int) -> int:
+    d = int(d)
+    if d < 32 or d > N2V_MAX_DIM or d % 32:
+        raise ValueError(f"{fn}: the embedding width must be a multiple of 32 in [32, {N2V_MAX_DIM}], got {d}")
+    return d
+
+
+def _n2v_walks(ptr, adj, start, length: int, p: float, q: float, seed: int, index_base: int) -> torch.Tensor:
+    """The launch of node2vec_walks without its checks (start int64 1-D, every id valid)."""
+    W, n = start.numel(), ptr.numel() - 1
+    walks = torch.empty((W, length), dtype=torch.int32, device=ptr.device)
+    if W == 0:
+        return walks
+    ps, ss = _row(start)
+    check(lib.twowl_n2v_walks(ptr.data_ptr(), adj.data_ptr(), n, ps, ss, W, length, p, q, seed & (2 ** 64 - 1), index_base,
+                              walks.data_ptr(), _stream()), "n2v_walks")
+    _count()
+    return walks
+
+
+def node2vec_walks(ptr: torch.Tensor, adj: torch.Tensor, start: torch.Tensor, length: int, p: float = 1.0, q: float = 1.0,
+                   seed: Optional[int] = None, index_base: int = 0) -> torch.Tensor:
+    """node2vec's second-order biased random walks over a simple adjacency (simple_adjacency) -> int32 [W, length], row i the walk
+    from start[i]. The first step is uniform over N(start); after it, from cur with predecessor prev, the next node x in N(cur) is
+    drawn with probability proportional to 1/p if x == prev, 1 if x is a neighbour of prev and 1/q otherwise (node2vec's transition
+    rule for an unweighted graph). A walk from an isolated start is [s, -1, -1, ...].
+
+    Sampling is by rejection (KnightKing): x is proposed uniformly from N(cur), a 32-bit multiply-high whose bias is at most
+    d(cur) / 2^32, and accepted with probability w(x) / max(w); p = q = 1 accepts every proposal (DeepWalk). The draws are
+    counter-based, keyed by (seed, index_base + i, step, trial), so a walk depends on (seed, index_base + i, start[i]) alone:
+    node2vec_walks(.., start, base=0)[a:b] equals node2vec_walks(.., start[a:b], base=a) bit for bit. seed=None takes next_seed().
+    One host read (the bad-id count); raises IndexError for a start outside [0, N) and ValueError for length < 1 or p, q that are
+    not finite and > 0 or whose weight ratio max(w) / min(w) exceeds N2V_MAX_RATIO (the expected trials per step)."""
+    p, q = _n2v_pq("node2vec_walks", p, q)
+    length = int(length)
+    if length < 1:
+        raise ValueError(f"node2vec_walks: length must be >= 1, got {length}")
+    index_base = int(index_base)
+    if index_base < 0:
+        raise ValueError(f"node2vec_walks: index_base must be >= 0, got {index_base}")
+    _need_cuda(ptr, adj, start)
+    _check_graph("node2vec_walks", ptr, adj)
+    start = start.reshape(-1).to(torch.int64)
+    n = ptr.numel() - 1
+    if start.numel():
+        nbad = int(((start < 0) | (start >= n)).sum())
+        if nbad:
+            raise IndexError(f"node2vec_walks: {nbad} start id(s) outside [0, {n})")
+    return _n2v_walks(ptr, adj, start, length, p, q, next_seed() if seed is None else int(seed), index_base)
+
+
+def _n2v_step(emb, exp_avg, exp_avg_sq, step, walks, negs, window: int, lr: float, betas, eps: float) -> torch.Tensor:
+    """The launch of node2vec_step without its id check."""
+    n, d = emb.shape
+    B, L = walks.shape
+    K = negs.shape[2]
+    loss = torch.empty((), dtype=torch.float64, device=emb.device)
+    nb = lib.twowl_n2v_step_workspace_bytes(B, L, window, K, d)
+    ws = _ws(nb, emb.device)
+    check(lib.twowl_n2v_step(emb.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), step.data_ptr(), n, d, walks.data_ptr(),
+                             negs.data_ptr(), B, L, window, K, float(lr), float(betas[0]), float(betas[1]), float(eps), loss.data_ptr(),
+                             ws.data_ptr(), nb, _stream()), "n2v_step")
+    _count(1 + (9 + _sort_launches(max(1, n).bit_length()) + 3 if B * L else 0) + 1)
+    return loss
+
+
+def _n2v_step_args(emb, exp_avg, exp_avg_sq, step, walks, negs, window):
+    _need_cuda(emb, exp_avg, exp_avg_sq, step, walks, negs)
+    assert emb.dim() == 2 and all(t.dtype == torch.float32 and t.is_contiguous() and t.shape == emb.shape for t in (emb, exp_avg, exp_avg_sq)), \
+        "node2vec_step: emb / exp_avg / exp_avg_sq must be contiguous fp32 [N, d] of one shape"
+    assert step.dtype == torch.int64 and step.numel() == 1, "node2vec_step: step must be an int64 device scalar"
+    assert walks.dim() == 2 and walks.dtype == torch.int32 and walks.is_contiguous(), "node2vec_step: walks must be contiguous int32 [B, L]"
+    assert negs.dim() == 3 and negs.dtype == torch.int32 and negs.is_contiguous() and negs.shape[:2] == walks.shape, \
+        "node2vec_step: negs must be contiguous int32 [B, L, K]"
+    _n2v_dim("node2vec_step", emb.shape[1])
+    window = int(window)
+    if window < 1:
+        raise ValueError(f"node2vec_step: window must be >= 1, got {window}")
+    if negs.shape[2] < 1:
+        raise ValueError("node2vec_step: negs must hold K >= 1 negatives per token")
+    return window
+
+
+def node2vec_step(emb: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor, step: torch.Tensor, walks: torch.Tensor,
+                  negs: torch.Tensor, window: int, lr: float = 0.01, betas=(0.9, 0.999), eps: float = 1e-8) -> torch.Tensor:
+    """One skip-gram step with negative sampling on the embedding table emb (fp32 [N, d], d a multiple of 32 up to 512), in place,
+    with lazy Adam -> the loss, a 0-dim float64 device tensor (no host read).
+
+    Positive pairs are (walks[b, i], walks[b, i + o]) for 1 <= o <= window, i + o < L, both entries >= 0 (walks int32 [B, L], -1
+    padding); negative pairs are (walks[b, i], negs[b, i, j]) for every j < K (negs int32 [B, L, K]) of each token i with at least
+    one positive pair; self pairs are kept. Loss = mean_pos softplus(-e_a . e_b) + mean_neg softplus(e_a . e_b) (PyG Node2Vec's
+    objective). The rows in any pair are updated exactly as torch.optim.SparseAdam updates the coalesced gradient of an
+    nn.Embedding(sparse=True), the gradient taken from the table before the step: exp_avg, exp_avg_sq and the int64 device scalar
+    `step` (the step count, advanced only when the batch has a positive pair) are the optimiser state. No other row changes; a
+    batch without a positive pair changes nothing and its loss is 0. Bitwise repeatable. One host read (the id check); raises
+    IndexError for an id outside [-1, N) in walks or [0, N) in negs and ValueError for d, window < 1 or K < 1."""
+    window = _n2v_step_args(emb, exp_avg, exp_avg_sq, step, walks, negs, window)
+    n = emb.shape[0]
+    if walks.numel():
+        bad = ((walks < -1) | (walks >= n)).sum()
+        if negs.numel():
+            bad = bad + ((negs < 0) | (negs >= n)).sum()
+        nbad = int(bad)
+        if nbad:
+            raise IndexError(f"node2vec_step: {nbad} id(s) outside [-1, {n}) in walks or [0, {n}) in negs")
+    return _n2v_step(emb, exp_avg, exp_avg_sq, step, walks, negs, window, lr, betas, eps)
+
+
+def embedding_dot(emb: torch.Tensor, u: torch.Tensor, v: torch.Tensor) -> torch.Tensor:
+    """Link scores of an embedding table (fp32 [N, d], d a multiple of 32 up to 512) -> fp32 [P], out[i] = e_u[i] . e_v[i], one warp
+    per pair with node2vec_step's dot routine: (u, v) and (v, u) give the same bits. One host read; raises IndexError for an id
+    outside [0, N)."""
+    _need_cuda(emb, u, v)
+    assert emb.dim() == 2 and emb.dtype == torch.float32 and emb.is_contiguous(), "embedding_dot: emb must be contiguous fp32 [N, d]"
+    d = _n2v_dim("embedding_dot", emb.shape[1])
+    u, v = u.reshape(-1).to(torch.int64), v.reshape(-1).to(torch.int64)
+    assert u.numel() == v.numel(), "embedding_dot: u / v size mismatch"
+    n, P = emb.shape[0], u.numel()
+    out = torch.empty(P, dtype=torch.float32, device=emb.device)
+    if P == 0:
+        return out
+    nbad = int(((u < 0) | (u >= n) | (v < 0) | (v >= n)).sum())
+    if nbad:
+        raise IndexError(f"embedding_dot: {nbad} id(s) outside [0, {n})")
+    (pu, su), (pv, sv) = _row(u), _row(v)
+    check(lib.twowl_embedding_dot(emb.data_ptr(), n, d, pu, su, pv, sv, P, out.data_ptr(), _stream()), "embedding_dot")
+    _count()
+    return out
+
+
+def node2vec(ptr: torch.Tensor, adj: torch.Tensor, dim: int = 128, walk_length: int = 80, walks_per_node: int = 10, window: int = 10,
+             neg: int = 1, p: float = 1.0, q: float = 1.0, epochs: int = 1, batch_walks: int = 1024, lr: float = 0.01,
+             seed: int = 0) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Train node2vec embeddings over a simple adjacency (simple_adjacency) -> (emb fp32 [N, dim], losses float64 [epochs], on the
+    device). PyG Node2Vec's mini-batch recipe: emb starts N(0, 1); each epoch walks every node walks_per_node times in an order
+    permuted by a generator seeded with `seed`, batch_walks walks at a time (node2vec_walks, index_base = the walk's index in the
+    run), draws window * neg uniform negatives per token from the same generator (neg = negatives per positive pair) and runs one
+    node2vec_step (lazy Adam, lr). losses[e] is the mean of epoch e's batch losses. The walk defaults are the node2vec paper's. No
+    host read; two calls with the same arguments return the same bits on the same device. Raises ValueError for p, q as
+    node2vec_walks does, dim as node2vec_step does, or a count < 1."""
+    p, q = _n2v_pq("node2vec", p, q)
+    dim = _n2v_dim("node2vec", dim)
+    ints = dict(walk_length=walk_length, walks_per_node=walks_per_node, window=window, neg=neg, epochs=epochs, batch_walks=batch_walks)
+    for k, val in ints.items():
+        if int(val) < 1:
+            raise ValueError(f"node2vec: {k} must be >= 1, got {val}")
+    L, R, win, K, epochs, bw = (int(ints[k]) for k in ("walk_length", "walks_per_node", "window", "neg", "epochs", "batch_walks"))
+    K *= win
+    _need_cuda(ptr, adj)
+    _check_graph("node2vec", ptr, adj)
+    dev, n = ptr.device, ptr.numel() - 1
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(int(seed))
+    emb = torch.randn((n, dim), generator=gen, device=dev)
+    exp_avg, exp_avg_sq = torch.zeros_like(emb), torch.zeros_like(emb)
+    step = torch.zeros((), dtype=torch.int64, device=dev)
+    losses = torch.zeros(epochs, dtype=torch.float64, device=dev)
+    W = n * R
+    if W == 0:
+        return emb, losses
+    nodes = torch.arange(n, device=dev).repeat(R)
+    walk_seed = int(seed) & (2 ** 62 - 1)
+    for e in range(epochs):
+        starts = nodes[torch.randperm(W, generator=gen, device=dev)]
+        total = torch.zeros((), dtype=torch.float64, device=dev)
+        for b0 in range(0, W, bw):
+            b1 = min(W, b0 + bw)
+            walks = _n2v_walks(ptr, adj, starts[b0:b1], L, p, q, walk_seed, e * W + b0)
+            negs = torch.randint(0, n, (b1 - b0, L, K), generator=gen, device=dev, dtype=torch.int32)
+            total += _n2v_step(emb, exp_avg, exp_avg_sq, step, walks, negs, win, lr, (0.9, 0.999), 1e-8)
+        losses[e] = total / -(-W // bw)
+    return emb, losses
