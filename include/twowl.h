@@ -155,14 +155,13 @@ int twowl_narrow_i32(const int64_t* in, int64_t stride, int64_t n, int32_t* out,
  * i.e. self-loops removed, one self-loop added. A CSR row r with row_skip_mask[r] set counts as empty. */
 int twowl_gcn_dinv(const int64_t* ptr, const int32_t* col, int64_t M, int32_t flip, int32_t row_flip,
                    const uint8_t* skip_mask, const uint8_t* row_skip_mask, float* dinv, void* stream);
-/* same with entries removed by a per-ENTRY mask (entry_mask[k] != 0: entry k of the CSR does not exist) - the node graph
- * of one training step is the cached CSR of the whole graph minus the sampled edges (sample_block, utils.py:61-64). */
-int twowl_gcn_dinv_entries(const int64_t* ptr, const int32_t* col, int64_t M, const uint8_t* entry_mask, float* dinv,
-                           void* stream);
-/* the same for the node rows [row_lo, row_hi) only (dinv keeps its [M] shape; the rest is untouched): one rank's node block of a
- * row-sharded step, which then all-gathers the blocks (twowl_b200.rowshard). Only entry_mask[ptr[row_lo] .. ptr[row_hi]) is read. */
-int twowl_gcn_dinv_entries_rows(const int64_t* ptr, const int32_t* col, int64_t M, const uint8_t* entry_mask, int64_t row_lo,
-                                int64_t row_hi, float* dinv, void* stream);
+/* the same (no flips, no skip masks) with entries removed by a per-ENTRY mask (entry_mask[k] != 0: entry k of the CSR does not
+ * exist) - the node graph of one training step is the cached CSR of the whole graph minus the sampled edges (sample_block,
+ * utils.py:61-64) - for the node rows [row_lo, row_hi) only: dinv keeps its [M] shape and the rest is untouched, and only
+ * entry_mask[ptr[row_lo] .. ptr[row_hi]) is read. One GPU passes [0, M); a rank of a row-sharded step passes its node block and
+ * then all-gathers the blocks (twowl_b200.rowshard). */
+int twowl_gcn_dinv_entries(const int64_t* ptr, const int32_t* col, int64_t M, const uint8_t* entry_mask, int64_t row_lo,
+                           int64_t row_hi, float* dinv, void* stream);
 /* out[k] = mask[ids[k]] (uint8) - a per-edge mask carried to the entry order of a CSR built by twowl_csr_build. */
 int twowl_gather_u8(const uint8_t* mask, const int32_t* ids, int64_t n, uint8_t* out, void* stream);
 
@@ -294,23 +293,17 @@ int twowl_graphnorm_bwd(const float* x, const float* dout, int64_t M, int32_t C,
 
 /* Both GraphNorm branches of one pair layer in one pass (they share the output / the incoming gradient):
  *   apply2: out = act(drop(GN_f(xf))) + act(drop(GN_r(xr)))     - the conv2s[i](x) + conv2s_r[i](x) of model.py:77
- *   bwd2:   dxf, dxr and dparams_f[4C], dparams_r[4C] from one dout. */
+ * Its backward (dxf, dxr and dparams_f[4C], dparams_r[4C] from one dout) is twowl_graphnorm_bwd2_sums + _apply below. */
 int twowl_graphnorm_apply2(const float* xf, const float* xr, int64_t M, int32_t C, const float* stats_f,
                            const float* stats_r, const float* wf, const float* bf, const float* mf, const float* wr,
                            const float* br, const float* mr, float p_drop, uint64_t seed_f, uint64_t seed_r,
                            int32_t relu, float* out, void* stream);
-size_t twowl_graphnorm_bwd2_workspace_bytes(int64_t M, int32_t C);
-int twowl_graphnorm_bwd2(const float* xf, const float* xr, const float* dout, int64_t M, int32_t C,
-                         const float* stats_f, const float* stats_r, const float* wf, const float* bf, const float* mf,
-                         const float* wr, const float* br, const float* mr, float p_drop, uint64_t seed_f,
-                         uint64_t seed_r, int32_t relu, float* dxf, float* dxr, float* dparams_f, float* dparams_r,
-                         void* ws, size_t ws_bytes, void* stream);
 
 /* LAST pair layer + readout (model.py:77-83): when the output of conv2s[i](x) + conv2s_r[i](x) only feeds x[idx], the two
  * GraphNorm(+Dropout+ReLU) branches are evaluated at the 2L rows idx selects, never for the whole pair table:
  *   fwd: pred[l] = sum_c hn[idx[2l],c] * hn[idx[2l+1],c] * w[c] + b,   hn[r] = act(drop(GN_f(xf[r]))) + act(drop(GN_r(xr[r])))
  *   bwd: from dpred[L]: dense dxf, dxr [M,C] (GraphNorm's statistics give every row a gradient), dparams_f / dparams_r [4C] as in
- *        twowl_graphnorm_bwd2, dw[C], db[1]. The incoming gradient is zero outside the selected rows, so the column reductions
+ *        twowl_graphnorm_bwd, dw[C], db[1]. The incoming gradient is zero outside the selected rows, so the column reductions
  *        run over the 2L positions only and the dense pass reads xf, xr once. A row selected several times adds its positions in
  *        ascending order (deterministic).
  *   Masked links: a NEGATIVE id in idx[2l] / idx[2l+1] masks link l (pred[l] = 0, no gradient) - a row-sharded caller marks the
@@ -327,29 +320,22 @@ int twowl_gn2_readout_bwd(const float* xf, const float* xr, int64_t M, int32_t C
                           const float* w, const float* dpred, float* dxf, float* dxr, float* dparams_f, float* dparams_r, float* dw,
                           float* db, void* ws, size_t ws_bytes, void* stream);
 
-/* The same backward without its dense pass, for a consumer that makes dxf / dxr on the fly (twowl_pair_dw_gn): everything
- * row-sparse is done here - G[2L,C] = gradient w.r.t. hn at every selected position, head[M] / next[2L] = the chains of positions
- * that select the same row, the parameter gradients, and per branch consts[4][C] = (P, Q, sc, of) such that
- *   dx[r] = P*x[r] + Q + sc * mask(sc*x[r] + of) * sum_{positions j selecting r, ascending} G[j]
- * (consts = [f: P,Q,sc,of | r: P,Q,sc,of], 8*C floats). */
-size_t twowl_gn2_readout_bwd_prepare_workspace_bytes(int64_t M, int64_t L, int32_t C);
-int twowl_gn2_readout_bwd_prepare(const float* xf, const float* xr, int64_t M, int32_t C, const float* stats_f,
-                                  const float* stats_r, const float* wf, const float* bf, const float* mf, const float* wr,
-                                  const float* br, const float* mr, float p_drop, uint64_t seed_f, uint64_t seed_r,
-                                  int32_t relu, const int64_t* idx, int64_t sidx, int64_t L, const float* w,
-                                  const float* dpred, float* G, int32_t* head, int32_t* next, float* consts, float* dparams_f,
-                                  float* dparams_r, float* dw, float* db, void* ws, size_t ws_bytes, void* stream);
-
-/* Row-sharded pair table (the pair rows cut into contiguous blocks over several GPUs, SURVEY 8(e)): every column reduction
- * of the path stops at raw double sums that the caller adds over the ranks (torch.distributed all_reduce of a few KB), then the
- * second half runs on the global sums. One GPU never needs these: twowl_pair_conv / twowl_gn2_readout_bwd_prepare do both halves.
+/* The pair-layer backwards in two halves, split at their column reductions: the first half stops at raw double column sums over the
+ * caller's rows, the second runs on those sums. A row-sharded pair table (the pair rows cut into contiguous blocks over several
+ * GPUs, SURVEY 8(e)) adds the sums over the ranks in between (torch.distributed all_reduce of a few KB) and passes the global row
+ * count M_total; one GPU calls the halves back to back with M_total = M, which gives the fused reduction's bits.
  *   twowl_graphnorm_stats_from_moments: GraphNorm (mean, inv_std) from moments[2C] = column (sum, sum of squares) over M rows
  *     (twowl_conv_args.moments, summed over ranks; M = global row count) - replaces the per-rank finalize of model.py:38.
- *   twowl_gn2_readout_bwd_rows: the row part of twowl_gn2_readout_bwd_prepare over this rank's positions -> G, head, next and
- *     colsums[6][C] (per branch sum g_y, sum g_y*n; dpred.weight; dpred.bias in column 0 of the sixth).
- *   twowl_gn2_readout_bwd_finish: from the rank-summed colsums and M_total -> consts[8C], dparams_f/r[4C], dw[C], db[1].
- *   twowl_graphnorm_bwd2_sums / _apply: twowl_graphnorm_bwd2 (non-last pair layers) cut the same way: colsums[4][C] = per branch
- *     (sum g_y, sum g_y*n) over the rank's rows; _apply = finals on the rank-summed sums with M_total + the dense dx pass. */
+ *   twowl_gn2_readout_bwd_rows / _finish: twowl_gn2_readout_bwd without its dense pass, for a consumer that makes dxf / dxr on the
+ *     fly (twowl_pair_dw_gn). _rows does everything row-sparse: G[2L,C] = gradient w.r.t. hn at every selected position, head[M] /
+ *     next[2L] = the chains of positions that select the same row, and colsums[6][C] (per branch sum g_y, sum g_y*n; dpred.weight;
+ *     dpred.bias in column 0 of the sixth). _finish gives the parameter gradients dparams_f/r[4C], dw[C], db[1] and per branch
+ *     consts[4][C] = (P, Q, sc, of) such that
+ *       dx[r] = P*x[r] + Q + sc * mask(sc*x[r] + of) * sum_{positions j selecting r, ascending} G[j]
+ *     (consts = [f: P,Q,sc,of | r: P,Q,sc,of], 8*C floats).
+ *   twowl_graphnorm_bwd2_sums / _apply: the backward of both GraphNorm branches of a non-last pair layer (twowl_graphnorm_apply2):
+ *     colsums[4][C] = per branch (sum g_y, sum g_y*n) over the caller's rows; _apply = the finals on the summed sums with M_total
+ *     + the dense dx pass. */
 int twowl_graphnorm_stats_from_moments(const double* moments, int64_t M, int32_t C, const float* mean_scale, float eps,
                                        float* stats, void* stream);
 size_t twowl_gn2_readout_bwd_rows_workspace_bytes(int64_t M, int64_t L, int32_t C);
@@ -449,7 +435,7 @@ int twowl_pair_dw_ld(const float* dOf, const float* dOr, const float* rsf, const
                      int32_t C, int64_t ld_dO, int64_t ld_H, float* dWf, float* dWr, void* ws, size_t ws_bytes, void* stream);
 
 /* The same with the gradients made on the fly from the layer's OUTPUTS Of, Or (last pair layer, after
- * twowl_gn2_readout_bwd_prepare): the shared-memory pass that scales and splits the tiles first turns them into
+ * twowl_gn2_readout_bwd_rows / _finish): the shared-memory pass that scales and splits the tiles first turns them into
  * dO = P*O + Q (+ the selected rows' term), writes dOf / dOr [M,C] for the later consumers, and the dense GraphNorm-backward
  * pass (2 reads + 2 writes of [M,C]) disappears. ws as twowl_pair_dw. */
 int twowl_pair_dw_gn(const float* Of, const float* Or, const float* consts, const float* G, const int32_t* head,
@@ -606,26 +592,19 @@ int twowl_embedding_dot(const float* emb, int64_t num_nodes, int32_t d, const in
 /* When ei2 is the full wedge join of (pos_edge, pred_edge) minus the wedges whose source edge is blocked
  * (what get_ei2 + blockei2 produce), the pair-level GCNConv factorises exactly through a per-node sum
  * (DESIGN.md "Factorised pair aggregation"); [2,T] is never materialised.
- * prepare: for every pair row b in [0,R) and both directions d (0: edge2=[a^1;b], 1: edge2_r=[a;b^1])
+ * prepare: for every pair row b in the two ranges [lo0, hi0) and [lo1, hi1) (even bounds: rows 2k / 2k+1 stay together;
+ * hi0 <= lo1) and both directions d (0: edge2=[a^1;b], 1: edge2_r=[a;b^1])
  *   centre[d][b] (int32)  node whose in-list feeds row b      dinv[d][b] = deg^-1/2
  *   selfw[d][b] = 0 if the row's own id-self-loop is among its wedges (unblocked edge) else dinv^2
- * cnt[i] = number of unblocked observed edges with target i (int32[N]). */
+ * written one range after the other into [2, R'] outputs, R' = (hi0 - lo0) + (hi1 - lo1). The whole table is [0, R), [R, R); a
+ * rank's block of the row-sharded step (twowl_b200.rowshard) is its slice of the observed pairs (rows < E) followed by its slice of
+ * the prediction pairs (rows >= E), so that every rank carries the same share of both.
+ * cnt[i] = number of unblocked observed edges with target i (int32[N]), always over ALL observed edges. */
 int twowl_wedge_prepare(const int32_t* src /*[R]*/, const int32_t* dst_e /*[E]*/, int64_t E, int64_t R, int64_t N,
-                        const uint8_t* blocked /*[E] or NULL*/, const int64_t* in_ptr /*[N+1]*/, int32_t* cnt /*[N]*/,
-                        int32_t* centre /*[2,R]*/, float* dinv /*[2,R]*/, float* selfw /*[2,R]*/,
-                        int32_t* bnode /*[2,R]: node whose S row r feeds (backward gather), -1 if none*/, void* stream);
-/* The same constants for the pair rows [row_lo, row_hi) only (even bounds: rows 2k / 2k+1 stay together): one rank's block of
- * a row-sharded step (twowl_b200.rowshard). cnt[N] is still the count over ALL live in-edges (every rank holds the int edge
- * lists); centre / dinv / selfw / bnode are [2, row_hi - row_lo]. */
-int twowl_wedge_prepare_rows(const int32_t* src, const int32_t* dst_e, int64_t E, int64_t R, int64_t N, const uint8_t* blocked,
-                             const int64_t* in_ptr, int64_t row_lo, int64_t row_hi, int32_t* cnt, int32_t* centre, float* dinv,
-                             float* selfw, int32_t* bnode, void* stream);
-/* The same for TWO ranges of pair rows [lo0, hi0) and [lo1, hi1) (even bounds, hi0 <= lo1), written one after the other into
- * [2, (hi0 - lo0) + (hi1 - lo1)] outputs: a rank's block of the row-sharded step is its slice of the observed pairs (rows < E)
- * followed by its slice of the prediction pairs (rows >= E), so that every rank carries the same share of both. */
-int twowl_wedge_prepare_ranges(const int32_t* src, const int32_t* dst_e, int64_t E, int64_t R, int64_t N, const uint8_t* blocked,
-                               const int64_t* in_ptr, int64_t lo0, int64_t hi0, int64_t lo1, int64_t hi1, int32_t* cnt,
-                               int32_t* centre, float* dinv, float* selfw, int32_t* bnode, void* stream);
+                        const uint8_t* blocked /*[E] or NULL*/, const int64_t* in_ptr /*[N+1]*/, int64_t lo0, int64_t hi0,
+                        int64_t lo1, int64_t hi1, int32_t* cnt /*[N]*/, int32_t* centre /*[2,R']*/, float* dinv /*[2,R']*/,
+                        float* selfw /*[2,R']*/, int32_t* bnode /*[2,R']: node whose S row r feeds (backward gather), -1 if none*/,
+                        void* stream);
 /* apply (forward):  out[b] = dinv[b]*S[centre[b]] + selfw[b]*Z[b] + bias   (centre < 0: no S term) */
 int twowl_wedge_apply_fwd(const float* S, const float* Z, const int32_t* centre, const float* dinv,
                           const float* selfw, const float* bias, int64_t R, int32_t C, float* out, void* stream);

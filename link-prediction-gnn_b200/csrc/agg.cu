@@ -438,8 +438,7 @@ __global__ void __launch_bounds__(kAggThreads) k_plan_long(const int64_t* __rest
 __global__ void __launch_bounds__(kAggThreads) k_gcn_dinv(const int64_t* __restrict__ ptr, const int32_t* __restrict__ col,
                                                           int64_t M, int flip, int row_flip,
                                                           const uint8_t* __restrict__ skip_mask,
-                                                          const uint8_t* __restrict__ row_skip_mask,
-                                                          const uint8_t* __restrict__ entry_mask, float* __restrict__ dinv) {
+                                                          const uint8_t* __restrict__ row_skip_mask, float* __restrict__ dinv) {
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = ((int64_t)blockIdx.x * kAggThreads + threadIdx.x) >> 5;
   const int64_t nwarps = ((int64_t)gridDim.x * kAggThreads) >> 5;
@@ -460,12 +459,42 @@ __global__ void __launch_bounds__(kAggThreads) k_gcn_dinv(const int64_t* __restr
 #pragma unroll
       for (int u = 0; u < U; ++u) {
         const int64_t k = k0 + u * 32 + lane;
-        on[u] = k < ke && !(entry_mask && entry_mask[k]);
+        on[u] = k < ke;
         cc[u] = on[u] ? __ldg(col + k) : 0;
       }
 #pragma unroll
       for (int u = 0; u < U; ++u)
         c += (on[u] && ((int64_t)(cc[u] ^ flip) != m) && !(skip_mask && skip_mask[cc[u]])) ? 1 : 0;
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
+    if (lane == 0) dinv[m] = rsqrtf_exact((float)(c + 1));
+  }
+}
+
+// the same count over the rows [row_lo, row_hi) of a cached CSR minus the entries a per-ENTRY mask removes:
+// deg[m] = 1 + #{k in row m : !entry_mask[k], col[k] != m}
+__global__ void __launch_bounds__(kAggThreads) k_gcn_dinv_entries(const int64_t* __restrict__ ptr, const int32_t* __restrict__ col,
+                                                                  const uint8_t* __restrict__ entry_mask, int64_t row_lo,
+                                                                  int64_t row_hi, float* __restrict__ dinv) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp0 = ((int64_t)blockIdx.x * kAggThreads + threadIdx.x) >> 5;
+  const int64_t nwarps = ((int64_t)gridDim.x * kAggThreads) >> 5;
+  for (int64_t m = row_lo + warp0; m < row_hi; m += nwarps) {
+    const int64_t kb = ptr[m], ke = ptr[m + 1];
+    int c = 0;
+    constexpr int U = 8;
+    for (int64_t k0 = kb; k0 < ke; k0 += 32 * U) {
+      int cc[U];
+      bool on[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int64_t k = k0 + u * 32 + lane;
+        on[u] = k < ke && !(entry_mask && entry_mask[k]);
+        cc[u] = on[u] ? __ldg(col + k) : 0;
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u) c += (on[u] && (int64_t)cc[u] != m) ? 1 : 0;
     }
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
@@ -483,17 +512,18 @@ extern "C" int twowl_gcn_dinv(const int64_t* ptr, const int32_t* col, int64_t M,
   TW_CHECK_ARG(!(row_flip && (M & 1)), "gcn_dinv: row_flip needs an even row count");
   if (M == 0) return 0;
   k_gcn_dinv<<<grid_for(M, kAggThreads / 32, 8), kAggThreads, 0, (cudaStream_t)stream>>>(ptr, col, M, flip, row_flip, skip_mask,
-                                                                                      row_skip_mask, nullptr, dinv);
+                                                                                      row_skip_mask, dinv);
   TW_LAUNCH_CHECK();
   return 0;
 }
 
-extern "C" int twowl_gcn_dinv_entries(const int64_t* ptr, const int32_t* col, int64_t M, const uint8_t* entry_mask, float* dinv,
-                                      void* stream) {
-  TW_CHECK_ARG(M >= 0, "gcn_dinv_entries: negative M");
-  if (M == 0) return 0;
-  k_gcn_dinv<<<grid_for(M, kAggThreads / 32, 8), kAggThreads, 0, (cudaStream_t)stream>>>(ptr, col, M, 0, 0, nullptr, nullptr,
-                                                                                      entry_mask, dinv);
+extern "C" int twowl_gcn_dinv_entries(const int64_t* ptr, const int32_t* col, int64_t M, const uint8_t* entry_mask, int64_t row_lo,
+                                      int64_t row_hi, float* dinv, void* stream) {
+  TW_CHECK_ARG(M >= 0 && row_lo >= 0 && row_lo <= row_hi && row_hi <= M, "gcn_dinv_entries: rows [%lld, %lld) outside [0, %lld]",
+               (long long)row_lo, (long long)row_hi, (long long)M);
+  if (row_hi == row_lo) return 0;
+  k_gcn_dinv_entries<<<grid_for(row_hi - row_lo, kAggThreads / 32, 8), kAggThreads, 0, (cudaStream_t)stream>>>(ptr, col, entry_mask,
+                                                                                                          row_lo, row_hi, dinv);
   TW_LAUNCH_CHECK();
   return 0;
 }

@@ -54,7 +54,7 @@ struct DwParams {
   float* part;  // [gridDim.x][dw_part_rows(C)][C]: fp32 running sums (C = 128), or the same shape in double (C <= 64)
   // GN = true: the A tiles are the OUTPUTS O_f, O_r of the last pair layer and the gradients are made on the fly
   // (twowl_pair_dw_gn): dO = P * O + Q (+ sc * g_y on the rows the readout selected), written to dOf / dOr as well
-  const float* consts;   // [2 branches][4][C] = (P, Q, sc, of), twowl_gn2_readout_bwd_prepare
+  const float* consts;   // [2 branches][4][C] = (P, Q, sc, of), twowl_gn2_readout_bwd_finish
   const float* G;        // [2L, C] gradient of the selected rows, by position
   const int32_t* head;   // [M] first position that selects a row, -1 = none
   const int32_t* next;   // [2L] next position selecting the same row

@@ -838,40 +838,6 @@ extern "C" int twowl_graphnorm_apply2(const float* xf, const float* xr, int64_t 
   return 0;
 }
 
-extern "C" size_t twowl_graphnorm_bwd2_workspace_bytes(int64_t M, int32_t C) {
-  (void)M;
-  return align_up((size_t)kNormMaxCtas * 4 * (size_t)C * sizeof(double)) + 2 * align_up(3 * (size_t)C * sizeof(float));
-}
-
-extern "C" int twowl_graphnorm_bwd2(const float* xf, const float* xr, const float* dout, int64_t M, int32_t C,
-                                    const float* stats_f, const float* stats_r, const float* wf, const float* bf, const float* mf,
-                                    const float* wr, const float* br, const float* mr, float p_drop, uint64_t seed_f,
-                                    uint64_t seed_r, int32_t relu, float* dxf, float* dxr, float* dparams_f, float* dparams_r,
-                                    void* ws, size_t ws_bytes, void* stream) {
-  if (int rc = check_mc("graphnorm_bwd2", M, C)) return rc;
-  TW_CHECK_ARG(M > 0, "graphnorm_bwd2: needs at least one row");
-  TW_CHECK_ARG(aligned16(xf) && aligned16(xr) && aligned16(dout) && aligned16(dxf) && aligned16(dxr),
-               "graphnorm_bwd2: 16-byte alignment required");
-  TW_CHECK_ARG(p_drop >= 0.f && p_drop < 1.f, "graphnorm_bwd2: dropout p=%f outside [0,1)", p_drop);
-  TW_CHECK_WS(ws_bytes, twowl_graphnorm_bwd2_workspace_bytes(M, C));
-  cudaStream_t s = (cudaStream_t)stream;
-  Carver c(ws);
-  double* part = c.take<double>((size_t)kNormMaxCtas * 4 * C);
-  float* sums_f = c.take<float>(3 * (size_t)C);
-  float* sums_r = c.take<float>(3 * (size_t)C);
-  const uint32_t thresh = p_drop > 0.f ? drop_thresh(p_drop) : 0u;
-  const float inv_keep = 1.f / (1.f - p_drop);
-  const int grid = norm_grid(M, C);
-  k_gn_bwd2_partial<<<grid, kNormThreads, red_smem(C, 4), s>>>(xf, xr, dout, M, C, stats_f, stats_r, wf, bf, mf, wr, br, mr, thresh,
-                                                               inv_keep, seed_f, seed_r, relu, part);
-  k_gn_bwd_final<<<(int)cdiv(C, 4), 128, 0, s>>>(part, grid, 4, 0, M, C, stats_f, wf, mf, sums_f, dparams_f);
-  k_gn_bwd_final<<<(int)cdiv(C, 4), 128, 0, s>>>(part, grid, 4, 2, M, C, stats_r, wr, mr, sums_r, dparams_r);
-  k_gn_bwd2_dx<<<grid, kNormThreads, 0, s>>>(xf, xr, dout, M, C, stats_f, stats_r, wf, bf, mf, wr, br, mr, thresh, inv_keep, seed_f,
-                                             seed_r, relu, sums_f, sums_r, dxf, dxr);
-  TW_LAUNCH_CHECK();
-  return 0;
-}
-
 extern "C" int twowl_gn2_readout_fwd(const float* xf, const float* xr, int64_t M, int32_t C, const float* stats_f,
                                      const float* stats_r, const float* wf, const float* bf, const float* mf, const float* wr,
                                      const float* br, const float* mr, float p_drop, uint64_t seed_f, uint64_t seed_r,
@@ -928,18 +894,6 @@ static int gn2_prepare_finish(const double* part, int nparts, int64_t M_stat, in
   TW_LAUNCH_CHECK();
   return 0;
 }
-static int gn2_prepare(const float* xf, const float* xr, int64_t M, int32_t C, const float* stats_f, const float* stats_r,
-                       const float* wf, const float* bf, const float* mf, const float* wr, const float* br, const float* mr,
-                       uint32_t thresh, float inv_keep, uint64_t seed_f, uint64_t seed_r, int32_t relu, const int64_t* idx, int64_t sidx,
-                       int64_t L, const float* w, const float* dpred, float* G, int32_t* head, int32_t* next, double* part, float* sums_f,
-                       float* sums_r, float* dparams_f, float* dparams_r, float* dw, float* db, cudaStream_t s) {
-  int nparts = 0;
-  if (int rc = gn2_prepare_rows(xf, xr, M, C, stats_f, stats_r, wf, bf, mf, wr, br, mr, thresh, inv_keep, seed_f, seed_r, relu, idx, sidx,
-                                L, w, dpred, G, head, next, part, &nparts, s))
-    return rc;
-  return gn2_prepare_finish(part, nparts, M, C, stats_f, stats_r, wf, mf, wr, mr, sums_f, sums_r, dparams_f, dparams_r, dw, db, s);
-}
-
 extern "C" size_t twowl_gn2_readout_bwd_workspace_bytes(int64_t M, int64_t L, int32_t C) {
   const size_t l = (size_t)(L > 0 ? L : 1);
   return align_up(2 * l * (size_t)C * sizeof(float)) + align_up((size_t)(M > 0 ? M : 1) * sizeof(int32_t)) + align_up(2 * l * sizeof(int32_t)) +
@@ -969,8 +923,11 @@ extern "C" int twowl_gn2_readout_bwd(const float* xf, const float* xr, int64_t M
   float* sums_r = c.take<float>(3 * (size_t)C);
   const uint32_t thresh = p_drop > 0.f ? drop_thresh(p_drop) : 0u;
   const float inv_keep = 1.f / (1.f - p_drop);
-  if (int rc = gn2_prepare(xf, xr, M, C, stats_f, stats_r, wf, bf, mf, wr, br, mr, thresh, inv_keep, seed_f, seed_r, relu, idx, sidx, L, w,
-                           dpred, G, head, next, part, sums_f, sums_r, dparams_f, dparams_r, dw, db, s))
+  int nparts = 0;
+  if (int rc = gn2_prepare_rows(xf, xr, M, C, stats_f, stats_r, wf, bf, mf, wr, br, mr, thresh, inv_keep, seed_f, seed_r, relu, idx, sidx,
+                                L, w, dpred, G, head, next, part, &nparts, s))
+    return rc;
+  if (int rc = gn2_prepare_finish(part, nparts, M, C, stats_f, stats_r, wf, mf, wr, mr, sums_f, sums_r, dparams_f, dparams_r, dw, db, s))
     return rc;
   k_gn_bwd2_dx_rows<<<norm_grid(M, C), kNormThreads, 0, s>>>(xf, xr, G, head, next, M, C, stats_f, stats_r, wf, bf, mf, wr, br, mr, thresh,
                                                              inv_keep, seed_f, seed_r, relu, sums_f, sums_r, dxf, dxr);
@@ -978,41 +935,11 @@ extern "C" int twowl_gn2_readout_bwd(const float* xf, const float* xr, int64_t M
   return 0;
 }
 
-extern "C" size_t twowl_gn2_readout_bwd_prepare_workspace_bytes(int64_t M, int64_t L, int32_t C) {
-  (void)M, (void)L;
-  return align_up((size_t)kNormMaxCtas * 6 * (size_t)C * sizeof(double)) + 2 * align_up(3 * (size_t)C * sizeof(float));
-}
-
-extern "C" int twowl_gn2_readout_bwd_prepare(const float* xf, const float* xr, int64_t M, int32_t C, const float* stats_f,
-                                             const float* stats_r, const float* wf, const float* bf, const float* mf, const float* wr,
-                                             const float* br, const float* mr, float p_drop, uint64_t seed_f, uint64_t seed_r,
-                                             int32_t relu, const int64_t* idx, int64_t sidx, int64_t L, const float* w,
-                                             const float* dpred, float* G, int32_t* head, int32_t* next, float* consts, float* dparams_f,
-                                             float* dparams_r, float* dw, float* db, void* ws, size_t ws_bytes, void* stream) {
-  if (int rc = check_mc("gn2_readout_bwd_prepare", M, C)) return rc;
-  TW_CHECK_ARG(M > 0 && M < 0x7fffffffLL && L >= 0 && 2 * L < 0x7fffffffLL, "gn2_readout_bwd_prepare: sizes out of range");
-  TW_CHECK_ARG(aligned16(xf) && aligned16(xr) && aligned16(G) && aligned16(w) && aligned16(consts) && head && next,
-               "gn2_readout_bwd_prepare: bad pointers");
-  TW_CHECK_ARG(p_drop >= 0.f && p_drop < 1.f, "gn2_readout_bwd_prepare: dropout p=%f outside [0,1)", p_drop);
-  TW_CHECK_WS(ws_bytes, twowl_gn2_readout_bwd_prepare_workspace_bytes(M, L, C));
-  cudaStream_t s = (cudaStream_t)stream;
-  Carver c(ws);
-  double* part = c.take<double>((size_t)kNormMaxCtas * 6 * C);
-  float* sums_f = c.take<float>(3 * (size_t)C);
-  float* sums_r = c.take<float>(3 * (size_t)C);
-  const uint32_t thresh = p_drop > 0.f ? drop_thresh(p_drop) : 0u;
-  if (int rc = gn2_prepare(xf, xr, M, C, stats_f, stats_r, wf, bf, mf, wr, br, mr, thresh, 1.f / (1.f - p_drop), seed_f, seed_r, relu, idx,
-                           sidx, L, w, dpred, G, head, next, part, sums_f, sums_r, dparams_f, dparams_r, dw, db, s))
-    return rc;
-  k_gn_bwd_consts<<<(int)cdiv(C, 128), 128, 0, s>>>(stats_f, wf, bf, mf, sums_f, C, consts);
-  k_gn_bwd_consts<<<(int)cdiv(C, 128), 128, 0, s>>>(stats_r, wr, br, mr, sums_r, C, consts + 4 * (size_t)C);
-  TW_LAUNCH_CHECK();
-  return 0;
-}
-
-// ---------------------------------------------------------------- row-sharded pair table ----------
-// The pair table cut into row blocks over several GPUs: column reductions stop at raw double sums, the caller adds them over
-// the ranks (one all-reduce of a few KB), and the second half runs on the global sums.
+// ---------------------------------------------------------------- backward halves ------------------
+// The pair-layer backwards split at their column reductions: the first half stops at raw double sums over the caller's rows,
+// a row-sharded caller adds them over the ranks (one all-reduce of a few KB), and the second half runs on the global sums. One
+// GPU calls the halves back to back: the second half's warp_part_sum over nparts = 1 returns each sum unchanged, so the result
+// is bit for bit that of one fused reduction.
 
 // colsums[v][c] = sum over CTAs of part[.][v][c] (a warp per (v, c), fixed order)
 __global__ void k_part_reduce_raw(const double* __restrict__ part, int nparts, int nv, int C, double* __restrict__ out) {
@@ -1093,9 +1020,9 @@ extern "C" int twowl_gn2_readout_bwd_finish(const double* colsums, int64_t M_tot
   return 0;
 }
 
-// twowl_graphnorm_bwd2 cut at its column reduction (non-last pair layers of a row-sharded pair table): _sums gives the raw
-// fp64 column sums [4][C] = per branch (sum g_y, sum g_y*n) over this rank's rows; _apply runs the finals on the rank-summed
-// sums with the global row count M_total, then the dense dx pass over the local rows.
+// GraphNorm backward of both branches of a non-last pair layer: _sums gives the raw fp64 column sums [4][C] = per branch
+// (sum g_y, sum g_y*n) over the caller's rows; _apply runs the finals on the (rank-summed) sums with the total row count M_total,
+// then the dense dx pass over the caller's rows.
 extern "C" size_t twowl_graphnorm_bwd2_sums_workspace_bytes(int64_t M, int32_t C) {
   (void)M;
   return align_up((size_t)kNormMaxCtas * 4 * (size_t)C * sizeof(double));

@@ -245,37 +245,6 @@ __global__ void __launch_bounds__(kRowThreads) k_wedge_apply_bwd(const float* __
   }
 }
 
-// gcn_norm degrees of the node rows [row_lo, row_hi) of a cached CSR minus the entries a per-entry mask removes
-// (twowl_gcn_dinv_entries for ONE node block of a row-sharded step): dinv[m] = (1 + #{k in row m: !entry_mask[k], col[k] != m})^-1/2.
-// One warp per row, 8 x 32 entries per iteration with all loads issued before any is used; integer counting, exact.
-__global__ void __launch_bounds__(kRowThreads) k_gcn_dinv_rows(const int64_t* __restrict__ ptr, const int32_t* __restrict__ col,
-                                                               const uint8_t* __restrict__ entry_mask, int64_t row_lo, int64_t row_hi,
-                                                               float* __restrict__ dinv) {
-  const int lane = threadIdx.x & 31;
-  const int64_t warp0 = ((int64_t)blockIdx.x * kRowThreads + threadIdx.x) >> 5;
-  const int64_t nwarps = ((int64_t)gridDim.x * kRowThreads) >> 5;
-  for (int64_t m = row_lo + warp0; m < row_hi; m += nwarps) {
-    const int64_t kb = ptr[m], ke = ptr[m + 1];
-    int c = 0;
-    constexpr int U = 8;
-    for (int64_t k0 = kb; k0 < ke; k0 += 32 * U) {
-      int cc[U];
-      bool on[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const int64_t k = k0 + u * 32 + lane;
-        on[u] = k < ke && !(entry_mask && entry_mask[k]);
-        cc[u] = on[u] ? __ldg(col + k) : 0;
-      }
-#pragma unroll
-      for (int u = 0; u < U; ++u) c += (on[u] && (int64_t)cc[u] != m) ? 1 : 0;
-    }
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
-    if (lane == 0) dinv[m] = rsqrtf_exact((float)(c + 1));
-  }
-}
-
 static int check_c(const char* op, int C) {
   TW_CHECK_ARG(C >= 4 && (C & 3) == 0 && C <= 1024, "%s: C=%d must be a multiple of 4 in [4,1024]", op, C);
   return 0;
@@ -351,24 +320,11 @@ extern "C" int twowl_readout_bwd(const float* H, const int64_t* idx, int64_t sid
 }
 
 extern "C" int twowl_wedge_prepare(const int32_t* src, const int32_t* dst_e, int64_t E, int64_t R, int64_t N,
-                                   const uint8_t* blocked, const int64_t* in_ptr, int32_t* cnt, int32_t* centre, float* dinv,
-                                   float* selfw, int32_t* bnode, void* stream) {
+                                   const uint8_t* blocked, const int64_t* in_ptr, int64_t lo0, int64_t hi0, int64_t lo1, int64_t hi1,
+                                   int32_t* cnt, int32_t* centre, float* dinv, float* selfw, int32_t* bnode, void* stream) {
   TW_CHECK_ARG(E >= 0 && R >= E && N >= 0, "wedge_prepare: need 0 <= E <= R and N >= 0");
-  cudaStream_t s = (cudaStream_t)stream;
-  if (N > 0) k_wedge_cnt_init<<<grid_for(N, kRowThreads), kRowThreads, 0, s>>>(in_ptr, N, cnt);
-  if (blocked && E > 0 && N > 0) k_wedge_cnt_block<<<grid_for(E, kRowThreads), kRowThreads, 0, s>>>(dst_e, E, N, blocked, cnt);
-  if (R > 0) k_wedge_rows<<<grid_for(R, kRowThreads), kRowThreads, 0, s>>>(src, dst_e, E, R, N, blocked, cnt, 0, R, R, 0, centre, dinv, selfw, bnode);
-  TW_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int twowl_wedge_prepare_ranges(const int32_t* src, const int32_t* dst_e, int64_t E, int64_t R, int64_t N,
-                                          const uint8_t* blocked, const int64_t* in_ptr, int64_t lo0, int64_t hi0, int64_t lo1,
-                                          int64_t hi1, int32_t* cnt, int32_t* centre, float* dinv, float* selfw, int32_t* bnode,
-                                          void* stream) {
-  TW_CHECK_ARG(E >= 0 && R >= E && N >= 0, "wedge_prepare_ranges: need 0 <= E <= R and N >= 0");
   TW_CHECK_ARG(lo0 >= 0 && lo0 <= hi0 && hi0 <= lo1 && lo1 <= hi1 && hi1 <= R && !((lo0 | hi0 | lo1 | hi1) & 1),
-               "wedge_prepare_ranges: [%lld, %lld) and [%lld, %lld) must be even-bounded, ordered, disjoint ranges of the %lld pair rows",
+               "wedge_prepare: [%lld, %lld) and [%lld, %lld) must be even-bounded, ordered, disjoint ranges of the %lld pair rows",
                (long long)lo0, (long long)hi0, (long long)lo1, (long long)hi1, (long long)R);
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t n0 = hi0 - lo0, n1 = hi1 - lo1;
@@ -380,27 +336,6 @@ extern "C" int twowl_wedge_prepare_ranges(const int32_t* src, const int32_t* dst
   if (n1 > 0)
     k_wedge_rows<<<grid_for(n1, kRowThreads), kRowThreads, 0, s>>>(src, dst_e, E, R, N, blocked, cnt, lo1, hi1, n0 + n1, n0, centre, dinv,
                                                                    selfw, bnode);
-  TW_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int twowl_wedge_prepare_rows(const int32_t* src, const int32_t* dst_e, int64_t E, int64_t R, int64_t N,
-                                        const uint8_t* blocked, const int64_t* in_ptr, int64_t row_lo, int64_t row_hi, int32_t* cnt,
-                                        int32_t* centre, float* dinv, float* selfw, int32_t* bnode, void* stream) {
-  TW_CHECK_ARG(row_lo >= 0 && row_lo <= row_hi && row_hi <= R && !((row_lo | row_hi) & 1),
-               "wedge_prepare_rows: [%lld, %lld) must be an even-bounded range of the %lld pair rows", (long long)row_lo,
-               (long long)row_hi, (long long)R);
-  return twowl_wedge_prepare_ranges(src, dst_e, E, R, N, blocked, in_ptr, row_lo, row_hi, row_hi, row_hi, cnt, centre, dinv, selfw, bnode,
-                                    stream);
-}
-
-extern "C" int twowl_gcn_dinv_entries_rows(const int64_t* ptr, const int32_t* col, int64_t M, const uint8_t* entry_mask, int64_t row_lo,
-                                           int64_t row_hi, float* dinv, void* stream) {
-  TW_CHECK_ARG(M >= 0 && row_lo >= 0 && row_lo <= row_hi && row_hi <= M, "gcn_dinv_entries_rows: rows [%lld, %lld) outside [0, %lld]",
-               (long long)row_lo, (long long)row_hi, (long long)M);
-  if (row_hi == row_lo) return 0;
-  k_gcn_dinv_rows<<<grid_for(row_hi - row_lo, kRowThreads / 32, 8), kRowThreads, 0, (cudaStream_t)stream>>>(ptr, col, entry_mask, row_lo,
-                                                                                                        row_hi, dinv);
   TW_LAUNCH_CHECK();
   return 0;
 }

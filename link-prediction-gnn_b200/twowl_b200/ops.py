@@ -372,14 +372,18 @@ def gcn_dinv(ptr, col, M: int, flip: int = 0, row_flip: int = 0, skip_mask=None,
     return dinv
 
 
-def gcn_dinv_entries(ptr, col, M: int, entry_mask) -> torch.Tensor:
-    """gcn_norm degree of a cached CSR minus the entries a per-entry mask removes."""
-    _need_cuda(ptr, col, entry_mask)
-    dinv = torch.empty(M, dtype=torch.float32, device=ptr.device)
-    check(lib.twowl_gcn_dinv_entries(ptr.data_ptr(), col.data_ptr(), M, entry_mask.data_ptr(), dinv.data_ptr(), _stream()),
-          "gcn_dinv_entries")
+def gcn_dinv_entries(ptr, col, M: int, entry_mask, rows=None, out=None) -> torch.Tensor:
+    """gcn_norm degree of a cached CSR minus the entries a per-entry mask removes, for the node rows rows = (lo, hi) (default: all
+    M) -> out (fp32, at least M elements; a new [M] tensor by default) with out[lo:hi] written and the rest untouched."""
+    _need_cuda(ptr, col, entry_mask, out)
+    if out is None:
+        out = torch.empty(M, dtype=torch.float32, device=ptr.device)
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() >= M
+    lo, hi = (0, M) if rows is None else rows
+    check(lib.twowl_gcn_dinv_entries(ptr.data_ptr(), col.data_ptr(), M, entry_mask.data_ptr(), int(lo), int(hi), out.data_ptr(),
+                                     _stream()), "gcn_dinv_entries")
     _count()
-    return dinv
+    return out
 
 
 def gather_u8(mask: torch.Tensor, ids: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -391,16 +395,6 @@ def gather_u8(mask: torch.Tensor, ids: torch.Tensor, out: Optional[torch.Tensor]
     check(lib.twowl_gather_u8(mask.data_ptr(), ids.data_ptr(), ids.numel(), out.data_ptr(), _stream()), "gather_u8")
     _count()
     return out
-
-
-def gcn_dinv_entries_rows(ptr, col, M: int, entry_mask, lo: int, hi: int, dinv: torch.Tensor) -> torch.Tensor:
-    """gcn_dinv_entries for the node rows [lo, hi) only, written into dinv[lo:hi] (dinv: fp32, at least M elements)."""
-    _need_cuda(ptr, col, entry_mask, dinv)
-    assert dinv.dtype == torch.float32 and dinv.is_contiguous() and dinv.numel() >= M
-    check(lib.twowl_gcn_dinv_entries_rows(ptr.data_ptr(), col.data_ptr(), M, entry_mask.data_ptr(), int(lo), int(hi), dinv.data_ptr(),
-                                          _stream()), "gcn_dinv_entries_rows")
-    _count()
-    return dinv
 
 
 LONG_ROW = 64     # TWOWL_LONG_ROW of include/twowl.h: rows with more entries go through the long-row passes of seg_reduce
@@ -569,52 +563,12 @@ def gn2_readout_bwd(xf, xr, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r: 
     return dxf, dxr, dpf, dpr, dw, db
 
 
-def gn2_readout_bwd_prepare(xf, xr, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r: int, relu: bool, idx, w, dpred):
+def gn2_readout_bwd_prepare(xf, xr, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r: int, relu: bool, idx, w, dpred,
+                            M_total: Optional[int] = None, all_reduce=None):
     """The row-sparse part of gn2_readout_bwd for a consumer that makes dxf / dxr on the fly (pair_dw_gn):
-    -> (G [2L,C], head int32[M], next int32[2L], consts [8C], dparams_f, dparams_r [4C], dw [1,C], db [1])."""
-    M, C = xf.shape
-    dev = xf.device
-    idx = idx.reshape(-1)
-    L = idx.numel() // 2
-    G = torch.empty((max(2 * L, 1), C), dtype=torch.float32, device=dev)
-    head = torch.empty(M, dtype=torch.int32, device=dev)
-    nxt = torch.empty(max(2 * L, 1), dtype=torch.int32, device=dev)
-    consts = torch.empty(8 * C, dtype=torch.float32, device=dev)
-    dpf = torch.empty(4 * C, dtype=torch.float32, device=dev)
-    dpr = torch.empty(4 * C, dtype=torch.float32, device=dev)
-    dw = torch.empty((1, C), dtype=torch.float32, device=dev)
-    db = torch.empty(1, dtype=torch.float32, device=dev)
-    nb = lib.twowl_gn2_readout_bwd_prepare_workspace_bytes(M, L, C)
-    ws = _ws(nb, dev)
-    p, s = _row(idx)
-    dpred = dpred.contiguous()
-    with _P("gn2_readout_bwd_prepare", M * 4 + L * (48 * C + 40)):
-        check(lib.twowl_gn2_readout_bwd_prepare(xf.data_ptr(), xr.data_ptr(), M, C, sf.data_ptr(), sr.data_ptr(), pf[0].data_ptr(),
-                                                pf[1].data_ptr(), pf[2].data_ptr(), pr[0].data_ptr(), pr[1].data_ptr(),
-                                                pr[2].data_ptr(), float(p_drop), int(seed_f), int(seed_r), int(relu), p, s, L,
-                                                w.data_ptr(), dpred.data_ptr(), G.data_ptr(), head.data_ptr(), nxt.data_ptr(),
-                                                consts.data_ptr(), dpf.data_ptr(), dpr.data_ptr(), dw.data_ptr(), db.data_ptr(),
-                                                ws.data_ptr(), nb, _stream()), "gn2_readout_bwd_prepare")
-    _count(9)
-    return G, head, nxt, consts, dpf, dpr, dw, db
-
-
-# ------------------------------------------------------------------------------ GraphNorm
-
-def graphnorm_stats_from_moments(moments, M_total: int, mean_scale, eps: float) -> torch.Tensor:
-    """GraphNorm (mean, inv_std)[2C] from the rank-summed column (sum, sum of squares) float64[2C] over M_total rows."""
-    _need_cuda(moments, mean_scale)
-    C = mean_scale.numel()
-    stats = torch.empty(2 * C, dtype=torch.float32, device=moments.device)
-    check(lib.twowl_graphnorm_stats_from_moments(moments.data_ptr(), int(M_total), C, mean_scale.data_ptr(), float(eps),
-                                                 stats.data_ptr(), _stream()), "graphnorm_stats_from_moments")
-    _count()
-    return stats
-
-
-def gn2_readout_bwd_rows(xf, xr, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r: int, relu: bool, idx, w, dpred):
-    """Row part of gn2_readout_bwd_prepare over this rank's rows / positions:
-    -> (G [2L,C], head int32[M], next int32[2L], colsums float64[6,C]) - colsums are summed over the ranks by the caller."""
+    -> (G [2L,C], head int32[M], next int32[2L], consts [8C], dparams_f, dparams_r [4C], dw [1,C], db [1]).
+    On one row block of a row-sharded pair table, `all_reduce` (a callable applied in place) sums the fp64 column sums [6,C] over
+    the ranks between the two halves, and M_total is the whole table's row count (default: M)."""
     M, C = xf.shape
     dev = xf.device
     idx = idx.reshape(-1)
@@ -634,13 +588,8 @@ def gn2_readout_bwd_rows(xf, xr, sf, sr, pf, pr, p_drop: float, seed_f: int, see
                                              w.data_ptr(), dpred.data_ptr(), G.data_ptr(), head.data_ptr(), nxt.data_ptr(),
                                              colsums.data_ptr(), ws.data_ptr(), nb, _stream()), "gn2_readout_bwd_rows")
     _count(4)
-    return G, head, nxt, colsums
-
-
-def gn2_readout_bwd_finish(colsums, M_total: int, sf, sr, pf, pr):
-    """-> (consts [8C], dparams_f, dparams_r [4C], dw [1,C], db [1]) from the rank-summed colsums of gn2_readout_bwd_rows."""
-    C = colsums.shape[1]
-    dev = colsums.device
+    if all_reduce is not None:
+        all_reduce(colsums)
     consts = torch.empty(8 * C, dtype=torch.float32, device=dev)
     dpf = torch.empty(4 * C, dtype=torch.float32, device=dev)
     dpr = torch.empty(4 * C, dtype=torch.float32, device=dev)
@@ -648,12 +597,25 @@ def gn2_readout_bwd_finish(colsums, M_total: int, sf, sr, pf, pr):
     db = torch.empty(1, dtype=torch.float32, device=dev)
     nb = lib.twowl_gn2_readout_bwd_finish_workspace_bytes(C)
     ws = _ws(nb, dev)
-    check(lib.twowl_gn2_readout_bwd_finish(colsums.data_ptr(), int(M_total), C, sf.data_ptr(), sr.data_ptr(), pf[0].data_ptr(),
-                                           pf[1].data_ptr(), pf[2].data_ptr(), pr[0].data_ptr(), pr[1].data_ptr(), pr[2].data_ptr(),
-                                           consts.data_ptr(), dpf.data_ptr(), dpr.data_ptr(), dw.data_ptr(), db.data_ptr(),
-                                           ws.data_ptr(), nb, _stream()), "gn2_readout_bwd_finish")
+    check(lib.twowl_gn2_readout_bwd_finish(colsums.data_ptr(), int(M if M_total is None else M_total), C, sf.data_ptr(), sr.data_ptr(),
+                                           pf[0].data_ptr(), pf[1].data_ptr(), pf[2].data_ptr(), pr[0].data_ptr(), pr[1].data_ptr(),
+                                           pr[2].data_ptr(), consts.data_ptr(), dpf.data_ptr(), dpr.data_ptr(), dw.data_ptr(),
+                                           db.data_ptr(), ws.data_ptr(), nb, _stream()), "gn2_readout_bwd_finish")
     _count(6)
-    return consts, dpf, dpr, dw, db
+    return G, head, nxt, consts, dpf, dpr, dw, db
+
+
+# ------------------------------------------------------------------------------ GraphNorm
+
+def graphnorm_stats_from_moments(moments, M_total: int, mean_scale, eps: float) -> torch.Tensor:
+    """GraphNorm (mean, inv_std)[2C] from the rank-summed column (sum, sum of squares) float64[2C] over M_total rows."""
+    _need_cuda(moments, mean_scale)
+    C = mean_scale.numel()
+    stats = torch.empty(2 * C, dtype=torch.float32, device=moments.device)
+    check(lib.twowl_graphnorm_stats_from_moments(moments.data_ptr(), int(M_total), C, mean_scale.data_ptr(), float(eps),
+                                                 stats.data_ptr(), _stream()), "graphnorm_stats_from_moments")
+    _count()
+    return stats
 
 
 def graphnorm_stats(x, mean_scale, eps: float) -> torch.Tensor:
@@ -785,50 +747,21 @@ def bias_layernorm_bwd(g, z, bias, stats, p_drop: float, seed: int) -> torch.Ten
 
 # ------------------------------------------------------------------------------ structured wedge path
 
-def wedge_prepare(src32, dst_e32, E: int, R: int, N: int, blocked, in_ptr):
+def wedge_prepare(src32, dst_e32, E: int, R: int, N: int, blocked, in_ptr, ranges=None):
+    """Per-row constants of the pair rows ranges = ((lo0, hi0), (lo1, hi1)), written one range after the other (default: the whole
+    table, ((0, R), (R, R))) -> (cnt [N], centre, dinv, selfw, bnode [2, (hi0 - lo0) + (hi1 - lo1)])."""
+    (lo0, hi0), (lo1, hi1) = ((0, R), (R, R)) if ranges is None else ranges
     dev = src32.device
-    cnt = torch.empty(max(N, 1), dtype=torch.int32, device=dev)
-    centre = torch.empty((2, R), dtype=torch.int32, device=dev)
-    dinv = torch.empty((2, R), dtype=torch.float32, device=dev)
-    selfw = torch.empty((2, R), dtype=torch.float32, device=dev)
-    bnode = torch.empty((2, R), dtype=torch.int32, device=dev)
-    check(lib.twowl_wedge_prepare(src32.data_ptr(), dst_e32.data_ptr(), E, R, N, _p(blocked), in_ptr.data_ptr(),
-                                  cnt.data_ptr(), centre.data_ptr(), dinv.data_ptr(), selfw.data_ptr(), bnode.data_ptr(),
-                                  _stream()), "wedge_prepare")
-    _count(3)
-    return cnt, centre, dinv, selfw, bnode
-
-
-def wedge_prepare_rows(src32, dst_e32, E: int, R: int, N: int, blocked, in_ptr, lo: int, hi: int):
-    """wedge_prepare for the pair rows [lo, hi) only -> (cnt [N], centre, dinv, selfw, bnode [2, hi - lo])."""
-    dev = src32.device
-    Rl = hi - lo
+    Rl = (hi0 - lo0) + (hi1 - lo1)
     cnt = torch.empty(max(N, 1), dtype=torch.int32, device=dev)
     centre = torch.empty((2, Rl), dtype=torch.int32, device=dev)
     dinv = torch.empty((2, Rl), dtype=torch.float32, device=dev)
     selfw = torch.empty((2, Rl), dtype=torch.float32, device=dev)
     bnode = torch.empty((2, Rl), dtype=torch.int32, device=dev)
-    check(lib.twowl_wedge_prepare_rows(src32.data_ptr(), dst_e32.data_ptr(), E, R, N, _p(blocked), in_ptr.data_ptr(), int(lo), int(hi),
-                                       cnt.data_ptr(), centre.data_ptr(), dinv.data_ptr(), selfw.data_ptr(), bnode.data_ptr(),
-                                       _stream()), "wedge_prepare_rows")
-    _count(3)
-    return cnt, centre, dinv, selfw, bnode
-
-
-def wedge_prepare_ranges(src32, dst_e32, E: int, R: int, N: int, blocked, in_ptr, r0, r1):
-    """wedge_prepare for the pair rows r0 = [lo0, hi0) followed by r1 = [lo1, hi1) -> (cnt [N], centre, dinv, selfw, bnode
-    [2, (hi0 - lo0) + (hi1 - lo1)]): one rank's block of the row-sharded step."""
-    dev = src32.device
-    Rl = (r0[1] - r0[0]) + (r1[1] - r1[0])
-    cnt = torch.empty(max(N, 1), dtype=torch.int32, device=dev)
-    centre = torch.empty((2, Rl), dtype=torch.int32, device=dev)
-    dinv = torch.empty((2, Rl), dtype=torch.float32, device=dev)
-    selfw = torch.empty((2, Rl), dtype=torch.float32, device=dev)
-    bnode = torch.empty((2, Rl), dtype=torch.int32, device=dev)
-    check(lib.twowl_wedge_prepare_ranges(src32.data_ptr(), dst_e32.data_ptr(), E, R, N, _p(blocked), in_ptr.data_ptr(), int(r0[0]),
-                                         int(r0[1]), int(r1[0]), int(r1[1]), cnt.data_ptr(), centre.data_ptr(), dinv.data_ptr(),
-                                         selfw.data_ptr(), bnode.data_ptr(), _stream()), "wedge_prepare_ranges")
-    _count(4)
+    check(lib.twowl_wedge_prepare(src32.data_ptr(), dst_e32.data_ptr(), E, R, N, _p(blocked), in_ptr.data_ptr(), int(lo0), int(hi0),
+                                  int(lo1), int(hi1), cnt.data_ptr(), centre.data_ptr(), dinv.data_ptr(), selfw.data_ptr(),
+                                  bnode.data_ptr(), _stream()), "wedge_prepare")
+    _count(2 + (hi0 > lo0) + (hi1 > lo1))
     return cnt, centre, dinv, selfw, bnode
 
 
@@ -1002,26 +935,11 @@ def graphnorm_apply2(xf, xr, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r:
     return out
 
 
-def graphnorm_bwd2(xf, xr, dout, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r: int, relu: bool):
-    M, C = xf.shape
-    dxf, dxr = torch.empty_like(xf), torch.empty_like(xr)
-    dpf = torch.empty(4 * C, dtype=torch.float32, device=xf.device)
-    dpr = torch.empty(4 * C, dtype=torch.float32, device=xf.device)
-    nb = lib.twowl_graphnorm_bwd2_workspace_bytes(M, C)
-    ws = _ws(nb, xf.device)
-    with _P("graphnorm_bwd2", M * C * 4 * 8):
-        check(lib.twowl_graphnorm_bwd2(xf.data_ptr(), xr.data_ptr(), dout.data_ptr(), M, C, sf.data_ptr(), sr.data_ptr(),
-                                       pf[0].data_ptr(), pf[1].data_ptr(), pf[2].data_ptr(), pr[0].data_ptr(), pr[1].data_ptr(),
-                                       pr[2].data_ptr(), float(p_drop), int(seed_f), int(seed_r), int(relu), dxf.data_ptr(),
-                                       dxr.data_ptr(), dpf.data_ptr(), dpr.data_ptr(), ws.data_ptr(), nb, _stream()),
-              "graphnorm_bwd2")
-    _count(4)
-    return dxf, dxr, dpf, dpr
-
-
-def graphnorm_bwd2_sharded(xf, xr, dout, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r: int, relu: bool, M_total: int, all_reduce):
-    """graphnorm_bwd2 over this rank's rows of a row-sharded pair table: the fp64 column sums [4,C] are summed over the ranks by
-    `all_reduce` (a callable applied in place) between the two halves. -> (dxf, dxr, dparams_f, dparams_r) as graphnorm_bwd2."""
+def graphnorm_bwd2(xf, xr, dout, sf, sr, pf, pr, p_drop: float, seed_f: int, seed_r: int, relu: bool, M_total: Optional[int] = None,
+                   all_reduce=None):
+    """Backward of graphnorm_apply2 -> (dxf, dxr, dparams_f, dparams_r). On one row block of a row-sharded pair table,
+    `all_reduce` (a callable applied in place) sums the fp64 column sums [4,C] over the ranks between the two halves, and M_total
+    is the whole table's row count (default: M)."""
     M, C = xf.shape
     dev = xf.device
     colsums = torch.empty((4, C), dtype=torch.float64, device=dev)
@@ -1033,7 +951,8 @@ def graphnorm_bwd2_sharded(xf, xr, dout, sf, sr, pf, pr, p_drop: float, seed_f: 
         check(lib.twowl_graphnorm_bwd2_sums(xf.data_ptr(), xr.data_ptr(), dout.data_ptr(), M, C, *ptrs, colsums.data_ptr(),
                                             ws.data_ptr(), nb, _stream()), "graphnorm_bwd2_sums")
     _count(2)
-    all_reduce(colsums)
+    if all_reduce is not None:
+        all_reduce(colsums)
     dxf, dxr = torch.empty_like(xf), torch.empty_like(xr)
     dpf = torch.empty(4 * C, dtype=torch.float32, device=dev)
     dpr = torch.empty(4 * C, dtype=torch.float32, device=dev)
@@ -1041,8 +960,8 @@ def graphnorm_bwd2_sharded(xf, xr, dout, sf, sr, pf, pr, p_drop: float, seed_f: 
     ws2 = _ws(nb2, dev)
     with _P("graphnorm_bwd2", M * C * 4 * 5):
         check(lib.twowl_graphnorm_bwd2_apply(xf.data_ptr(), xr.data_ptr(), dout.data_ptr(), M, C, *ptrs, colsums.data_ptr(),
-                                             int(M_total), dxf.data_ptr(), dxr.data_ptr(), dpf.data_ptr(), dpr.data_ptr(),
-                                             ws2.data_ptr(), nb2, _stream()), "graphnorm_bwd2_apply")
+                                             int(M if M_total is None else M_total), dxf.data_ptr(), dxr.data_ptr(), dpf.data_ptr(),
+                                             dpr.data_ptr(), ws2.data_ptr(), nb2, _stream()), "graphnorm_bwd2_apply")
     _count(3)
     return dxf, dxr, dpf, dpr
 

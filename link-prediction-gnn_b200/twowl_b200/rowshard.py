@@ -330,7 +330,7 @@ def node_graph_block(edge1, N: int, shard: "RowShard") -> G.NodeGraph:
     if t1 > t0:
         ops.gather_u8(tag[1], base.tids[t0:t1], out=temask[t0:t1])
     dinv = torch.empty(B * shard.world, dtype=torch.float32, device=base.ids.device)
-    ops.gcn_dinv_entries_rows(base.ptr, base.col, N, emask, lo, hi, dinv)
+    ops.gcn_dinv_entries(base.ptr, base.col, N, emask, rows=(lo, hi), out=dinv)
     shard.all_gather_blocks(dinv.view(-1, 1), B, "node dinv [N]")
     return G.NodeGraph(N, base.ptr, base.col, base.tptr, base.tcol, dinv[:N], base.plan, base.tplan, base.ids, base.tids, emask, temask)
 
@@ -507,9 +507,8 @@ class _ShardedPairLayer(torch.autograd.Function):
         H, wf, gwf, gbf, gmf, wr, gwr, gbr, gmr, Of, Or, sf, sr, SH, *rows = ctx.saved_tensors
         shard, loc, R_total, n_node, p_drop, seed_f, seed_r = ctx.meta
         C = wf.shape[0]
-        dOf, dOr, dpf, dpr = ops.graphnorm_bwd2_sharded(Of, Or, g.contiguous(), sf, sr, (gwf, gbf, gmf), (gwr, gbr, gmr), p_drop, seed_f,
-                                                        seed_r, True, R_total,
-                                                        lambda t: shard.all_reduce(t, "GraphNorm-backward column sums [4,C] f64"))
+        dOf, dOr, dpf, dpr = ops.graphnorm_bwd2(Of, Or, g.contiguous(), sf, sr, (gwf, gbf, gmf), (gwr, gbr, gmr), p_drop, seed_f, seed_r,
+                                                True, R_total, lambda t: shard.all_reduce(t, "GraphNorm-backward column sums [4,C] f64"))
         dWf, dWr = ops.pair_dw(dOf, dOr, rows[2][0], rows[2][1], H)
         dh, dWf, dWr = _layer_backward(shard, loc, rows, n_node, H, wf, wr, SH, dOf, dOr, dWf, dWr)
         gf, gr = _param_grads(shard, C, dpf, dpr)
@@ -546,10 +545,9 @@ class _ShardedLastLayer(torch.autograd.Function):
         shard, loc, R_total, n_node, p_drop, seed_f, seed_r, init_inside = ctx.meta
         C = wf.shape[0]
         pf, pr = (gwf, gbf, gmf), (gwr, gbr, gmr)
-        Gp, head, nxt, colsums = ops.gn2_readout_bwd_rows(Of, Or, sf, sr, pf, pr, p_drop, seed_f, seed_r, True, idx_l, pw.contiguous(),
-                                                          g.reshape(-1))
-        shard.all_reduce(colsums, "readout / GraphNorm-backward column sums [6,C] f64")
-        consts, dpf, dpr, dpw, dpb = ops.gn2_readout_bwd_finish(colsums, R_total, sf, sr, pf, pr)
+        Gp, head, nxt, consts, dpf, dpr, dpw, dpb = ops.gn2_readout_bwd_prepare(
+            Of, Or, sf, sr, pf, pr, p_drop, seed_f, seed_r, True, idx_l, pw.contiguous(), g.reshape(-1), R_total,
+            lambda t: shard.all_reduce(t, "readout / GraphNorm-backward column sums [6,C] f64"))
         dOf, dOr, dWf, dWr = ops.pair_dw_gn(Of, Or, consts, Gp, head, nxt, p_drop, seed_f, seed_r, True, rows[2][0], rows[2][1], H)
         dh, dWf, dWr = _layer_backward(shard, loc, rows, n_node, H, wf, wr, SH, dOf, dOr, dWf, dWr, pair_sum_out=init_inside)
         if init_inside:      # dh holds one row per pair: this block's part of dx from it, summed over the ranks range by range
@@ -649,8 +647,8 @@ def forward_pairs(model, x, pos, idx, ei2):
     ranges = blocks_of(wedges.E, pt.R, shard.rank, shard.world)
     loc = _local(wedges, pt, ranges, shard.chunks if shard.world > 1 else 1)
     # per-row constants of THIS block only (the degree counts are global: every rank holds the int edge lists)
-    _, centre, dinv, selfw, bnode = ops.wedge_prepare_ranges(wedges.src, wedges.dst_e, wedges.E, wedges.R, wedges.n_node, wedges.blocked,
-                                                             wedges.in_ptr, ranges[0], ranges[1])
+    _, centre, dinv, selfw, bnode = ops.wedge_prepare(wedges.src, wedges.dst_e, wedges.E, wedges.R, wedges.n_node, wedges.blocked,
+                                                      wedges.in_ptr, ranges)
     rows = (centre, dinv, selfw, bnode)
     blocked_l = wedges.blocked[ranges[0][0]:ranges[0][1]] if wedges.blocked is not None else None
     idx_l, link_dest = own_links_first(mask_links(idx, ranges))

@@ -662,7 +662,7 @@ def test_pair_dw_wide_tiles_vs_fp64(U, M, Co, Ci):
 @pytest.mark.parametrize("M,C,L,p", [(64, 64, 10, 0.0), (5000, 32, 700, 0.3), (70001, 64, 9000, 0.0), (70001, 64, 9000, 0.5),
                                      (40001, 128, 5000, 0.0), (40001, 128, 5000, 0.4)])
 def test_pair_dw_gn_matches_two_pass(U, M, C, L, p):
-    """twowl_gn2_readout_bwd_prepare + twowl_pair_dw_gn (GraphNorm backward made inside the weight-gradient kernel) against
+    """twowl_gn2_readout_bwd_rows + _finish + twowl_pair_dw_gn (GraphNorm backward made inside the weight-gradient kernel) against
     the two-pass path twowl_gn2_readout_bwd + twowl_pair_dw: same dO_f, dO_r, dW_f, dW_r and parameter gradients."""
     from twowl_b200 import ops
     torch.manual_seed(M + C + L)
