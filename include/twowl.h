@@ -587,6 +587,53 @@ int twowl_n2v_step(float* emb, float* exp_avg, float* exp_avg_sq, int64_t* step,
 int twowl_embedding_dot(const float* emb, int64_t num_nodes, int32_t d, const int64_t* u, int64_t s_u, const int64_t* v, int64_t s_v,
                         int64_t P, float* out, void* stream);
 
+/* SEAL (Zhang & Chen 2018) enclosing subgraphs over a simple adjacency (ptr, adj) of twowl_simple_adjacency, one per query pair
+ * (u[q], v[q]) (int64, element strides):
+ *   nodes:  layer 0 = {u, v}; layer t (1 <= t <= hops, hops in {1, 2, 3}) = the neighbours of layer t-1 not seen in an earlier
+ *           layer. A layer of more than max_nodes_per_hop nodes (0 = no cap) keeps the max_nodes_per_hop with the smallest
+ *           hash_u32(seed, (index_base + q) << 32 | node), ties by id; the dropped nodes count as seen (the SEAL authors'
+ *           k_hop_subgraph). The subgraph's nodes are listed in ascending global id (its local order).
+ *   edges:  the induced edges minus (u, v) and (v, u), both directions, as ids into the batch's node list (node_ptr[q] + local),
+ *           in (row, col) order: edge_index = int64 [2, n_edges] (rows, then cols).
+ *   z:      DRNL: du = BFS distance from u in the subgraph without v, dv from v without u, d = du + dv,
+ *           z = 1 + min(du, dv) + (d/2) (d/2 + d%2 - 1); z(u) = z(v) = 1; 0 where du or dv is infinite (int32).
+ *   twowl_seal_count: node_ptr / edge_ptr (int64 [Q+1]) = exclusive scans of the per-query node and edge counts; info (int64[2])
+ *           = (endpoints outside [0, num_nodes), queries with u == v). A refused query counts 0 and is skipped by the fill.
+ *   twowl_seal_fill: nodes (int64), z and edge_index from the count's node_ptr / edge_ptr, n_edges = edge_ptr[Q].
+ * One CTA per query over `blocks` CTAs, each with a workspace slice of 5 num_nodes + 1 int32 (twowl_seal_workspace_bytes): any
+ * subgraph size fits. The result depends on (seed, index_base + q, u[q], v[q]) and the graph alone; bitwise repeatable. */
+size_t twowl_seal_workspace_bytes(int64_t num_nodes, int64_t Q, int64_t blocks);
+int twowl_seal_count(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* u, int64_t s_u, const int64_t* v,
+                     int64_t s_v, int64_t Q, int64_t index_base, int32_t hops, int32_t max_nodes_per_hop, uint64_t seed,
+                     int64_t blocks, int64_t* node_ptr, int64_t* edge_ptr, int64_t* info, void* ws, size_t ws_bytes, void* stream);
+int twowl_seal_fill(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const int64_t* u, int64_t s_u, const int64_t* v,
+                    int64_t s_v, int64_t Q, int64_t index_base, int32_t hops, int32_t max_nodes_per_hop, uint64_t seed,
+                    int64_t blocks, const int64_t* node_ptr, const int64_t* edge_ptr, int64_t n_edges, int64_t* nodes,
+                    int32_t* z, int64_t* edge_index, void* ws, size_t ws_bytes, void* stream);
+
+/* DGCNN pieces (SEAL's readout over a batch of subgraphs), fp32, any width:
+ *   label_gather:  out[m, c] (+= with accumulate) W[c ld + min(max(z[m], 0), ld - 1)]: the linear map of one_hot(z) by W [C, ld].
+ *   tanh_slice:    fwd out[m ld + off + c] = tanh(h[m, c]) for h [M, C]; bwd dh[m, c] = g[o] (1 - y[o]^2), o = m ld + off + c.
+ *   sortpool:      per graph b (rows [gptr[b], gptr[b+1]) of X [*, D]) the rows by X[., key_col] descending, ties by row, the first k
+ *                  into out [B, k, D] and their rows into idx [B, k] (-1 and zeros past the graph's size). bwd: dX [n_rows, D] =
+ *                  g routed back to the kept rows, 0 elsewhere (written, no accumulation).
+ *   bias_act:      out [B, Lin / pool, C] = dropout_p(max over pool consecutive rows of act(Y [B, Lin, C] + bias)), act = ReLU when
+ *                  relu, pool 1 or 2 (ties to the first row), dropout mask hash_u32(seed, output index). bwd: dY [B, Lin, C].
+ *   im2col:        out [B L2, C kw] with out[b L2 + p, c kw + j] = P[b, p + j, c] (P [B, L1, C], L2 = L1 - kw + 1): Conv1d(C, ., kw)
+ *                  as one product with weight.view(out, C kw). bwd: dP summed over j in ascending order (no atomics). */
+int twowl_label_gather(const float* W, int32_t C, int64_t ld, const int64_t* z, int64_t M, int32_t accumulate, float* out, void* stream);
+int twowl_tanh_slice_fwd(const float* h, int64_t M, int32_t C, float* out, int64_t ld, int64_t off, void* stream);
+int twowl_tanh_slice_bwd(const float* g, const float* y, int64_t ld, int64_t off, int64_t M, int32_t C, float* dh, void* stream);
+int twowl_sortpool_fwd(const float* X, int32_t D, int32_t key_col, const int64_t* gptr, int64_t B, int32_t k, float* out, int32_t* idx,
+                       void* stream);
+int twowl_sortpool_bwd(const float* g, const int32_t* idx, int64_t B, int32_t k, int32_t D, int64_t n_rows, float* dX, void* stream);
+int twowl_bias_act_fwd(const float* Y, const float* bias, int64_t B, int32_t Lin, int32_t C, int32_t pool, int32_t relu, float p_drop,
+                       uint64_t seed, float* out, void* stream);
+int twowl_bias_act_bwd(const float* g, const float* Y, const float* bias, int64_t B, int32_t Lin, int32_t C, int32_t pool, int32_t relu,
+                       float p_drop, uint64_t seed, float* dY, void* stream);
+int twowl_im2col_fwd(const float* P, int64_t B, int32_t L1, int32_t C, int32_t kw, float* out, void* stream);
+int twowl_im2col_bwd(const float* g, int64_t B, int32_t L1, int32_t C, int32_t kw, float* dP, void* stream);
+
 /* ------------------------------------------------------------------ structured wedge path ------- */
 
 /* When ei2 is the full wedge join of (pos_edge, pred_edge) minus the wedges whose source edge is blocked

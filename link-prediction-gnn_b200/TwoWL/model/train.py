@@ -290,3 +290,77 @@ def train_routine(dsname, mod, opt, trn_ds, val_ds, tst_ds, epoch, verbose=True,
     if verbose and record_dir is not None:
         _record_run(record_dir, dsname, tst_score, finished - started, fpr, tpr)
     return best_val
+
+
+def _seal_graph(dataset):
+    from twowl_b200 import graph
+    return graph.simple_adjacency(dataset.ei, dataset.x.shape[0])
+
+
+def _seal_train_pairs(dataset):
+    """SEAL's training targets: the undirected pairs of ei (pos1[:E:2], label 1) and the negatives pos1[E::2] (label 0)."""
+    n_edges = dataset.ei.shape[1]
+    pos, neg = dataset.pos1[:n_edges:2], dataset.pos1[n_edges::2]
+    y = torch.cat((torch.ones(pos.shape[0], device=pos.device), torch.zeros(neg.shape[0], device=pos.device)))
+    return torch.cat((pos, neg)).to(torch.long), y
+
+
+def seal_fit(trn_ds, epochs, batch_size, lr=1e-4, hops=1, max_nodes_per_hop=0, seed=0, node_feat=None, hidden=32, num_layers=3,
+             dropout=0.5):
+    """Train SEAL's DGCNN (TwoWL.model.seal) on a training split (extension: the reference's SEAL baseline, SURVEY row 6)
+    -> (model, losses float64 [steps]). Targets: every undirected pair of trn_ds.ei and the negatives pos1[E::2]; each batch of
+    batch_size targets (a seeded permutation per epoch) gets its enclosing subgraphs extracted on the fly over the split's graph
+    (ops.seal_subgraphs, hops / max_nodes_per_hop), then forward, BCE-with-logits, backward and a FusedAdam step (lr). SortPooling's
+    k and max_z come from the training subgraphs (PyG's 60% rule, seal.sort_pool_k). node_feat [N, F] is optional per-node input.
+    The same seed gives the same losses and weights bit for bit."""
+    from TwoWL.model.seal import DGCNN, sort_pool_k
+    from twowl_b200.optim import FusedAdam
+    ptr, adj = _seal_graph(trn_ds)
+    pairs, y = _seal_train_pairs(trn_ds)
+    T = pairs.shape[0]
+    sub_kw = dict(hops=hops, max_nodes_per_hop=max_nodes_per_hop, seed=seed)
+    sizes = ops.seal_subgraph_sizes(ptr, adj, pairs[:, 0], pairs[:, 1], **sub_kw)
+    max_z = 1
+    for q in range(0, T, 4096):
+        sub = ops.seal_subgraphs(ptr, adj, pairs[q:q + 4096, 0], pairs[q:q + 4096, 1], index_base=q, **sub_kw)
+        max_z = max(max_z, int(sub.z.max()) if sub.z.numel() else 1)
+    with torch.random.fork_rng(devices=[pairs.device]):
+        torch.manual_seed(seed)
+        mod = DGCNN(max_z, sort_pool_k(sizes), hidden, num_layers, 0 if node_feat is None else node_feat.shape[1], dropout)
+    mod = mod.to(pairs.device).train()
+    opt = FusedAdam(mod.parameters(), lr=lr)
+    gen = torch.Generator(device="cpu")
+    gen.manual_seed(seed)
+    losses = []
+    step = 0
+    for _ in range(epochs):
+        perm = torch.randperm(T, generator=gen).to(pairs.device)
+        for b in range(0, T, batch_size):
+            ids = perm[b:b + batch_size]
+            # a capped layer's sample keys on the target's position in this epoch's order: a fresh sample per epoch
+            sub = ops.seal_subgraphs(ptr, adj, pairs[ids, 0], pairs[ids, 1], index_base=b, **sub_kw)
+            opt.zero_grad()
+            loss = F2.bce_with_logits(mod(sub, node_feat, seed=(seed * 1000003 + step) % (2 ** 62)), y[ids].unsqueeze(-1))
+            loss.backward()
+            opt.step()
+            losses.append(loss.detach().double().reshape(1))
+            step += 1
+    mod.eval()
+    return mod, (torch.cat(losses).cpu() if losses else torch.zeros(0, dtype=torch.float64))
+
+
+@torch.no_grad()
+def seal_scores(mod, dataset, hops=1, max_nodes_per_hop=0, seed=0, node_feat=None, batch_size=1024):
+    """SEAL logits of the dataset's prediction pairs pos1[E::2] -> fp32 [P], in the order of test(): each pair's enclosing subgraph
+    over the split's graph (ops.seal_subgraphs, index_base = the pair's index), scored by the DGCNN in eval mode.
+    rank_scores(seal_scores(mod, ds), ds) and ops.auc(scores, ds.y[0::2]) rank it like any other score."""
+    mod.eval()
+    ptr, adj = _seal_graph(dataset)
+    n_edges = dataset.ei.shape[1]
+    pairs = dataset.pos1[n_edges::2][: dataset.y.shape[0] // 2].to(torch.long)
+    out = []
+    for q in range(0, pairs.shape[0], batch_size):
+        sub = ops.seal_subgraphs(ptr, adj, pairs[q:q + batch_size, 0], pairs[q:q + batch_size, 1], hops=hops,
+                                 max_nodes_per_hop=max_nodes_per_hop, seed=seed, index_base=q)
+        out.append(mod(sub, node_feat).reshape(-1))
+    return torch.cat(out) if out else torch.zeros(0, device=pairs.device)

@@ -8,7 +8,7 @@ instead of CSR by target), not an autograd trace of torch ops.
 """
 from __future__ import annotations
 
-from typing import Optional, Tuple
+from typing import List, Optional, Tuple
 
 import torch
 from torch import Tensor
@@ -656,3 +656,170 @@ def bce_with_logits(logits: Tensor, labels: Tensor) -> Tensor:
     """F.binary_cross_entropy_with_logits(logits, labels) (mean reduction, train.py:37) with its gradient made in the same pass:
     two launches for loss forward + backward instead of torch's chain."""
     return _bce_with_logits(logits, labels)[0]
+
+
+# ------------------------------------------------------------------------------ SEAL / DGCNN (TwoWL/model/seal.py)
+
+
+@torch.library.custom_op("twowl::seal_input", mutates_args=())
+def seal_input(weight: Tensor, z: Tensor, feat: Optional[Tensor]) -> Tensor:
+    """The first GCNConv's linear map of [one_hot(z, L) | feat] by weight [C, L + F] (L = weight.shape[1] - F, z in [0, L)): the
+    feature product, then the columns weight[:, z] added by a gather (no one-hot matrix)."""
+    L = weight.shape[1] - (0 if feat is None else feat.shape[1])
+    if feat is None:
+        return ops.label_gather(weight, z)
+    out = ops.linear_fwd(_pad4(feat), _pad4(weight[:, L:]))
+    return ops.label_gather(weight, z, out=out)
+
+
+@seal_input.register_fake
+def _(weight, z, feat):
+    return weight.new_empty((z.numel(), weight.shape[0]))
+
+
+def _si_setup(ctx, inputs, output):
+    weight, z, feat = inputs
+    ctx.save_for_backward(z, feat)
+    ctx.L = weight.shape[1] - (0 if feat is None else feat.shape[1])
+
+
+def _si_bwd(ctx, g):
+    z, feat = ctx.saved_tensors
+    g = g.contiguous()
+    # d weight[:, l] = sum of g over the nodes labelled l: a segmented sum over the nodes grouped by label
+    ptr, ids = ops.csr_build(z, ctx.L)
+    dW = ops.seg_reduce(ptr, ids, ctx.L, g, plan=ops.seg_plan(ptr, ctx.L, ids.numel())).t()
+    if feat is not None:
+        dW = torch.cat((dW, ops.linear_bwd_weight(g, _pad4(feat))[:, :feat.shape[1]]), dim=1)
+    return dW.contiguous(), None, None
+
+
+seal_input.register_autograd(_si_bwd, setup_context=_si_setup)
+
+
+@torch.library.custom_op("twowl::seal_tanh", mutates_args=())
+def seal_tanh(h: Tensor) -> Tensor:
+    return ops.tanh_slice_fwd(h, torch.empty_like(h), 0)
+
+
+@seal_tanh.register_fake
+def _(h):
+    return torch.empty_like(h)
+
+
+def _st_setup(ctx, inputs, output):
+    ctx.save_for_backward(output)
+
+
+def _st_bwd(ctx, g):
+    (y,) = ctx.saved_tensors
+    return ops.tanh_slice_bwd(g.contiguous(), y, 0, y.shape[1])
+
+
+seal_tanh.register_autograd(_st_bwd, setup_context=_st_setup)
+
+
+@torch.library.custom_op("twowl::seal_tanh_concat", mutates_args=())
+def seal_tanh_concat(hs: List[Tensor], offs: List[int], width: int) -> Tensor:
+    """[n, width]: tanh(hs[i]) in columns [offs[i], offs[i] + hs[i].shape[1]], zeros elsewhere (DGCNN's concatenated latents)."""
+    out = hs[0].new_zeros((hs[0].shape[0], width))
+    for h, off in zip(hs, offs):
+        ops.tanh_slice_fwd(h, out, off)
+    return out
+
+
+@seal_tanh_concat.register_fake
+def _(hs, offs, width):
+    return hs[0].new_empty((hs[0].shape[0], width))
+
+
+def _stc_setup(ctx, inputs, output):
+    hs, offs, width = inputs
+    ctx.save_for_backward(output)
+    ctx.meta = [(off, h.shape[1]) for h, off in zip(hs, offs)]
+
+
+def _stc_bwd(ctx, g):
+    (y,) = ctx.saved_tensors
+    g = g.contiguous()
+    return [ops.tanh_slice_bwd(g, y, off, C) for off, C in ctx.meta], None, None
+
+
+seal_tanh_concat.register_autograd(_stc_bwd, setup_context=_stc_setup)
+
+
+@torch.library.custom_op("twowl::sort_pool", mutates_args=())
+def sort_pool(x: Tensor, gptr: Tensor, k: int, key_col: int) -> Tuple[Tensor, Tensor]:
+    """PyG global_sort_pool with ties broken by row -> (out [B, k, D], idx int32 [B, k]); only out is differentiable."""
+    return ops.sortpool_fwd(x, gptr, k, key_col)
+
+
+@sort_pool.register_fake
+def _(x, gptr, k, key_col):
+    B = gptr.shape[0] - 1
+    return x.new_empty((B, k, x.shape[1])), x.new_empty((B, k), dtype=torch.int32)
+
+
+def _sp_setup(ctx, inputs, output):
+    ctx.save_for_backward(output[1])
+    ctx.n_rows = inputs[0].shape[0]
+    ctx.mark_non_differentiable(output[1])
+    ctx.set_materialize_grads(False)
+
+
+def _sp_bwd(ctx, g, _g_idx):
+    (idx,) = ctx.saved_tensors
+    return ops.sortpool_bwd(g, idx, ctx.n_rows), None, None, None
+
+
+sort_pool.register_autograd(_sp_bwd, setup_context=_sp_setup)
+
+
+@torch.library.custom_op("twowl::bias_act", mutates_args=())
+def bias_act(y: Tensor, bias: Tensor, B: int, pool: int, relu: bool, p_drop: float, seed: int) -> Tensor:
+    """ops.bias_act_fwd: bias + ReLU (optional) + max-pool over `pool` rows + dropout, y [B * Lin, C]."""
+    return ops.bias_act_fwd(y, bias, B, pool, relu, p_drop, seed)
+
+
+@bias_act.register_fake
+def _(y, bias, B, pool, relu, p_drop, seed):
+    return y.new_empty((B * ((y.shape[0] // max(B, 1)) // pool), y.shape[1]))
+
+
+def _ba_setup(ctx, inputs, output):
+    y, bias, B, pool, relu, p_drop, seed = inputs
+    ctx.save_for_backward(y, bias)
+    ctx.meta = (B, pool, relu, p_drop, seed)
+
+
+def _ba_bwd(ctx, g):
+    y, bias = ctx.saved_tensors
+    dy = ops.bias_act_bwd(g, y, bias, *ctx.meta)
+    return dy, ops.colsum(dy), None, None, None, None, None
+
+
+bias_act.register_autograd(_ba_bwd, setup_context=_ba_setup)
+
+
+@torch.library.custom_op("twowl::im2col", mutates_args=())
+def im2col(p: Tensor, B: int, kw: int) -> Tensor:
+    """ops.im2col_fwd: Conv1d's input windows as rows, p [B * L1, C] -> [B * (L1 - kw + 1), C * kw]."""
+    return ops.im2col_fwd(p, B, kw)
+
+
+@im2col.register_fake
+def _(p, B, kw):
+    L1 = p.shape[0] // B
+    return p.new_empty((B * (L1 - kw + 1), p.shape[1] * kw))
+
+
+def _i2c_setup(ctx, inputs, output):
+    p, B, kw = inputs
+    ctx.meta = (B, p.shape[0] // B, p.shape[1], kw)
+
+
+def _i2c_bwd(ctx, g):
+    return ops.im2col_bwd(g, *ctx.meta), None, None
+
+
+im2col.register_autograd(_i2c_bwd, setup_context=_i2c_setup)

@@ -1550,3 +1550,204 @@ def node2vec(ptr: torch.Tensor, adj: torch.Tensor, dim: int = 128, walk_length: 
             total += _n2v_step(emb, exp_avg, exp_avg_sq, step, walks, negs, win, lr, (0.9, 0.999), 1e-8)
         losses[e] = total / -(-W // bw)
     return emb, losses
+
+
+# ------------------------------------------------------------------------------ SEAL: enclosing subgraphs and DGCNN pieces
+
+SEAL_MAX_WORKSPACE = 1 << 32   # default extraction workspace: 20 B per graph node for each CTA that runs at once
+_SEAL_MAX_BLOCKS = 4 * 148
+
+
+class SealBatch:
+    """A batch of enclosing subgraphs (seal_subgraphs): node_ptr int64 [Q+1], nodes int64 [n] (global ids, ascending within a
+    subgraph), z int32 [n] (DRNL labels), edge_index int64 [2, m] (ids into the batch's nodes, both directions, sorted by
+    (row, col), block-diagonal by subgraph) and batch int64 [n] (each node's subgraph)."""
+    __slots__ = ("node_ptr", "nodes", "z", "edge_index", "batch")
+
+    def __init__(self, node_ptr, nodes, z, edge_index, batch):
+        self.node_ptr, self.nodes, self.z, self.edge_index, self.batch = node_ptr, nodes, z, edge_index, batch
+
+    @property
+    def num_graphs(self) -> int:
+        return self.node_ptr.numel() - 1
+
+
+def _seal_args(fn: str, ptr, adj, src, dst, hops, max_nodes_per_hop, seed, index_base, max_workspace):
+    _need_cuda(ptr, adj, src, dst)
+    assert ptr.dim() == 1 and ptr.dtype == torch.int64 and ptr.is_contiguous(), f"{fn}: ptr must be contiguous int64 [N+1]"
+    assert adj.dim() == 1 and adj.dtype == torch.int32 and adj.is_contiguous(), f"{fn}: adj must be contiguous int32"
+    hops, cap = int(hops), int(max_nodes_per_hop)
+    if hops not in (1, 2, 3):
+        raise ValueError(f"{fn}: hops must be 1, 2 or 3, got {hops}")
+    if not 0 <= cap < 2 ** 31:
+        raise ValueError(f"{fn}: max_nodes_per_hop must be in [0, 2^31), got {cap}")
+    if not 0 <= int(index_base) < 2 ** 31:
+        raise ValueError(f"{fn}: index_base must be in [0, 2^31), got {index_base}")
+    src, dst = src.reshape(-1).to(torch.int64), dst.reshape(-1).to(torch.int64)
+    assert src.numel() == dst.numel(), f"{fn}: src / dst size mismatch"
+    n, Q = ptr.numel() - 1, src.numel()
+    budget = SEAL_MAX_WORKSPACE if max_workspace is None else int(max_workspace)
+    per_block = lib.twowl_seal_workspace_bytes(n, 0, 2) - lib.twowl_seal_workspace_bytes(n, 0, 1)
+    blocks = int(max(1, min(_SEAL_MAX_BLOCKS, max(Q, 1), budget // max(per_block, 1))))
+    nb = lib.twowl_seal_workspace_bytes(n, Q, blocks)
+    (ps, ss), (pd, sd) = (_row(src), _row(dst)) if Q else ((0, 1), (0, 1))
+    return (ptr.data_ptr(), adj.data_ptr(), n, ps, ss, pd, sd, Q, int(index_base), hops, cap, int(seed) & (2 ** 64 - 1), blocks), \
+        _ws(nb, ptr.device), nb, src, dst
+
+
+def _seal_count(fn, args, ws, nb, dev):
+    Q = args[7]
+    node_ptr = torch.empty(Q + 1, dtype=torch.int64, device=dev)
+    edge_ptr = torch.empty(Q + 1, dtype=torch.int64, device=dev)
+    info = torch.empty(2, dtype=torch.int64, device=dev)
+    check(lib.twowl_seal_count(*args, node_ptr.data_ptr(), edge_ptr.data_ptr(), info.data_ptr(), ws.data_ptr(), nb, _stream()), "seal_count")
+    _count(1 + 2 * 3 + int(Q > 0))
+    nbad, nself, n_nodes, n_edges = torch.cat((info, node_ptr[Q:], edge_ptr[Q:])).tolist()
+    if nbad:
+        raise IndexError(f"{fn}: {nbad} query id(s) outside [0, {args[2]})")
+    if nself:
+        raise ValueError(f"{fn}: {nself} query pair(s) with u == v")
+    return node_ptr, edge_ptr, n_nodes, n_edges
+
+
+def seal_subgraph_sizes(ptr: torch.Tensor, adj: torch.Tensor, src: torch.Tensor, dst: torch.Tensor, hops: int = 1,
+                        max_nodes_per_hop: int = 0, seed: int = 0, index_base: int = 0,
+                        max_workspace: Optional[int] = None) -> torch.Tensor:
+    """The node count of each pair's enclosing subgraph (the count pass of seal_subgraphs alone) -> int64 [Q]."""
+    args, ws, nb, src, dst = _seal_args("seal_subgraph_sizes", ptr, adj, src, dst, hops, max_nodes_per_hop, seed, index_base,
+                                        max_workspace)
+    node_ptr = _seal_count("seal_subgraph_sizes", args, ws, nb, ptr.device)[0]
+    return node_ptr[1:] - node_ptr[:-1]
+
+
+def seal_subgraphs(ptr: torch.Tensor, adj: torch.Tensor, src: torch.Tensor, dst: torch.Tensor, hops: int = 1,
+                   max_nodes_per_hop: int = 0, seed: int = 0, index_base: int = 0,
+                   max_workspace: Optional[int] = None) -> SealBatch:
+    """SEAL's enclosing subgraph of each pair (src[q], dst[q]) over a simple adjacency (simple_adjacency) -> SealBatch.
+
+    Nodes: {u, v}, then `hops` layers of unseen neighbours; a layer of more than max_nodes_per_hop nodes (0 = no cap) keeps the
+    ones with the smallest hash of (seed, index_base + q, node), ties by id, and the dropped ones stay seen (the SEAL authors'
+    k_hop_subgraph). The local order is ascending global id (PyG's relabel_nodes). Edges: the induced subgraph minus (u, v) and
+    (v, u). z: DRNL labels (PyG's drnl_node_labeling, in integers). A caller that cuts one query list into several calls passes
+    each call's offset as index_base to get the same subgraphs as one call. The result is bitwise repeatable and does not depend
+    on max_workspace (default SEAL_MAX_WORKSPACE), which only bounds how many queries run at once. One host read (the counts);
+    raises IndexError for an id outside [0, N) and ValueError for u == v, hops outside {1, 2, 3} or a negative cap."""
+    fn = "seal_subgraphs"
+    args, ws, nb, src, dst = _seal_args(fn, ptr, adj, src, dst, hops, max_nodes_per_hop, seed, index_base, max_workspace)
+    dev = ptr.device
+    node_ptr, edge_ptr, n_nodes, n_edges = _seal_count(fn, args, ws, nb, dev)
+    nodes = torch.empty(n_nodes, dtype=torch.int64, device=dev)
+    z = torch.empty(n_nodes, dtype=torch.int32, device=dev)
+    edge_index = torch.empty((2, n_edges), dtype=torch.int64, device=dev)
+    check(lib.twowl_seal_fill(*args, node_ptr.data_ptr(), edge_ptr.data_ptr(), n_edges, _p(nodes) if n_nodes else None,
+                              _p(z) if n_nodes else None, _p(edge_index) if n_edges else None, ws.data_ptr(), nb, _stream()),
+          "seal_fill")
+    _count(2)
+    Q = args[7]
+    batch = torch.repeat_interleave(torch.arange(Q, device=dev), node_ptr[1:] - node_ptr[:-1], output_size=n_nodes)
+    return SealBatch(node_ptr, nodes, z, edge_index, batch)
+
+
+def label_gather(W: torch.Tensor, z: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """out[m] (+)= W[:, z[m]] for W [C, L] (the linear map of one_hot(z, L) by W, without the one-hot matrix). With `out` the
+    columns are added to it in place."""
+    _need_cuda(W, z)
+    W = W.contiguous()
+    z = z.reshape(-1).to(torch.int64).contiguous()
+    C, L = W.shape
+    acc = out is not None
+    if out is None:
+        out = torch.empty((z.numel(), C), dtype=torch.float32, device=W.device)
+    check(lib.twowl_label_gather(W.data_ptr(), C, L, z.data_ptr(), z.numel(), int(acc), out.data_ptr(), _stream()), "label_gather")
+    _count()
+    return out
+
+
+def tanh_slice_fwd(h: torch.Tensor, out: torch.Tensor, off: int) -> torch.Tensor:
+    """out[:, off:off + C] = tanh(h) for h [M, C] (out [M, ld] contiguous)."""
+    _need_cuda(h, out)
+    M, C = h.shape
+    check(lib.twowl_tanh_slice_fwd(h.contiguous().data_ptr(), M, C, out.data_ptr(), out.shape[1], int(off), _stream()), "tanh_slice_fwd")
+    _count()
+    return out
+
+
+def tanh_slice_bwd(g: torch.Tensor, y: torch.Tensor, off: int, C: int) -> torch.Tensor:
+    """dh [M, C] = g[:, off:off + C] * (1 - y[:, off:off + C]^2) (g, y [M, ld] contiguous, of one shape)."""
+    _need_cuda(g, y)
+    assert g.shape == y.shape
+    M = g.shape[0]
+    dh = torch.empty((M, int(C)), dtype=torch.float32, device=g.device)
+    check(lib.twowl_tanh_slice_bwd(g.contiguous().data_ptr(), y.data_ptr(), g.shape[1], int(off), M, int(C), dh.data_ptr(), _stream()),
+          "tanh_slice_bwd")
+    _count()
+    return dh
+
+
+def sortpool_fwd(X: torch.Tensor, gptr: torch.Tensor, k: int, key_col: int):
+    """SortPooling: per graph the rows of X [n, D] by X[:, key_col] descending, ties by row, the first k -> (out [B, k, D] zero
+    padded, idx int32 [B, k] = the rows taken, -1 for padding)."""
+    _need_cuda(X, gptr)
+    X = X.contiguous()
+    B, D = gptr.numel() - 1, X.shape[1]
+    out = torch.empty((B, int(k), D), dtype=torch.float32, device=X.device)
+    idx = torch.empty((B, int(k)), dtype=torch.int32, device=X.device)
+    check(lib.twowl_sortpool_fwd(X.data_ptr(), D, int(key_col), gptr.data_ptr(), B, int(k), out.data_ptr(), idx.data_ptr(), _stream()),
+          "sortpool_fwd")
+    _count()
+    return out, idx
+
+
+def sortpool_bwd(g: torch.Tensor, idx: torch.Tensor, n_rows: int) -> torch.Tensor:
+    _need_cuda(g, idx)
+    B, k, D = g.shape
+    dX = torch.empty((int(n_rows), D), dtype=torch.float32, device=g.device)
+    check(lib.twowl_sortpool_bwd(g.contiguous().data_ptr(), idx.data_ptr(), B, k, D, int(n_rows), dX.data_ptr(), _stream()), "sortpool_bwd")
+    _count(2)
+    return dX
+
+
+def bias_act_fwd(Y: torch.Tensor, bias: torch.Tensor, B: int, pool: int, relu: bool, p_drop: float = 0.0, seed: int = 0) -> torch.Tensor:
+    """Y [B * Lin, C] -> [B * (Lin // pool), C]: dropout_p(max over `pool` consecutive rows of act(Y + bias)), act = ReLU when relu,
+    ties to the first row (nn.MaxPool1d(2, 2) after ReLU on Conv1d's [B, C, Lin] output, read transposed)."""
+    _need_cuda(Y, bias)
+    Y = Y.contiguous()
+    C = Y.shape[1]
+    Lin = Y.shape[0] // max(int(B), 1)
+    out = torch.empty((int(B) * (Lin // int(pool)), C), dtype=torch.float32, device=Y.device)
+    check(lib.twowl_bias_act_fwd(Y.data_ptr(), bias.contiguous().data_ptr(), int(B), max(Lin, 1), C, int(pool), int(relu), float(p_drop),
+                                 int(seed), out.data_ptr(), _stream()), "bias_act_fwd")
+    _count()
+    return out
+
+
+def bias_act_bwd(g: torch.Tensor, Y: torch.Tensor, bias: torch.Tensor, B: int, pool: int, relu: bool, p_drop: float = 0.0,
+                 seed: int = 0) -> torch.Tensor:
+    _need_cuda(g, Y, bias)
+    C = Y.shape[1]
+    Lin = Y.shape[0] // max(int(B), 1)
+    dY = torch.empty_like(Y)
+    check(lib.twowl_bias_act_bwd(g.contiguous().data_ptr(), Y.data_ptr(), bias.contiguous().data_ptr(), int(B), max(Lin, 1), C, int(pool),
+                                 int(relu), float(p_drop), int(seed), dY.data_ptr(), _stream()), "bias_act_bwd")
+    _count()
+    return dY
+
+
+def im2col_fwd(P: torch.Tensor, B: int, kw: int) -> torch.Tensor:
+    """P [B * L1, C] (row b L1 + t = position t of sample b) -> [B * L2, C * kw], L2 = L1 - kw + 1, column c kw + j = P[b, p + j, c]."""
+    _need_cuda(P)
+    P = P.contiguous()
+    C = P.shape[1]
+    L1 = P.shape[0] // int(B)
+    out = torch.empty((int(B) * (L1 - int(kw) + 1), C * int(kw)), dtype=torch.float32, device=P.device)
+    check(lib.twowl_im2col_fwd(P.data_ptr(), int(B), L1, C, int(kw), out.data_ptr(), _stream()), "im2col_fwd")
+    _count()
+    return out
+
+
+def im2col_bwd(g: torch.Tensor, B: int, L1: int, C: int, kw: int) -> torch.Tensor:
+    _need_cuda(g)
+    dP = torch.empty((int(B) * int(L1), int(C)), dtype=torch.float32, device=g.device)
+    check(lib.twowl_im2col_bwd(g.contiguous().data_ptr(), int(B), int(L1), int(C), int(kw), dP.data_ptr(), _stream()), "im2col_bwd")
+    _count()
+    return dP
