@@ -505,6 +505,29 @@ int twowl_link_heuristics(const int64_t* ptr, const int32_t* adj, int64_t num_no
                           int64_t s_v, int64_t P, const int64_t* chunk_off, int64_t n_chunks, float* out, void* ws, size_t ws_bytes,
                           void* stream);
 
+/* Common-neighbour lists of query pairs (u[i], v[i]) (int64[P] each, element strides) over a simple adjacency (ptr, adj) of
+ * twowl_simple_adjacency, optionally with entries deleted: entry_mask (uint8[nnz], NULL = none) != 0 marks an adjacency entry that is
+ * not an edge. CN(i) = N(u) ∩ N(v) over the unmasked entries (a masked entry of either list never yields a neighbour); u == v gives
+ * N(u). chunk_off / n_chunks come from twowl_link_plan (same decomposition and work split as twowl_link_heuristics). Two calls, with
+ * one host read between them:
+ *   twowl_common_neighbors_count: cn_ptr (int64[P+1]) = exclusive scan of |CN(i)| (0 for a pair with a bad id), chunk_base
+ *                                 (int64[n_chunks+1]) = exclusive scan of the chunk counts (read by the fill).
+ *   twowl_common_neighbors_fill:  cn_ids (int32[nnz_cn], nnz_cn = cn_ptr[P] < 2^31): row i = CN(i) in ascending id order;
+ *                                 cn_pair (int32[nnz_cn]) = the pair of every entry. No atomics: bitwise repeatable.
+ * twowl_adjacency_pair_mask: mask (uint8[nnz], zeroed by the call) = 1 at the entries of v in N(u) and of u in N(v) for every pair
+ * (u, v) that is an edge (u != v); info (int64[1], device) = ids outside [0, num_nodes). Such pairs, non-edges and u == v set
+ * nothing. adj may be NULL when nnz = 0. */
+size_t twowl_common_neighbors_count_workspace_bytes(int64_t P, int64_t n_chunks);
+int twowl_common_neighbors_count(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const uint8_t* entry_mask, const int64_t* u,
+                                 int64_t s_u, const int64_t* v, int64_t s_v, int64_t P, const int64_t* chunk_off, int64_t n_chunks,
+                                 int64_t* cn_ptr, int64_t* chunk_base, void* ws, size_t ws_bytes, void* stream);
+int twowl_common_neighbors_fill(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const uint8_t* entry_mask, const int64_t* u,
+                                int64_t s_u, const int64_t* v, int64_t s_v, int64_t P, const int64_t* chunk_off, int64_t n_chunks,
+                                const int64_t* cn_ptr, const int64_t* chunk_base, int64_t nnz_cn, int32_t* cn_ids, int32_t* cn_pair,
+                                void* stream);
+int twowl_adjacency_pair_mask(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, int64_t nnz, const int64_t* u, int64_t s_u,
+                              const int64_t* v, int64_t s_v, int64_t P, uint8_t* mask, int64_t* info, void* stream);
+
 /* Link recommendation over a simple adjacency (ptr, adj) of twowl_simple_adjacency: for each source s = src[q] (int64[Q], element
  * stride), the top k of its candidates C(s) = {v != s : v not in N(s), N(s) ∩ N(v) non-empty} by one of the four scores above.
  * With c = |N(s) ∩ N(v)|: cn = c; jaccard = c / (d(s) + d(v) - c) as an fp32 quotient; aa and ra add the same terms as

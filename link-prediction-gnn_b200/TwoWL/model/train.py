@@ -220,7 +220,15 @@ def rerank(mod, dataset):
     mod.eval()
     n_edges = dataset.ei.shape[1]
     targets = n_edges + torch.arange(dataset.y.shape[0], device=dataset.x.device)
-    logits = mod(dataset.x, dataset.ei, dataset.pos1, targets, dataset.ei2, True).reshape(-1)
+    return rerank_scores(mod(dataset.x, dataset.ei, dataset.pos1, targets, dataset.ei2, True), dataset)
+
+
+@torch.no_grad()
+def rerank_scores(scores, dataset):
+    """The table-sorting half of rerank() for any score of a candidate table's pairs (one per candidate, in the order of test(),
+    e.g. ncn_scores(mod, dataset)) -> (ids int64 [Q, k], scores fp32 [Q, k]): each row ordered by score descending, ties keeping the
+    heuristic's order, with the padding (-1) last at -inf."""
+    logits = scores.reshape(-1)
     mask = dataset.cand_mask
     table = torch.full(mask.shape, float("-inf"), dtype=logits.dtype, device=logits.device)
     table[mask] = logits
@@ -297,8 +305,8 @@ def _seal_graph(dataset):
     return graph.simple_adjacency(dataset.ei, dataset.x.shape[0])
 
 
-def _seal_train_pairs(dataset):
-    """SEAL's training targets: the undirected pairs of ei (pos1[:E:2], label 1) and the negatives pos1[E::2] (label 0)."""
+def _link_targets(dataset):
+    """The training targets of SEAL and NCN: the undirected pairs of ei (pos1[:E:2], label 1) and the negatives pos1[E::2] (label 0)."""
     n_edges = dataset.ei.shape[1]
     pos, neg = dataset.pos1[:n_edges:2], dataset.pos1[n_edges::2]
     y = torch.cat((torch.ones(pos.shape[0], device=pos.device), torch.zeros(neg.shape[0], device=pos.device)))
@@ -316,7 +324,7 @@ def seal_fit(trn_ds, epochs, batch_size, lr=1e-4, hops=1, max_nodes_per_hop=0, s
     from TwoWL.model.seal import DGCNN, sort_pool_k
     from twowl_b200.optim import FusedAdam
     ptr, adj = _seal_graph(trn_ds)
-    pairs, y = _seal_train_pairs(trn_ds)
+    pairs, y = _link_targets(trn_ds)
     T = pairs.shape[0]
     sub_kw = dict(hops=hops, max_nodes_per_hop=max_nodes_per_hop, seed=seed)
     sizes = ops.seal_subgraph_sizes(ptr, adj, pairs[:, 0], pairs[:, 1], **sub_kw)
@@ -363,4 +371,73 @@ def seal_scores(mod, dataset, hops=1, max_nodes_per_hop=0, seed=0, node_feat=Non
         sub = ops.seal_subgraphs(ptr, adj, pairs[q:q + batch_size, 0], pairs[q:q + batch_size, 1], hops=hops,
                                  max_nodes_per_hop=max_nodes_per_hop, seed=seed, index_base=q)
         out.append(mod(sub, node_feat).reshape(-1))
+    return torch.cat(out) if out else torch.zeros(0, device=pairs.device)
+
+
+def ncn_fit(trn_ds, epochs, batch_size, lr=1e-3, hidden=64, num_layers=2, dropout=0.3, cn=True, node_feat=None, seed=0):
+    """Train NCN (TwoWL.model.ncn; cn=False: the GCN + MLP-decoder baseline) on a training split (extension: the message-passing
+    link predictors of the OGB leaderboards) -> (model, losses float64 [steps]). Targets: every undirected pair of trn_ds.ei
+    (label 1) and the negatives pos1[E::2] (label 0), as seal_fit takes them, in a seeded permutation per epoch. Per batch of
+    batch_size targets, NCN's protocol: the batch's positive edges are removed from the encoder's graph (sample_block, which also
+    gives the degree input) and from the adjacency the common neighbours are read from (ops.adjacency_pair_mask passed to
+    ops.common_neighbors); then the full-graph encoder, the predictor on the batch, BCE-with-logits, backward and a FusedAdam step
+    (lr). Degrees are clipped to the split's maximum. node_feat [N, F] replaces the degree input. The same seed gives the same
+    losses and weights bit for bit."""
+    from TwoWL.model.ncn import NCN
+    from twowl_b200 import graph
+    from twowl_b200.optim import FusedAdam
+    N = trn_ds.x.shape[0]
+    ptr, adj = graph.simple_adjacency(trn_ds.ei, N)
+    pairs, y = _link_targets(trn_ds)
+    T, n_pos = pairs.shape[0], trn_ds.ei.shape[1] // 2
+    max_x = int(trn_ds.x.max()) if N else 0
+    with torch.random.fork_rng(devices=[pairs.device]):
+        torch.manual_seed(seed)
+        mod = NCN(max_x, hidden, num_layers, dropout, cn, 0 if node_feat is None else node_feat.shape[1])
+    mod = mod.to(pairs.device).train()
+    opt = FusedAdam(mod.parameters(), lr=lr)
+    gen = torch.Generator(device="cpu")
+    gen.manual_seed(seed)
+    losses = []
+    step = 0
+    for _ in range(epochs):
+        perm = torch.randperm(T, generator=gen).to(pairs.device)
+        for b in range(0, T, batch_size):
+            ids = perm[b:b + batch_size]
+            bp = pairs[ids]
+            pos = ids[ids < n_pos]                     # target k < n_pos is the undirected edge (ei[:, 2k], ei[:, 2k + 1])
+            ei_new, x_new, _ = sample_block(double(pos, for_index=True), N, trn_ds.ei, None)
+            cn_lists = None
+            if cn:
+                cn_lists = ops.common_neighbors(ptr, adj, bp[:, 0], bp[:, 1],
+                                                ops.adjacency_pair_mask(ptr, adj, pairs[pos, 0], pairs[pos, 1]))
+            opt.zero_grad()
+            logits = mod(x_new, ei_new, bp, cn_lists, node_feat, seed=(seed * 1000003 + step) % (2 ** 62))
+            loss = F2.bce_with_logits(logits, y[ids].unsqueeze(-1))
+            loss.backward()
+            opt.step()
+            losses.append(loss.detach().double().reshape(1))
+            step += 1
+    mod.eval()
+    return mod, (torch.cat(losses).cpu() if losses else torch.zeros(0, dtype=torch.float64))
+
+
+@torch.no_grad()
+def ncn_scores(mod, dataset, node_feat=None, batch_size=65536):
+    """NCN logits of the dataset's prediction pairs pos1[E::2] -> fp32 [P], in the order of test(): one encoder pass over dataset.ei
+    with nothing removed, then the predictor over batches of pairs with their common neighbours in the split's simple graph
+    (graph.simple_adjacency). A pair's logit depends on that pair alone, so the result does not depend on batch_size, bit for bit.
+    rank_scores(ncn_scores(mod, ds), ds), ops.auc(scores, ds.y[0::2]) and rerank_scores rank it like any other score."""
+    from twowl_b200 import graph
+    mod.eval()
+    N = dataset.x.shape[0]
+    ptr, adj = graph.simple_adjacency(dataset.ei, N)
+    n_edges = dataset.ei.shape[1]
+    pairs = dataset.pos1[n_edges::2][: dataset.y.shape[0] // 2].to(torch.long)
+    h = mod.encode(dataset.x, dataset.ei, node_feat)
+    out = []
+    for q in range(0, pairs.shape[0], batch_size):
+        bp = pairs[q:q + batch_size]
+        cn_lists = ops.common_neighbors(ptr, adj, bp[:, 0], bp[:, 1]) if mod.cn else None
+        out.append(mod.predict(h, bp, cn_lists).reshape(-1))
     return torch.cat(out) if out else torch.zeros(0, device=pairs.device)

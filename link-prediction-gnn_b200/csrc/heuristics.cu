@@ -518,6 +518,196 @@ __global__ void __launch_bounds__(kRecThreads) k_rec_out(const uint32_t* __restr
   }
 }
 
+// ---------------------------------------------------------------- common-neighbour lists -------------
+// The same decomposition as link_heuristics (twowl_link_plan's chunk_off): a short pair is probed by one 8-lane group, a long
+// pair's chunks by one warp each. An entry mask (uint8 per adjacency entry, NULL = none) deletes entries: a probe from a masked
+// entry of the shorter list finds nothing, and a hit on a masked entry of the longer list does not count.
+//   count  chunk counts into chunk_base[c], then pair counts (a long pair adds its chunks) into cn_ptr[i]; both scanned.
+//   fill   a round probes one strided position per lane; a group ballot ranks the hits, so they are written in probe order,
+//          which is ascending id order. A long pair's chunk c writes from cn_ptr[i] + chunk_base[c] - chunk_base[chunk_off[i]].
+
+// probes S[j] into L[lo, hi) (lo advances: S is sorted); true when S[j] is a common neighbour that no mask deletes
+__device__ __forceinline__ bool cn_probe(const int32_t* __restrict__ S, const uint8_t* __restrict__ mS, int j, const int32_t* __restrict__ L,
+                                         const uint8_t* __restrict__ mL, int& lo, int hi) {
+  if (mS && __ldg(mS + j)) return false;
+  const int32_t x = __ldg(S + j);
+  lo = lower_bound_i32(L, lo, hi, x);
+  return lo < hi && __ldg(L + lo) == x && !(mL && __ldg(mL + lo));
+}
+
+// the mask pointers of a pair's two lists (NULL without a mask)
+__device__ __forceinline__ void cn_masks(const int32_t* __restrict__ adj, const uint8_t* __restrict__ mask, const PairLists& pl,
+                                         const uint8_t** mS, const uint8_t** mL) {
+  *mS = mask ? mask + (pl.S - adj) : nullptr;
+  *mL = mask ? mask + (pl.L - adj) : nullptr;
+}
+
+struct CnChunk {
+  int64_t pair;
+  PairLists pl;
+  int j0, j1, llo, lhi;
+};
+
+// one warp per chunk c: its pair, probe range and the matching range of the longer list (k_lh_chunks' merge path)
+__device__ __forceinline__ CnChunk cn_chunk(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj, const int64_t* __restrict__ u,
+                                            int64_t s_u, const int64_t* __restrict__ v, int64_t s_v, int64_t P,
+                                            const int64_t* __restrict__ chunk_off, int64_t c) {
+  const int lane = threadIdx.x & 31;
+  CnChunk ch;
+  ch.pair = last_le(chunk_off, P, 0, c);
+  const int64_t k = c - chunk_off[ch.pair];
+  int64_t da, db;
+  ch.pl = pair_lists(ptr, adj, u[ch.pair * s_u], v[ch.pair * s_v], &da, &db);
+  ch.j0 = (int)(k * kHeurChunk);
+  ch.j1 = ch.j0 + kHeurChunk < ch.pl.ds ? ch.j0 + kHeurChunk : ch.pl.ds;
+  int bound = 0;
+  if (lane == 0) bound = lower_bound_i32(ch.pl.L, 0, ch.pl.dl, __ldg(ch.pl.S + ch.j0));
+  if (lane == 1) bound = lower_bound_i32(ch.pl.L, 0, ch.pl.dl, __ldg(ch.pl.S + ch.j1 - 1) + 1);   // ids < 2^31 - 1
+  ch.llo = __shfl_sync(0xffffffffu, bound, 0);
+  ch.lhi = __shfl_sync(0xffffffffu, bound, 1);
+  return ch;
+}
+
+__global__ void __launch_bounds__(kHeurThreads) k_cn_chunk_count(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj,
+                                                                 const uint8_t* __restrict__ mask, const int64_t* __restrict__ u,
+                                                                 int64_t s_u, const int64_t* __restrict__ v, int64_t s_v, int64_t P,
+                                                                 const int64_t* __restrict__ chunk_off, int64_t n_chunks,
+                                                                 int64_t* __restrict__ chunk_cnt) {
+  const int lane = threadIdx.x & 31;
+  for (int64_t c = (int64_t)blockIdx.x * kHeurWarps + (threadIdx.x >> 5); c < n_chunks; c += (int64_t)gridDim.x * kHeurWarps) {
+    const CnChunk ch = cn_chunk(ptr, adj, u, s_u, v, s_v, P, chunk_off, c);
+    const uint8_t *mS, *mL;
+    cn_masks(adj, mask, ch.pl, &mS, &mL);
+    int cnt = 0, lo = ch.llo;
+    for (int j = ch.j0 + lane; j < ch.j1; j += 32) cnt += cn_probe(ch.pl.S, mS, j, ch.pl.L, mL, lo, ch.lhi);
+    cnt = warp_sum_i(cnt);
+    if (lane == 0) chunk_cnt[c] = cnt;
+  }
+}
+
+// one 8-lane group per pair: the count of a short pair, or the sum of a long pair's chunk counts (0 for a bad id)
+__global__ void __launch_bounds__(kHeurThreads) k_cn_pair_count(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj,
+                                                                const uint8_t* __restrict__ mask, int64_t N, const int64_t* __restrict__ u,
+                                                                int64_t s_u, const int64_t* __restrict__ v, int64_t s_v, int64_t P,
+                                                                const int64_t* __restrict__ chunk_off, const int64_t* __restrict__ chunk_cnt,
+                                                                int64_t* __restrict__ cnt_out) {
+  const int g = (threadIdx.x & 31) / kHeurGroup, gl = threadIdx.x & (kHeurGroup - 1);
+  const int64_t stride = (int64_t)gridDim.x * kHeurGroups;
+  // the loop bound is warp-uniform so that every lane reaches the shuffles below
+  for (int64_t base = (int64_t)blockIdx.x * kHeurGroups + (threadIdx.x >> 5) * (32 / kHeurGroup); base < P; base += stride) {
+    const int64_t i = base + g;
+    int64_t cnt = 0;
+    if (i < P) {
+      const int64_t a = u[i * s_u], b = v[i * s_v];
+      if (id_ok(a, N) && id_ok(b, N)) {
+        int64_t da, db;
+        const PairLists pl = pair_lists(ptr, adj, a, b, &da, &db);
+        if (pl.ds > kHeurLong) {
+          if (gl == 0)
+            for (int64_t c = chunk_off[i], e = chunk_off[i + 1]; c < e; ++c) cnt += chunk_cnt[c];
+        } else {
+          const uint8_t *mS, *mL;
+          cn_masks(adj, mask, pl, &mS, &mL);
+          int lo = 0;
+          for (int j = gl; j < pl.ds; j += kHeurGroup) cnt += cn_probe(pl.S, mS, j, pl.L, mL, lo, pl.dl);
+        }
+      }
+    }
+#pragma unroll
+    for (int o = kHeurGroup / 2; o; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    if (i < P && gl == 0) cnt_out[i] = cnt;
+  }
+}
+
+// one warp per chunk of a long pair: its common neighbours from the chunk's base, in ascending order
+__global__ void __launch_bounds__(kHeurThreads) k_cn_chunk_fill(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj,
+                                                                const uint8_t* __restrict__ mask, const int64_t* __restrict__ u,
+                                                                int64_t s_u, const int64_t* __restrict__ v, int64_t s_v, int64_t P,
+                                                                const int64_t* __restrict__ chunk_off, int64_t n_chunks,
+                                                                const int64_t* __restrict__ cn_ptr, const int64_t* __restrict__ chunk_base,
+                                                                int32_t* __restrict__ ids, int32_t* __restrict__ pair) {
+  const int lane = threadIdx.x & 31;
+  const unsigned below = (1u << lane) - 1u;
+  for (int64_t c = (int64_t)blockIdx.x * kHeurWarps + (threadIdx.x >> 5); c < n_chunks; c += (int64_t)gridDim.x * kHeurWarps) {
+    const CnChunk ch = cn_chunk(ptr, adj, u, s_u, v, s_v, P, chunk_off, c);
+    const uint8_t *mS, *mL;
+    cn_masks(adj, mask, ch.pl, &mS, &mL);
+    int64_t out = cn_ptr[ch.pair] + chunk_base[c] - chunk_base[chunk_off[ch.pair]];
+    int lo = ch.llo;
+    for (int j0 = ch.j0; j0 < ch.j1; j0 += 32) {   // warp-uniform rounds
+      const int j = j0 + lane;
+      const bool hit = j < ch.j1 && cn_probe(ch.pl.S, mS, j, ch.pl.L, mL, lo, ch.lhi);
+      const unsigned b = __ballot_sync(0xffffffffu, hit);
+      if (hit) {
+        const int64_t e = out + __popc(b & below);
+        ids[e] = __ldg(ch.pl.S + j);
+        pair[e] = (int32_t)ch.pair;
+      }
+      out += __popc(b);
+    }
+  }
+}
+
+// one 8-lane group per short pair: its common neighbours from cn_ptr[i], in ascending order (long pairs: k_cn_chunk_fill)
+__global__ void __launch_bounds__(kHeurThreads) k_cn_pair_fill(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj,
+                                                               const uint8_t* __restrict__ mask, int64_t N, const int64_t* __restrict__ u,
+                                                               int64_t s_u, const int64_t* __restrict__ v, int64_t s_v, int64_t P,
+                                                               const int64_t* __restrict__ cn_ptr, int32_t* __restrict__ ids,
+                                                               int32_t* __restrict__ pair) {
+  const int lane = threadIdx.x & 31, g = lane / kHeurGroup, gl = lane & (kHeurGroup - 1);
+  const unsigned gmask = 0xffu << (g * kHeurGroup), below = (1u << lane) - 1u;
+  for (int64_t i = ((int64_t)blockIdx.x * kHeurThreads + threadIdx.x) / kHeurGroup; i < P; i += (int64_t)gridDim.x * kHeurGroups) {
+    const int64_t a = u[i * s_u], b = v[i * s_v];
+    if (!id_ok(a, N) || !id_ok(b, N)) continue;                 // uniform over the group, as is every branch below
+    int64_t da, db;
+    const PairLists pl = pair_lists(ptr, adj, a, b, &da, &db);
+    if (pl.ds > kHeurLong) continue;
+    const uint8_t *mS, *mL;
+    cn_masks(adj, mask, pl, &mS, &mL);
+    int64_t out = cn_ptr[i];
+    int lo = 0;
+    for (int j0 = 0; j0 < pl.ds; j0 += kHeurGroup) {            // group-uniform rounds
+      const int j = j0 + gl;
+      const bool hit = j < pl.ds && cn_probe(pl.S, mS, j, pl.L, mL, lo, pl.dl);
+      const unsigned bal = __ballot_sync(gmask, hit) & gmask;
+      if (hit) {
+        const int64_t e = out + __popc(bal & below);
+        ids[e] = __ldg(pl.S + j);
+        pair[e] = (int32_t)i;
+      }
+      out += __popc(bal);
+    }
+  }
+}
+
+// one thread per pair (u, v), u != v, both valid: mask the entry of v in N(u) and the entry of u in N(v), each where it exists
+// (on the symmetric simple adjacency: both, exactly when the pair is an edge); info[0] += bad ids
+__global__ void __launch_bounds__(kHeurThreads) k_adj_pair_mask(const int64_t* __restrict__ ptr, const int32_t* __restrict__ adj, int64_t N,
+                                                                const int64_t* __restrict__ u, int64_t s_u, const int64_t* __restrict__ v,
+                                                                int64_t s_v, int64_t P, uint8_t* __restrict__ mask,
+                                                                unsigned long long* __restrict__ info) {
+  int nbad = 0;
+  const int lane = threadIdx.x & 31;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i - lane < P; i += (int64_t)gridDim.x * blockDim.x) {
+    if (i < P) {
+      const int64_t a = u[i * s_u], b = v[i * s_v];
+      const bool oka = id_ok(a, N), okb = id_ok(b, N);
+      nbad += !oka + !okb;
+      if (oka && okb && a != b) {
+        const int64_t pa = ptr[a], pb = ptr[b];
+        const int da = (int)(ptr[a + 1] - pa), db = (int)(ptr[b + 1] - pb);
+        // each direction is looked up and checked on its own, so that a CSR that is not symmetric marks only entries it holds
+        const int ia = lower_bound_i32(adj + pa, 0, da, (int32_t)b);
+        if (ia < da && __ldg(adj + pa + ia) == (int32_t)b) mask[pa + ia] = 1;
+        const int ib = lower_bound_i32(adj + pb, 0, db, (int32_t)a);
+        if (ib < db && __ldg(adj + pb + ib) == (int32_t)a) mask[pb + ib] = 1;
+      }
+    }
+  }
+  nbad = warp_sum_i(nbad);
+  if (lane == 0 && nbad) atomicAdd(info, (unsigned long long)nbad);
+}
+
 }  // namespace twowl
 
 using namespace twowl;
@@ -701,5 +891,75 @@ extern "C" int twowl_recommend(const int64_t* ptr, const int32_t* adj, int64_t n
   }
   k_rec_out<<<grid_for(Qb * k, kRecThreads), kRecThreads, 0, s>>>(W, F, M, D, V, SC, Qb, k, q_begin, Q * k, ids, scores);
   TW_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" size_t twowl_common_neighbors_count_workspace_bytes(int64_t P, int64_t n_chunks) {
+  return align_up(scan_workspace_bytes(P > 0 ? P : 1)) + align_up(scan_workspace_bytes(n_chunks > 0 ? n_chunks : 1));
+}
+
+extern "C" int twowl_common_neighbors_count(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const uint8_t* entry_mask,
+                                            const int64_t* u, int64_t s_u, const int64_t* v, int64_t s_v, int64_t P,
+                                            const int64_t* chunk_off, int64_t n_chunks, int64_t* cn_ptr, int64_t* chunk_base, void* ws,
+                                            size_t ws_bytes, void* stream) {
+  TW_CHECK_ARG(P >= 0 && P < 0x7fffffffLL && num_nodes >= 0 && num_nodes < 0x7fffffffLL && n_chunks >= 0,
+               "common_neighbors_count: bad sizes (0 <= P < 2^31, 0 <= num_nodes < 2^31 - 1, n_chunks >= 0)");
+  TW_CHECK_ARG(ptr && cn_ptr && chunk_base && (P == 0 || (u && v && chunk_off)), "common_neighbors_count: null pointer");
+  TW_CHECK_WS(ws_bytes, twowl_common_neighbors_count_workspace_bytes(P, n_chunks));
+  cudaStream_t s = (cudaStream_t)stream;
+  Carver c(ws);
+  void* pws = c.take<char>(scan_workspace_bytes(P > 0 ? P : 1));
+  void* cws = c.take<char>(scan_workspace_bytes(n_chunks > 0 ? n_chunks : 1));
+  if (n_chunks > 0) {
+    k_cn_chunk_count<<<grid_for(n_chunks, kHeurWarps), kHeurThreads, 0, s>>>(ptr, adj, entry_mask, u, s_u, v, s_v, P, chunk_off, n_chunks,
+                                                                             chunk_base);
+    TW_LAUNCH_CHECK();
+  }
+  if (P > 0) {
+    k_cn_pair_count<<<grid_for(P, kHeurGroups), kHeurThreads, 0, s>>>(ptr, adj, entry_mask, num_nodes, u, s_u, v, s_v, P, chunk_off,
+                                                                       chunk_base, cn_ptr);
+    TW_LAUNCH_CHECK();
+  }
+  if (int rc = scan_exclusive_i64(cn_ptr, cn_ptr, P, pws, s)) return rc;
+  if (int rc = scan_exclusive_i64(chunk_base, chunk_base, n_chunks, cws, s)) return rc;
+  return 0;
+}
+
+extern "C" int twowl_common_neighbors_fill(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, const uint8_t* entry_mask,
+                                           const int64_t* u, int64_t s_u, const int64_t* v, int64_t s_v, int64_t P, const int64_t* chunk_off,
+                                           int64_t n_chunks, const int64_t* cn_ptr, const int64_t* chunk_base, int64_t nnz_cn,
+                                           int32_t* cn_ids, int32_t* cn_pair, void* stream) {
+  TW_CHECK_ARG(P >= 0 && P < 0x7fffffffLL && num_nodes >= 0 && num_nodes < 0x7fffffffLL && n_chunks >= 0 && nnz_cn >= 0 &&
+                   nnz_cn < 0x80000000LL,
+               "common_neighbors_fill: bad sizes (0 <= P < 2^31, 0 <= num_nodes < 2^31 - 1, n_chunks >= 0, 0 <= nnz_cn < 2^31)");
+  TW_CHECK_ARG(ptr && cn_ptr && chunk_base && (P == 0 || (u && v && chunk_off)) && (nnz_cn == 0 || (adj && cn_ids && cn_pair)),
+               "common_neighbors_fill: null pointer");
+  if (nnz_cn == 0) return 0;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (n_chunks > 0) {
+    k_cn_chunk_fill<<<grid_for(n_chunks, kHeurWarps), kHeurThreads, 0, s>>>(ptr, adj, entry_mask, u, s_u, v, s_v, P, chunk_off, n_chunks,
+                                                                            cn_ptr, chunk_base, cn_ids, cn_pair);
+    TW_LAUNCH_CHECK();
+  }
+  k_cn_pair_fill<<<grid_for(P, kHeurGroups), kHeurThreads, 0, s>>>(ptr, adj, entry_mask, num_nodes, u, s_u, v, s_v, P, cn_ptr, cn_ids,
+                                                                    cn_pair);
+  TW_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int twowl_adjacency_pair_mask(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, int64_t nnz, const int64_t* u,
+                                         int64_t s_u, const int64_t* v, int64_t s_v, int64_t P, uint8_t* mask, int64_t* info,
+                                         void* stream) {
+  TW_CHECK_ARG(P >= 0 && P < 0x7fffffffLL && num_nodes >= 0 && num_nodes < 0x7fffffffLL && nnz >= 0,
+               "adjacency_pair_mask: bad sizes (0 <= P < 2^31, 0 <= num_nodes < 2^31 - 1, nnz >= 0)");
+  TW_CHECK_ARG(ptr && info && (P == 0 || (u && v)) && (nnz == 0 || (adj && mask)), "adjacency_pair_mask: null pointer");
+  cudaStream_t s = (cudaStream_t)stream;
+  TW_CUDA(cudaMemsetAsync(info, 0, sizeof(int64_t), s));
+  if (nnz > 0) TW_CUDA(cudaMemsetAsync(mask, 0, (size_t)nnz, s));
+  if (P > 0) {
+    k_adj_pair_mask<<<grid_for(P, kHeurThreads), kHeurThreads, 0, s>>>(ptr, adj, num_nodes, u, s_u, v, s_v, P, mask,
+                                                                       reinterpret_cast<unsigned long long*>(info));
+    TW_LAUNCH_CHECK();
+  }
   return 0;
 }

@@ -289,6 +289,54 @@ def _pi_bwd(ctx, g):
 
 pair_init.register_autograd(_pi_bwd, setup_context=_pi_setup)
 
+
+def batch_pair_init(x: Tensor, pairs: Tensor) -> Tensor:
+    """pair_init for a batch of query pairs (int64 [B, 2]): x[pairs[:, 0]] * x[pairs[:, 1]]. The by-source / by-destination CSRs the
+    backward reads are built here for this batch, not cached: they live as long as the batch."""
+    N, B = x.shape[0], pairs.shape[0]
+    ptr_s, ids_s = ops.csr_build(pairs[:, 0], N)
+    ptr_d, ids_d = ops.csr_build(pairs[:, 1], N)
+    return pair_init(x, ops.narrow_i32(pairs[:, 0]), ops.narrow_i32(pairs[:, 1]), ptr_s, ids_s, ops.seg_plan(ptr_s, N, B), ptr_d, ids_d,
+                     ops.seg_plan(ptr_d, N, B), False)
+
+# ------------------------------------------------------------------------------ common-neighbour sum (TwoWL/model/ncn.py)
+
+
+@torch.library.custom_op("twowl::cn_aggregate", mutates_args=())
+def _cn_aggregate(h: Tensor, cn_ptr: Tensor, cn_ids: Tensor, cn_pair: Tensor, plan: Tensor) -> Tensor:
+    return ops.seg_reduce(cn_ptr, cn_ids, cn_ptr.numel() - 1, h.contiguous(), plan=plan)
+
+
+@_cn_aggregate.register_fake
+def _(h, cn_ptr, cn_ids, cn_pair, plan):
+    return h.new_empty((cn_ptr.shape[0] - 1, h.shape[1]))
+
+
+def _cna_setup(ctx, inputs, output):
+    h, cn_ptr, cn_ids, cn_pair, plan = inputs
+    ctx.save_for_backward(cn_ids, cn_pair)
+    ctx.N = h.shape[0]
+
+
+def _cna_bwd(ctx, g):
+    cn_ids, cn_pair = ctx.saved_tensors
+    N = ctx.N
+    # dh[w] = sum of g[p] over the pairs p whose list holds w: the entries grouped by node with a stable sort, so that each node's
+    # pairs come in ascending order, then one segmented sum
+    tptr, tids = ops.csr_build(cn_ids.to(torch.int64), N)
+    tcol = ops.gather_cols(tids, cn_pair.to(torch.int64))
+    return ops.seg_reduce(tptr, tcol, N, g.contiguous(), plan=ops.seg_plan(tptr, N, tcol.numel())), None, None, None, None
+
+
+_cn_aggregate.register_autograd(_cna_bwd, setup_context=_cna_setup)
+
+
+def cn_aggregate(h: Tensor, cn) -> Tensor:
+    """out [P, C] with out[p] = sum of h[w] over w in CN(p), for cn an ops.CommonNeighbors of P pairs and h [N, C] (C % 4 == 0).
+    Forward and backward are segmented sums in a fixed order (no float atomics): bitwise repeatable."""
+    P = cn.num_pairs
+    return _cn_aggregate(h, cn.ptr, cn.ids, cn.pair, ops.seg_plan(cn.ptr, P, cn.ids.numel()))
+
 # ------------------------------------------------------------------------------ readout
 
 

@@ -1126,6 +1126,98 @@ def link_heuristics(ptr: torch.Tensor, adj: torch.Tensor, u: torch.Tensor, v: to
     return out
 
 
+def _scan_launches(n: int) -> int:
+    """Launches of one scan_exclusive_i64 over n values: three kernels, or one memset when n is 0."""
+    return 3 if n > 0 else 1
+
+
+class CommonNeighbors:
+    """The common neighbours of a batch of query pairs (common_neighbors), as a CSR by pair: ptr int64 [P+1], ids int32 [nnz] (row p =
+    CN(p) in ascending id order) and pair int32 [nnz] (each entry's pair, nondecreasing: what a backward by node needs)."""
+    __slots__ = ("ptr", "ids", "pair")
+
+    def __init__(self, ptr, ids, pair):
+        self.ptr, self.ids, self.pair = ptr, ids, pair
+
+    @property
+    def num_pairs(self) -> int:
+        return self.ptr.numel() - 1
+
+
+def _check_adjacency(fn: str, ptr, adj):
+    assert ptr.dim() == 1 and ptr.dtype == torch.int64 and ptr.is_contiguous(), f"{fn}: ptr must be contiguous int64 [N+1]"
+    assert adj.dim() == 1 and adj.dtype == torch.int32 and adj.is_contiguous(), f"{fn}: adj must be contiguous int32"
+
+
+def adjacency_pair_mask(ptr: torch.Tensor, adj: torch.Tensor, u: torch.Tensor, v: torch.Tensor) -> torch.Tensor:
+    """uint8 [nnz] over a simple adjacency (simple_adjacency): 1 at the entries of v in N(u) and of u in N(v) for every pair (u[i],
+    v[i]) that is an edge - the mask that deletes those edges for common_neighbors. Non-edges and u == v set nothing. One host
+    read; raises IndexError when an id lies outside [0, N)."""
+    _need_cuda(ptr, adj, u, v)
+    _check_adjacency("adjacency_pair_mask", ptr, adj)
+    u, v = u.reshape(-1).to(torch.int64), v.reshape(-1).to(torch.int64)
+    assert u.numel() == v.numel(), "adjacency_pair_mask: u / v size mismatch"
+    dev, n, P = ptr.device, ptr.numel() - 1, u.numel()
+    (pu, su), (pv, sv) = (_row(u), _row(v)) if P else ((0, 1), (0, 1))
+    mask = torch.empty(adj.numel(), dtype=torch.uint8, device=dev)
+    info = torch.empty(1, dtype=torch.int64, device=dev)
+    check(lib.twowl_adjacency_pair_mask(ptr.data_ptr(), adj.data_ptr(), n, adj.numel(), pu, su, pv, sv, P, mask.data_ptr(),
+                                        info.data_ptr(), _stream()), "adjacency_pair_mask")
+    _count(1 + int(adj.numel() > 0) + int(P > 0))
+    nbad = int(info.item())
+    if nbad:
+        raise IndexError(f"adjacency_pair_mask: {nbad} id(s) outside [0, {n})")
+    return mask
+
+
+def common_neighbors(ptr: torch.Tensor, adj: torch.Tensor, u: torch.Tensor, v: torch.Tensor,
+                     entry_mask: Optional[torch.Tensor] = None) -> CommonNeighbors:
+    """The common neighbours CN(i) = N(u[i]) ∩ N(v[i]) of each query pair over a simple adjacency (simple_adjacency) ->
+    CommonNeighbors. entry_mask (uint8 [nnz], e.g. adjacency_pair_mask) deletes the adjacency entries it marks. u == v gives N(u).
+    The pairs are cut as link_heuristics cuts them, |CN(i)| equals its cn row, and the lists are bitwise repeatable. Two host
+    reads (the plan, the total); raises IndexError when an id lies outside [0, N) and ValueError when the lists would hold
+    2^31 or more entries (split the query list)."""
+    fn = "common_neighbors"
+    _need_cuda(ptr, adj, u, v, entry_mask)
+    _check_adjacency(fn, ptr, adj)
+    if entry_mask is not None:
+        assert entry_mask.dtype == torch.uint8 and entry_mask.is_contiguous() and entry_mask.numel() == adj.numel(), \
+            f"{fn}: entry_mask must be contiguous uint8 [nnz]"
+    u, v = u.reshape(-1).to(torch.int64), v.reshape(-1).to(torch.int64)
+    assert u.numel() == v.numel(), f"{fn}: u / v size mismatch"
+    dev, n, P = ptr.device, ptr.numel() - 1, u.numel()
+    (pu, su), (pv, sv) = (_row(u), _row(v)) if P else ((0, 1), (0, 1))
+    chunk_off = torch.empty(P + 1, dtype=torch.int64, device=dev)
+    info = torch.empty(3, dtype=torch.int64, device=dev)
+    nb = lib.twowl_link_plan_workspace_bytes(P)
+    ws = _ws(nb, dev)
+    check(lib.twowl_link_plan(ptr.data_ptr(), n, pu, su, pv, sv, P, chunk_off.data_ptr(), info.data_ptr(), ws.data_ptr(), nb,
+                              _stream()), "link_plan")
+    _count(1 + int(P > 0) + _scan_launches(P))
+    nbad, n_chunks, _ = info.tolist()
+    if nbad:
+        raise IndexError(f"{fn}: {nbad} query id(s) outside [0, {n})")
+    cn_ptr = torch.empty(P + 1, dtype=torch.int64, device=dev)
+    chunk_base = torch.empty(n_chunks + 1, dtype=torch.int64, device=dev)
+    nb = lib.twowl_common_neighbors_count_workspace_bytes(P, n_chunks)
+    ws = _ws(nb, dev)
+    mp = _p(entry_mask)
+    check(lib.twowl_common_neighbors_count(ptr.data_ptr(), adj.data_ptr(), n, mp, pu, su, pv, sv, P, chunk_off.data_ptr(), n_chunks,
+                                           cn_ptr.data_ptr(), chunk_base.data_ptr(), ws.data_ptr(), nb, _stream()),
+          "common_neighbors_count")
+    _count(int(n_chunks > 0) + int(P > 0) + _scan_launches(P) + _scan_launches(n_chunks))
+    total = int(cn_ptr[P].item())
+    if total >= 2 ** 31:
+        raise ValueError(f"{fn}: the lists would hold {total} >= 2^31 entries; pass fewer pairs per call")
+    ids = torch.empty(total, dtype=torch.int32, device=dev)
+    pair = torch.empty(total, dtype=torch.int32, device=dev)
+    check(lib.twowl_common_neighbors_fill(ptr.data_ptr(), adj.data_ptr(), n, mp, pu, su, pv, sv, P, chunk_off.data_ptr(), n_chunks,
+                                          cn_ptr.data_ptr(), chunk_base.data_ptr(), total, _p(ids) if total else None,
+                                          _p(pair) if total else None, _stream()), "common_neighbors_fill")
+    _count((int(n_chunks > 0) + 1) if total else 0)
+    return CommonNeighbors(cn_ptr, ids, pair)
+
+
 RECOMMEND_MAX_ENTRIES = 1 << 26   # default expansion budget of one batch: 44 B of workspace per entry, about 3 GB
 
 
