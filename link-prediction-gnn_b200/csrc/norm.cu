@@ -589,12 +589,15 @@ __global__ void __launch_bounds__(kNormThreads) k_gn2_readout_bwd_rows(const flo
 
 // per-row chains of the positions that select it: head[row] -> position -> next[position] -> ... -> -1.
 // The chain ORDER is a race outcome and never reaches a result: consumers add a row's positions in ascending order.
+// A position joins a chain only if its link is live, i.e. its partner id is not negative either: k_gn2_readout_bwd_rows writes
+// no G row for a masked link, so a chain through one would add uninitialised workspace to the row's gradient.
 __global__ void __launch_bounds__(kNormThreads) k_row_chains(const int64_t* __restrict__ idx, int64_t sidx, int64_t n, int64_t M,
                                                              int32_t* __restrict__ head, int32_t* __restrict__ next) {
   for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
     const int64_t r = idx[j * sidx];
     if (r == kMaskedTail) break;   // packed list: no later position selects a row, and next[] is only read along the chains
-    next[j] = (r >= 0 && r < M) ? atomicExch(&head[r], (int32_t)j) : -1;
+    const bool live = r >= 0 && r < M && idx[(j ^ 1) * sidx] >= 0;
+    next[j] = live ? atomicExch(&head[r], (int32_t)j) : -1;
   }
 }
 
