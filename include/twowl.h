@@ -528,6 +528,38 @@ int twowl_common_neighbors_fill(const int64_t* ptr, const int32_t* adj, int64_t 
 int twowl_adjacency_pair_mask(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, int64_t nnz, const int64_t* u, int64_t s_u,
                               const int64_t* v, int64_t s_v, int64_t P, uint8_t* mask, int64_t* info, void* stream);
 
+/* Subgraph sketches of BUDDY (Chamberlain et al., ICLR 2023; csrc/sketch.cu). Each node holds a MinHash row (uint32[num_perm],
+ * num_perm a multiple of 32 in [32, 1024]) and a HyperLogLog row (uint8[m], m = 2^hll_p, hll_p in [4, 10]) of a node set; the rows
+ * of hop d describe N_{<=d}(u), the nodes within d hops. Rows are 16-byte aligned (mh, hll: 16-byte aligned base pointers).
+ *   twowl_sketch_init: the sets {u}. With seed_mh = 2 seed and seed_hll = 2 seed + 1 (mod 2^64) and common.cuh's hash_u32:
+ *     mh[u][j] = hash_u32(seed_mh, (j << 32) | u);
+ *     h = hash_u32(seed_hll, u), w = h >> hll_p: hll[u][h & (m - 1)] = w ? clz32(w) - hll_p + 1 : 33 - hll_p, every other register 0.
+ *   twowl_sketch_hop: one propagation step, mh_out[u] = min(mh_in[u], mh_in[w] for w in adj(u)) elementwise and hll_out[u] = max(...)
+ *     bytewise, over the entries entry_mask (uint8[nnz], NULL = none) does not mark. A row longer than `chunk` entries (chunk in
+ *     [1, 2^30]) is cut into chunks of `chunk` entries whose partial results a second pass combines; min and max are exact, so the
+ *     bits do not depend on chunk. in and out must not overlap. ws: twowl_sketch_hop_workspace_bytes (the plan + chunk partials).
+ *   twowl_sketch_pair_features: with the sketches of hops 0..hops (hops in [1, 3]) stacked as mh [hops+1, N, num_perm] and
+ *     hll [hops+1, N, m], out (fp32 [P, hops^2 + 2 hops]) for each pair (u[i], v[i]) = [A(1,1), A(1,2), .., A(k,k), B_u(1..k),
+ *     B_v(1..k)], k = hops:
+ *       est(M)   HyperLogLog estimate of a register row: Z = sum_j 2^-M[j] (double, exact), V = #zero registers, E = alpha_m m^2 / Z
+ *                (alpha_16 = 0.673, alpha_32 = 0.697, alpha_64 = 0.709, else 0.7213 / (1 + 1.079 / m)); m ln(m / V) when V > 0 and
+ *                that is at most 10, 20, 40, 80, 220, 400, 900 for hll_p = 4 .. 10, else E
+ *       I(a,b)   = J(a,b) U(a,b), J = fraction of equal entries of mh[a][u] and mh[b][v], U = est(bytewise max of hll[a][u], hll[b][v]);
+ *                I(0,.) = I(.,0) = 0
+ *       A(a,b)   = (I(a,b) + I(a-1,b-1)) - (I(a-1,b) + I(a,b-1)), summed in this order so that (v, u) gives A transposed
+ *       B_u(a)   = est(hll[a][u]) - est(hll[a-1][u]) - sum_b A(a,b);  B_v(b) = est(hll[b][v]) - est(hll[b-1][v]) - sum_a A(a,b)
+ *     in double, each clamped at 0 and rounded once to fp32. A pair with an id outside [0, num_nodes) gets zeros and is counted in
+ *     info[0] (int64, device). */
+#define TWOWL_SKETCH_MAX_HOPS 3
+int twowl_sketch_init(int64_t num_nodes, int32_t num_perm, int32_t hll_p, uint64_t seed, int32_t* minhash, uint8_t* hll, void* stream);
+size_t twowl_sketch_hop_workspace_bytes(int64_t nnz, int32_t num_perm, int32_t hll_p, int64_t chunk);
+int twowl_sketch_hop(const int64_t* ptr, const int32_t* adj, int64_t num_nodes, int64_t nnz, const uint8_t* entry_mask, int32_t num_perm,
+                     int32_t hll_p, int64_t chunk, const int32_t* mh_in, const uint8_t* hll_in, int32_t* mh_out, uint8_t* hll_out, void* ws,
+                     size_t ws_bytes, void* stream);
+int twowl_sketch_pair_features(int32_t hops, int64_t num_nodes, int32_t num_perm, int32_t hll_p, const int32_t* minhash, const uint8_t* hll,
+                               const int64_t* u, int64_t s_u, const int64_t* v, int64_t s_v, int64_t P, float* out, int64_t* info,
+                               void* stream);
+
 /* Link recommendation over a simple adjacency (ptr, adj) of twowl_simple_adjacency: for each source s = src[q] (int64[Q], element
  * stride), the top k of its candidates C(s) = {v != s : v not in N(s), N(s) ∩ N(v) non-empty} by one of the four scores above.
  * With c = |N(s) ∩ N(v)|: cn = c; jaccard = c / (d(s) + d(v) - c) as an fp32 quotient; aa and ra add the same terms as

@@ -441,3 +441,83 @@ def ncn_scores(mod, dataset, node_feat=None, batch_size=65536):
         cn_lists = ops.common_neighbors(ptr, adj, bp[:, 0], bp[:, 1]) if mod.cn else None
         out.append(mod.predict(h, bp, cn_lists).reshape(-1))
     return torch.cat(out) if out else torch.zeros(0, device=pairs.device)
+
+
+def _buddy_batch_features(ptr, adj, pairs, ids, n_pos, hops, sketch_args):
+    """buddy_fit's structure features of the targets pairs[ids] -> (fp32 [B, hops² + 2 hops], the positive target ids): the
+    split's simple adjacency (ptr, adj) is sketched with the batch's positive edges masked out, then the pairs are read."""
+    pos = ids[ids < n_pos]                             # target k < n_pos is the undirected edge (ei[:, 2k], ei[:, 2k + 1])
+    mask = ops.adjacency_pair_mask(ptr, adj, pairs[pos, 0], pairs[pos, 1])
+    sk = ops.link_sketches(ptr, adj, hops, entry_mask=mask, **sketch_args)
+    return ops.sketch_features(sk, pairs[ids, 0], pairs[ids, 1]), pos
+
+
+def buddy_fit(trn_ds, epochs, batch_size, lr=1e-3, hops=2, num_perm=128, hll_p=8, dropout=0.5, hidden=32, node_feat=None, seed=0):
+    """Train BUDDY (TwoWL.model.buddy; extension: the subgraph-sketching link predictors of the OGB leaderboards) on a training
+    split -> (model, losses float64 [steps]). Targets and their order are ncn_fit's: every undirected pair of trn_ds.ei (label 1)
+    and the negatives pos1[E::2] (label 0), in a seeded permutation per epoch. Per batch of batch_size targets, NCN's protocol: the
+    batch's positive edges are deleted before its features are made, so no target link is seen. The split's simple adjacency is
+    sketched with those edges masked out (ops.adjacency_pair_mask, ops.link_sketches with hops / num_perm / hll_p, sketch seed
+    `seed`) and the batch's ops.sketch_features read from it; with node_feat [N, F] the propagation runs over sample_block's graph.
+    Then forward, BCE-with-logits, backward and a FusedAdam step (lr). A trailing batch of one target is skipped (training-mode
+    BatchNorm needs two). The same seed gives the same losses and weights bit for bit."""
+    from TwoWL.model.buddy import BUDDY
+    from twowl_b200 import graph
+    from twowl_b200.optim import FusedAdam
+    N = trn_ds.x.shape[0]
+    ptr, adj = graph.simple_adjacency(trn_ds.ei, N)
+    pairs, y = _link_targets(trn_ds)
+    T, n_pos = pairs.shape[0], trn_ds.ei.shape[1] // 2
+    with torch.random.fork_rng(devices=[pairs.device]):
+        torch.manual_seed(seed)
+        mod = BUDDY(hops, dropout, 0 if node_feat is None else node_feat.shape[1], hidden)
+    mod.sketch_args = dict(num_perm=num_perm, hll_p=hll_p, seed=seed)
+    mod = mod.to(pairs.device).train()
+    opt = FusedAdam(mod.parameters(), lr=lr)
+    gen = torch.Generator(device="cpu")
+    gen.manual_seed(seed)
+    losses = []
+    step = 0
+    for _ in range(epochs):
+        perm = torch.randperm(T, generator=gen).to(pairs.device)
+        for b in range(0, T, batch_size):
+            ids = perm[b:b + batch_size]
+            if ids.numel() < 2:
+                continue
+            bp = pairs[ids]
+            sf, pos = _buddy_batch_features(ptr, adj, pairs, ids, n_pos, hops, mod.sketch_args)
+            xs = None
+            if node_feat is not None:
+                ei_new, _, _ = sample_block(double(pos, for_index=True), N, trn_ds.ei, None)
+                xs = mod.propagate(node_feat, ei_new)
+            opt.zero_grad()
+            logits = mod(sf, bp, xs, seed=(seed * 1000003 + step) % (2 ** 62))
+            loss = F2.bce_with_logits(logits, y[ids].unsqueeze(-1))
+            loss.backward()
+            opt.step()
+            losses.append(loss.detach().double().reshape(1))
+            step += 1
+    mod.eval()
+    return mod, (torch.cat(losses).cpu() if losses else torch.zeros(0, dtype=torch.float64))
+
+
+@torch.no_grad()
+def buddy_scores(mod, dataset, node_feat=None, batch_size=65536):
+    """BUDDY logits of the dataset's prediction pairs pos1[E::2] -> fp32 [P], in the order of test(): the split's simple graph is
+    sketched once with nothing removed (the num_perm / hll_p / seed buddy_fit trained with), the propagation of node_feat runs over
+    dataset.ei, and the model scores batches of pairs in eval mode. A pair's logit depends on that pair alone, so the result does
+    not depend on batch_size, bit for bit. rank_scores(buddy_scores(mod, ds), ds), ops.auc(scores, ds.y[0::2]) and rerank_scores
+    rank it like any other score."""
+    from twowl_b200 import graph
+    mod.eval()
+    N = dataset.x.shape[0]
+    ptr, adj = graph.simple_adjacency(dataset.ei, N)
+    n_edges = dataset.ei.shape[1]
+    pairs = dataset.pos1[n_edges::2][: dataset.y.shape[0] // 2].to(torch.long)
+    sk = ops.link_sketches(ptr, adj, mod.hops, **mod.sketch_args)
+    xs = mod.propagate(node_feat, dataset.ei) if node_feat is not None else None
+    out = []
+    for q in range(0, pairs.shape[0], batch_size):
+        bp = pairs[q:q + batch_size]
+        out.append(mod(ops.sketch_features(sk, bp[:, 0], bp[:, 1]), bp, xs).reshape(-1))
+    return torch.cat(out) if out else torch.zeros(0, device=pairs.device)

@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "twowl_b200")
 LIB = os.path.join(OUT_DIR, "libtwowl_b200.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["prims.cu", "index_ops.cu", "agg.cu", "norm.cu", "pair_ops.cu", "linear.cu", "pair_conv.cu", "dw_tc.cu", "metrics.cu", "sampler.cu", "nodefeat.cu", "train_ops.cu", "heuristics.cu", "walks.cu", "node2vec.cu", "seal.cu"]
+SOURCES = ["prims.cu", "index_ops.cu", "agg.cu", "norm.cu", "pair_ops.cu", "linear.cu", "pair_conv.cu", "dw_tc.cu", "metrics.cu", "sampler.cu", "nodefeat.cu", "train_ops.cu", "heuristics.cu", "walks.cu", "node2vec.cu", "seal.cu", "sketch.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC"] + os.environ.get("TWOWL_NVCC_DEFS", "").split()   # e.g. -DTWOWL_DW_FLUSH=2 (tuning builds)
 

@@ -1218,6 +1218,92 @@ def common_neighbors(ptr: torch.Tensor, adj: torch.Tensor, u: torch.Tensor, v: t
     return CommonNeighbors(cn_ptr, ids, pair)
 
 
+SKETCH_MAX_HOPS = 3      # TWOWL_SKETCH_MAX_HOPS of include/twowl.h
+SKETCH_CHUNK = 64        # rows of the adjacency longer than this are cut into chunks of this many entries (any value gives the same bits)
+
+
+class LinkSketches:
+    """BUDDY's per-node sketches of the d-hop neighbourhoods N_{<=d}(x), d = 0 .. hops (link_sketches): minhash int32 [hops+1, N,
+    num_perm] (uint32 bits) and hll uint8 [hops+1, N, 2^hll_p], with the parameters they were built with."""
+    __slots__ = ("minhash", "hll", "hops", "num_perm", "hll_p", "seed")
+
+    def __init__(self, minhash, hll, hops, num_perm, hll_p, seed):
+        self.minhash, self.hll, self.hops, self.num_perm, self.hll_p, self.seed = minhash, hll, hops, num_perm, hll_p, seed
+
+    @property
+    def num_nodes(self) -> int:
+        return self.minhash.shape[1]
+
+    @property
+    def num_features(self) -> int:
+        return self.hops * self.hops + 2 * self.hops
+
+
+def _sketch_params(fn: str, hops: int, num_perm: int, hll_p: int):
+    if not 1 <= int(hops) <= SKETCH_MAX_HOPS:
+        raise ValueError(f"{fn}: hops = {hops} outside [1, {SKETCH_MAX_HOPS}]")
+    if not (32 <= int(num_perm) <= 1024 and int(num_perm) % 32 == 0):
+        raise ValueError(f"{fn}: num_perm = {num_perm} must be a multiple of 32 in [32, 1024]")
+    if not 4 <= int(hll_p) <= 10:
+        raise ValueError(f"{fn}: hll_p = {hll_p} outside [4, 10]")
+
+
+def link_sketches(ptr: torch.Tensor, adj: torch.Tensor, hops: int = 2, num_perm: int = 128, hll_p: int = 8, seed: int = 0,
+                  entry_mask: Optional[torch.Tensor] = None, chunk: int = SKETCH_CHUNK) -> LinkSketches:
+    """BUDDY's MinHash and HyperLogLog sketches of every node's d-hop neighbourhood, d = 0 .. hops, over a simple adjacency
+    (simple_adjacency) -> LinkSketches. Hop 0 sketches {x} (twowl_sketch_init defines the hashes from seed); hop d is the elementwise
+    min (MinHash) and bytewise max (HyperLogLog) of x's hop d-1 row and those of its neighbours. entry_mask (uint8 [nnz], e.g.
+    adjacency_pair_mask) deletes the adjacency entries it marks. chunk only sets how a long row is cut: the bits never depend on it.
+    No host read."""
+    fn = "link_sketches"
+    _need_cuda(ptr, adj, entry_mask)
+    _check_adjacency(fn, ptr, adj)
+    _sketch_params(fn, hops, num_perm, hll_p)
+    if not 1 <= int(chunk) <= 1 << 30:
+        raise ValueError(f"{fn}: chunk = {chunk} outside [1, 2^30]")
+    if entry_mask is not None:
+        assert entry_mask.dtype == torch.uint8 and entry_mask.is_contiguous() and entry_mask.numel() == adj.numel(), \
+            f"{fn}: entry_mask must be contiguous uint8 [nnz]"
+    hops, num_perm, hll_p, seed = int(hops), int(num_perm), int(hll_p), int(seed) % (2 ** 64)
+    dev, n, nnz, m = ptr.device, ptr.numel() - 1, adj.numel(), 1 << int(hll_p)
+    mh = torch.empty((hops + 1, n, num_perm), dtype=torch.int32, device=dev)
+    hll = torch.empty((hops + 1, n, m), dtype=torch.uint8, device=dev)
+    check(lib.twowl_sketch_init(n, num_perm, hll_p, seed, mh.data_ptr(), hll.data_ptr(), _stream()), "sketch_init")
+    _count(int(n > 0))
+    nb = lib.twowl_sketch_hop_workspace_bytes(nnz, num_perm, hll_p, int(chunk))
+    ws = _ws(nb, dev)
+    for d in range(1, hops + 1):
+        with _P("sketch_hop", (nnz + n) * (4 * num_perm + m) + n * (4 * num_perm + m)):
+            check(lib.twowl_sketch_hop(ptr.data_ptr(), _p(adj) if nnz else None, n, nnz, _p(entry_mask), num_perm, hll_p, int(chunk),
+                                       mh[d - 1].data_ptr(), hll[d - 1].data_ptr(), mh[d].data_ptr(), hll[d].data_ptr(),
+                                       ws.data_ptr(), nb, _stream()), "sketch_hop")
+        _count(5 if n else 0)
+    return LinkSketches(mh, hll, hops, num_perm, hll_p, seed)
+
+
+def sketch_features(sk: LinkSketches, u: torch.Tensor, v: torch.Tensor) -> torch.Tensor:
+    """BUDDY's structure features of the pairs (u[i], v[i]) from their sketches (link_sketches) -> fp32 [P, hops^2 + 2 hops]:
+    the estimated counts A(d1, d2) of nodes at distance exactly d1 from u and d2 from v (row-major over d1, d2 = 1 .. hops), then
+    B_u(d) and B_v(d), the nodes at distance d from one endpoint and more than hops from the other (include/twowl.h restates the
+    estimators). One host read; raises IndexError when an id lies outside [0, N)."""
+    fn = "sketch_features"
+    _need_cuda(sk.minhash, sk.hll, u, v)
+    _sketch_params(fn, sk.hops, sk.num_perm, sk.hll_p)
+    u, v = u.reshape(-1).to(torch.int64), v.reshape(-1).to(torch.int64)
+    assert u.numel() == v.numel(), f"{fn}: u / v size mismatch"
+    dev, n, P = sk.minhash.device, sk.num_nodes, u.numel()
+    (pu, su), (pv, sv) = (_row(u), _row(v)) if P else ((0, 1), (0, 1))
+    out = torch.empty((P, sk.num_features), dtype=torch.float32, device=dev)
+    info = torch.empty(1, dtype=torch.int64, device=dev)
+    check(lib.twowl_sketch_pair_features(sk.hops, n, sk.num_perm, sk.hll_p, sk.minhash.data_ptr(), sk.hll.data_ptr(), pu, su, pv, sv, P,
+                                         out.data_ptr(), info.data_ptr(), _stream()), "sketch_pair_features")
+    _count(1 + int(P > 0))
+    nbad = int(info.item())
+    if nbad:
+        raise IndexError(f"{fn}: {nbad} pair(s) with an id outside [0, {n})")
+    return out
+
+
 RECOMMEND_MAX_ENTRIES = 1 << 26   # default expansion budget of one batch: 44 B of workspace per entry, about 3 GB
 
 
